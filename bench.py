@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Asso hot path on B200 (contract: see the task statement / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c1] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c1] [--impl reference] [--dump-outputs DIR]
 
 Metric: Asso cover-score throughput in Gop/s (algorithmic ops = 2*m*n*nb_t per greedy step,
 SURVEY.md section 8d) plus fit() seconds, on BASELINE.json's Netflix-shaped config (c4) by default.
@@ -50,6 +50,56 @@ def load_peaks():
             p = json.load(fh)
         return p, "MEASURED_PEAKS.json"
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT = 64 << 20                                           # bytes --dump-outputs may write in all
+
+
+def dump_rows(out, name, total, row_bytes, budget, take):
+    """out[name] = take(rows): every row of a `total`-row output when they fit `budget` bytes, else a fixed seeded sample
+    of rows (the same in every run with the same arguments), whose indices go to out[name + '_rows']."""
+    keep = min(total, max(1, budget // max(row_bytes, 1)))
+    rows = np.arange(total) if keep == total else np.sort(np.random.default_rng(0).choice(total, keep, replace=False))
+    out[name] = take(rows)
+    if keep < total:
+        out[name + "_rows"] = rows.astype(np.float64)
+
+
+def write_dump(out_dir, arrays):
+    """arrays (name -> float32 / float64 array) -> out_dir/<name>.npy."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def loop_outputs(eng, table, n_steps, rank):
+    """What the greedy loop computed up to its last step, as its caller receives it: per step the winner, score, #used
+    rows and cumulative TP / FP; the factor columns U (m x n_steps) and V (n x n_steps) as 0/1; and the gains of the
+    scoring pass that ended the last step (0 for candidates no longer alive: their gains are not computed exactly).
+    Every rank must call it (U is gathered over the ranks); rank 0 gets the arrays, the others None."""
+    from pybmf_b200 import device
+    t = table[:n_steps]
+    parts = eng.gather_used_words(list(range(n_steps)))
+    if rank != 0:
+        return None
+    out = {"winner": t[:, 0].astype(np.float64), "score": t[:, 1].copy().view(np.float64),
+           "used": t[:, 2].astype(np.float64), "tp": t[:, 5].astype(np.float64), "fp": t[:, 6].astype(np.float64)}
+    U = eng.unpack_used(parts, n_steps)
+    dump_rows(out, "U", eng.m, 4 * n_steps, 48 << 20, lambda r: U[r].astype(np.float32))
+    won = t[:, 0] >= 0
+    V = np.zeros((eng.n, n_steps), np.float32)
+    if won.any():
+        V[:, won] = device.words_to_dense(eng.basis_words_host(t[won, 0]), eng.n).T
+    dump_rows(out, "V", eng.n, 4 * n_steps, 12 << 20, lambda r: V[r])
+    alive = eng.alive[: eng.n].cpu().numpy() != 0
+    out["gain_p"] = np.where(alive, eng.gain_p_red[: eng.n].cpu().numpy(), 0).astype(np.float64)
+    if not eng.integer_mode:                                    # general weights: the N sums are the second output
+        out["gain_n"] = np.where(alive, eng.gain_n_red[: eng.n].cpu().numpy(), 0).astype(np.float64)
+    return out
 
 
 class ClockSampler:
@@ -173,11 +223,13 @@ def run_cpu_arm(args, X, workload, tau, w_fp, standalone):
     return out
 
 
-def product_sweep(points, steps, warmup, rank, world):
+def product_sweep(points, steps, warmup, rank, world, dump=None):
     """BASELINE.json configs[4]: bit-packed Boolean product U o V^T and the TP/FP/FN counts behind
     evaluate(), m up to 1M, n up to 100k, k = 64, rows sharded over the ranks (no data-path collective,
     three int64 counters are all-reduced).  One step = one materialised product + one confusion pass
-    against the product recomputed on the fly.  Algorithmic bytes: m*n/8 written + m*n/8 read."""
+    against the product recomputed on the fly.  Algorithmic bytes: m*n/8 written + m*n/8 read.
+    With a `dump` dict, rank 0 adds per point the last step's TP / FP / FN and rows of its product (a seeded
+    sample of rank 0's rows where they exceed 8 MB as float32)."""
     import torch
     import torch.distributed as dist
     from pybmf_b200 import _native, device
@@ -251,6 +303,11 @@ def product_sweep(points, steps, warmup, rank, world):
         ok = bool(torch.equal(counts, counts2))
         all_reduce_sum(counts)
         tp, fp, fn = (int(v) for v in counts.cpu().numpy())
+        if dump is not None and rank == 0:
+            key = "c5_%dx%d" % (m, n)
+            dump[key + "_counts"] = np.array([tp, fp, fn], dtype=np.float64)
+            dump_rows(dump, key + "_product", m_loc, 4 * n, 8 << 20, lambda r: device.words_to_dense(
+                pd[torch.as_tensor(r, device=pd.device)].cpu().numpy(), n).astype(np.float32))
         bytes_one = m * words * 8.0                              # one bit matrix, all ranks
         prod_gbs = bytes_one * args.steps / (t[0].item() / 1e3) / 1e9
         conf_gbs = bytes_one * args.steps / (t[1].item() / 1e3) / 1e9
@@ -295,8 +352,11 @@ def run_product_sweep(args, rank, world, local_rank, real_stdout):
     sampler = ClockSampler(local_rank)
     sampler.start()
     sampler.mark()
-    results = product_sweep(points, args.steps, max(args.warmup, 1), rank, world)
+    dump = {} if args.dump_outputs else None
+    results = product_sweep(points, args.steps, max(args.warmup, 1), rank, world, dump)
     clocks = sampler.stop()
+    if dump:
+        write_dump(args.dump_outputs, dump)
     ceilings = None
     if rank == 0:
         # context: what a pure write / pure read stream reaches on this box with library kernels
@@ -458,7 +518,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip roofline_i8 / popc comparison / other_configs")
     ap.add_argument("--fit-repeats", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (float32 / float64, at most "
+                         "64 MB; larger outputs as a seeded row sample), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference does not run it")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -552,6 +619,10 @@ def main():
     launches = eng.launches - launches0
     table = eng.read_table(0, args.warmup + args.steps)
     done = int((table[args.warmup:, 7] == 2).sum())             # steps that really chose and applied a winner
+    if args.dump_outputs:
+        outputs = loop_outputs(eng, table, args.warmup + args.steps, rank)
+        if outputs is not None:
+            write_dump(args.dump_outputs, outputs)
     score_ms = [a.elapsed_time(b) for a, b in eng.score_events]
     eng.score_events = None
     # the scoring pass of timed step t sees nb - (warmup + t + 1) live candidates (the winner was just removed)
