@@ -336,6 +336,15 @@ int bmf_refine_column(const uint64_t* x_bits, int64_t m, int64_t n, int64_t word
                       int64_t kw, const uint64_t* vt_bits, int64_t k, int64_t col, int32_t wa,
                       int32_t wb, double w_fp, double w_fn, int64_t* out, bmf_stream_t stream);
 
+/* Columns col0 .. col0+ncols-1 of AssoIter.get_refined_column in ONE pass over the rows; out[c][0..4] += what
+ * bmf_refine_column(col0 + c) would accumulate after columns col0 .. col0+c-1 were refined (TP, FP, #used, sum P,
+ * sum N), and u_words ends as after those ncols launches.  0 <= col0, ncols >= 1, col0 + ncols <= k; the shape rules
+ * are those of bmf_refine_column.  Rows are independent: a caller holding a slice of the rows gets that slice's share
+ * of every counter. */
+int bmf_refine_sweep(const uint64_t* x_bits, int64_t m, int64_t n, int64_t words, uint64_t* u_words, int64_t kw,
+                     const uint64_t* vt_bits, int64_t k, int64_t col0, int64_t ncols, int32_t wa, int32_t wb,
+                     double w_fp, double w_fn, int64_t* out, bmf_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -65,6 +65,7 @@ SIGNATURES = {
     "bmf_transpose_bits": [_p, _i64, _i64, _i64, _p, _i64, _p],
     "bmf_probe_mma_rate": [_i32, _i32, _p, _p],
     "bmf_refine_column": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
+    "bmf_refine_sweep": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
 }
 
 

@@ -1993,6 +1993,128 @@ refine_column_kernel(const uint64_t* __restrict__ xb, int64_t m, int64_t n, int6
   }
 }
 
+// AssoIter.get_refined_column for columns col0 .. col0+ncols-1 in ONE pass over the rows.  Row i's new bit U[i, c]
+// depends only on X_i, V and row i's own usage bits, so a warp walks the columns of its row in order (the bits of
+// columns already refined in this sweep are read back from the usage word) and adds the row's state after column c to
+// column c's counters: the sums equal what ncols successive refine_column_kernel launches accumulate.
+// With A = the cover without column c, the cover before column c is A | (old bit ? v_c : 0), hence
+//   TP(A) = TP - (old ? P : 0),  FP(A) = FP - (old ? N : 0),   P = |x & ~A & v_c|,  N = |~x & ~A & v_c|
+// so the row's TP / FP are carried from column to column (counted once, against the starting cover) and every column
+// costs two popcounts per word (P and |~A & v_c|) instead of the four of refine_column_kernel.  The data row is read
+// from DRAM once and re-read from L1 / L2 for the following columns; V^T sits in shared memory when it fits (VS).
+template <bool VS>
+__device__ __forceinline__ ulonglong2 ld_vt2(const uint64_t* p) {
+  if constexpr (VS) return *reinterpret_cast<const ulonglong2*>(p);
+  else return ld_words2(p);
+}
+
+template <bool VS>
+__device__ __forceinline__ void sweep_cover(const uint64_t* uw, int64_t kw, const uint64_t* V, int64_t words, int64_t p0,
+                                            int64_t pairs, int64_t skip, ulonglong2 (&acc)[PU]) {
+#pragma unroll
+  for (int u = 0; u < PU; ++u) acc[u] = make_ulonglong2(0ull, 0ull);
+  for (int64_t q = 0; q < kw; ++q) {
+    uint64_t sel = uw[q];
+    if ((skip >> 6) == q) sel &= ~(1ull << (skip & 63));
+    while (sel) {
+      const int l = __ffsll((long long)sel) - 1;
+      sel &= sel - 1;
+      const uint64_t* vrow = V + (q * 64 + l) * words;
+#pragma unroll
+      for (int u = 0; u < PU; ++u) {
+        const int64_t p = p0 + 32 * u;
+        if (p < pairs) {
+          const ulonglong2 v = ld_vt2<VS>(vrow + 2 * p);
+          acc[u].x |= v.x;
+          acc[u].y |= v.y;
+        }
+      }
+    }
+  }
+}
+
+template <bool VS>
+__global__ void __launch_bounds__(256)
+refine_sweep_kernel(const uint64_t* __restrict__ xb, int64_t m, int64_t words, uint64_t* __restrict__ u_words,
+                    int64_t kw, const uint64_t* __restrict__ vt, int64_t k, int64_t col0, int64_t ncols, int wa, int wb,
+                    double neg_w_fp, double w_fn, int cnt_in_smem, unsigned long long* __restrict__ out) {
+  extern __shared__ __align__(16) uint64_t sweep_smem[];
+  const int lane = threadIdx.x & 31;
+  const int64_t pairs = words >> 1;
+  const uint64_t* V = vt;
+  unsigned long long* cnt = out;                                        // [ncols][5]
+  if (VS) {
+    for (int64_t q = threadIdx.x; q < k * pairs; q += blockDim.x)
+      reinterpret_cast<ulonglong2*>(sweep_smem)[q] = ld_words2(vt + 2 * q);
+    V = sweep_smem;
+  }
+  if (cnt_in_smem) {
+    cnt = reinterpret_cast<unsigned long long*>(sweep_smem + (VS ? k * words : 0));
+    for (int64_t q = threadIdx.x; q < ncols * 5; q += blockDim.x) cnt[q] = 0ull;
+  }
+  if (VS || cnt_in_smem) __syncthreads();
+  const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t i = warp0; i < m; i += nwarps) {
+    const uint64_t* x = xb + i * words;
+    uint64_t* uw = u_words + i * kw;
+    int tp = 0, pd = 0;
+    for (int64_t p0 = lane; p0 < pairs; p0 += 32 * PU) {                 // TP / FP of the starting cover
+      ulonglong2 c[PU];
+      sweep_cover<VS>(uw, kw, V, words, p0, pairs, -1, c);
+#pragma unroll
+      for (int u = 0; u < PU; ++u) {
+        const int64_t p = p0 + 32 * u;
+        if (p >= pairs) continue;
+        const ulonglong2 xv = ld_words2(x + 2 * p);
+        tp += __popcll(xv.x & c[u].x) + __popcll(xv.y & c[u].y);
+        pd += __popcll(c[u].x) + __popcll(c[u].y);
+      }
+    }
+    tp = warp_sum(tp);
+    int fp = warp_sum(pd) - tp;
+    for (int64_t j = 0; j < ncols; ++j) {
+      const int64_t col = col0 + j;
+      const uint64_t* vcol = V + col * words;
+      int P = 0, A = 0;
+      for (int64_t p0 = lane; p0 < pairs; p0 += 32 * PU) {
+        ulonglong2 c[PU];
+        sweep_cover<VS>(uw, kw, V, words, p0, pairs, col, c);           // cover without factor `col`
+#pragma unroll
+        for (int u = 0; u < PU; ++u) {
+          const int64_t p = p0 + 32 * u;
+          if (p >= pairs) continue;
+          const ulonglong2 xv = ld_words2(x + 2 * p);
+          const ulonglong2 v = ld_vt2<VS>(vcol + 2 * p);
+          const uint64_t nx = v.x & ~c[u].x, ny = v.y & ~c[u].y;
+          P += __popcll(xv.x & nx) + __popcll(xv.y & ny);
+          A += __popcll(nx) + __popcll(ny);                               // |v & ~c| = P + N
+        }
+      }
+      P = warp_sum(P);
+      const int N = warp_sum(A) - P;
+      const uint64_t bit = 1ull << (col & 63);
+      const bool old = (uw[col >> 6] & bit) != 0;
+      const int tpo = tp - (old ? P : 0), fpo = fp - (old ? N : 0);
+      const bool use = row_uses(wa, wb, neg_w_fp, w_fn, tpo, fpo, P, N);  // warp-uniform
+      tp = tpo + (use ? P : 0);
+      fp = fpo + (use ? N : 0);
+      __syncwarp();
+      if (lane == 0 && use != old) uw[col >> 6] ^= bit;                  // AssoIter.py:60: always overwritten
+      if (lane < 5) {
+        const int v = lane == 0 ? tp : lane == 1 ? fp : !use ? 0 : lane == 2 ? 1 : lane == 3 ? P : N;
+        if (v) atomicAdd(cnt + j * 5 + lane, (unsigned long long)v);
+      }
+      __syncwarp();
+    }
+  }
+  if (cnt_in_smem) {
+    __syncthreads();
+    for (int64_t q = threadIdx.x; q < ncols * 5; q += blockDim.x)
+      if (cnt[q]) atomicAdd(out + q, cnt[q]);
+  }
+}
+
 // =========================================================================================
 // GreConD+ expansion scores (PyBMF/models/GreConDPlus.py:267-308, `_expansion`): adding `pattern` to every row that is
 // not excluded, how much does each row's coverage score change?
@@ -2700,6 +2822,38 @@ extern "C" int bmf_refine_column(const uint64_t* x_bits, int64_t m, int64_t n, i
       x_bits, m, n, words, u_words, kw, vt_bits, col, wa, wb, -w_fp, w_fn,
       reinterpret_cast<unsigned long long*>(out));
   BMF_LAUNCH_CHECK("bmf_refine_column");
+  return 0;
+}
+
+extern "C" int bmf_refine_sweep(const uint64_t* x_bits, int64_t m, int64_t n, int64_t words, uint64_t* u_words,
+                                int64_t kw, const uint64_t* vt_bits, int64_t k, int64_t col0, int64_t ncols, int32_t wa,
+                                int32_t wb, double w_fp, double w_fn, int64_t* out, bmf_stream_t stream) {
+  BMF_REQUIRE(x_bits && u_words && vt_bits && out, "bmf_refine_sweep: null pointer");
+  BMF_REQUIRE(m > 0 && n > 0 && words % 2 == 0 && words * 64 >= n && kw > 0 && k <= kw * 64, "bmf_refine_sweep: bad shape");
+  BMF_REQUIRE(col0 >= 0 && ncols >= 1 && col0 + ncols <= k, "bmf_refine_sweep: columns out of range");
+  const size_t vt_bytes = (size_t)k * (size_t)words * sizeof(uint64_t);
+  const size_t cnt_bytes = (size_t)ncols * 5 * sizeof(unsigned long long);
+  const bool vs = vt_bytes <= 96 * 1024;                // V^T in shared memory; larger V^T is read through L1 / L2
+  const int cnt_in_smem = cnt_bytes <= 32 * 1024;       // per-block column counters, else atomics straight to `out`
+  const size_t smem = (vs ? vt_bytes : 0) + (cnt_in_smem ? cnt_bytes : 0);
+  const void* fn = vs ? (const void*)refine_sweep_kernel<true> : (const void*)refine_sweep_kernel<false>;
+  int rc = check_cuda(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "bmf_refine_sweep");
+  if (rc) return rc;
+  int per_sm = 0;
+  rc = check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, 256, smem), "bmf_refine_sweep");
+  if (rc) return rc;
+  int64_t blocks = ceil_div(m, 8);
+  const int64_t resident = (int64_t)num_sms() * (per_sm > 0 ? per_sm : 1);
+  if (blocks > resident) blocks = resident;              // every block stages V^T once: no more blocks than fit at once
+  if (vs)
+    refine_sweep_kernel<true><<<(unsigned)blocks, 256, smem, as_stream(stream)>>>(
+        x_bits, m, words, u_words, kw, vt_bits, k, col0, ncols, wa, wb, -w_fp, w_fn, cnt_in_smem,
+        reinterpret_cast<unsigned long long*>(out));
+  else
+    refine_sweep_kernel<false><<<(unsigned)blocks, 256, smem, as_stream(stream)>>>(
+        x_bits, m, words, u_words, kw, vt_bits, k, col0, ncols, wa, wb, -w_fp, w_fn, cnt_in_smem,
+        reinterpret_cast<unsigned long long*>(out));
+  BMF_LAUNCH_CHECK("bmf_refine_sweep");
   return 0;
 }
 

@@ -22,7 +22,7 @@ from scipy.sparse import csr_matrix, hstack, lil_matrix
 
 from . import _native, device
 from . import utils as U_
-from .engine import CoverEngine, all_reduce_sum, dist_ctx, integer_weights
+from .engine import CoverEngine, ShardPlan, _Trace, all_reduce_sum, dist_ctx, integer_weights
 
 CONFIG_KEYS = ("task", "seed", "display", "verbose", "scaling", "pixels", "show_logs", "save_model", "show_result")
 SILENT = bool(int(os.environ.get("PYBMF_B200_SILENT", "0")))
@@ -378,6 +378,64 @@ def _csr_to_lil_fast(A: csr_matrix) -> lil_matrix:
     return out
 
 
+def _local_rows(X):
+    """(plan, r0, r1, bit rows) of this rank's share of the training matrix under ShardPlan.  A generate.DeviceBits is
+    used as it is; of a host csr only the rank's rows are packed, from a zero-copy row view."""
+    rank, world = dist_ctx()
+    plan = ShardPlan(X.shape[0], world)
+    r0, r1 = plan.rows(rank)
+    if hasattr(X, "bits"):
+        assert (X.r0, X.r1) == (r0, r1), "DeviceBits rows must follow ShardPlan(m, world).rows(rank)"
+        return plan, r0, r1, X.bits
+    Xl = device.csr_rows_view(X, r0, r1)
+    if device.has_stored_zeros(Xl):                             # the packer takes every STORED entry as a one
+        Xl = device.drop_stored_zeros(Xl)
+    return plan, r0, r1, U_._bits_on_device(Xl)
+
+
+def _gather_rows(local, plan):
+    """This rank's row block (device tensor, >= its row count rows) -> the rows of ALL ranks as one host array, in row
+    order, on every rank: one all-gather.  Rank r's rows start at r times rank 0's row count (ShardPlan)."""
+    rank, world = dist_ctx()
+    if world == 1:
+        return local[: plan.m].cpu().numpy()
+    import torch.distributed as dist
+    r0, r1 = plan.rows(rank)
+    per = plan.rows(0)[1]
+    tail = tuple(local.shape[1:])
+    padded = torch.zeros((per,) + tail, dtype=local.dtype, device=local.device)
+    padded[: r1 - r0] = local[: r1 - r0]
+    gathered = torch.empty((world * per,) + tail, dtype=local.dtype, device=local.device)
+    dist.all_gather_into_tensor(gathered, padded)
+    return gathered[: plan.m].cpu().numpy()
+
+
+def replay_sweep(table, k, sum_x, size, w_fp, w_fn, best_error, best_score, n_stop):
+    """The host side of one AssoIter sweep (AssoIter.py:55-77) on the per-column table of bmf_refine_sweep summed over
+    all rows: row c holds (TP, FP, ...) of the whole matrix after column c was refined.
+
+    Returns (steps, stop, best_error, best_score, n_stop).  `steps` lists the columns the reference visits, in order, as
+    dicts {k, accepted, and for accepted columns: tp, fp, fn, score, error, score_before, error_before}; `stop` is the
+    column after which the reference stops (n_stop reached k), else None."""
+    steps = []
+    for c in range(k):
+        tp, fp = int(table[c][0]), int(table[c][1])
+        score = -w_fp * np.array(fp, dtype=np.int64) + w_fn * np.array(tp, dtype=np.int64)
+        fn = sum_x - tp
+        error = U_.rates(tp, fp, fn, size)["ERR"]
+        if error < best_error:
+            steps.append({"k": c, "accepted": True, "tp": tp, "fp": fp, "fn": fn, "score": score, "error": error,
+                          "score_before": best_score, "error_before": best_error})
+            best_error, best_score = error, score
+            n_stop = 0
+        else:
+            steps.append({"k": c, "accepted": False})
+            n_stop += 1
+            if n_stop == k:
+                return steps, c, best_error, best_score, n_stop
+    return steps, None, best_error, best_score, n_stop
+
+
 def _column(vec, n):
     """uint8 vector -> (n x 1) csr float64, the container set_factors() assigns from."""
     idx = np.flatnonzero(vec)
@@ -674,39 +732,50 @@ class AssoIter(Asso):
         BaseModel._init_factors(self)
 
     def _fit(self):
+        """Rows are sharded like Asso's (ShardPlan over the ranks of an initialised process group): each rank refines
+        only its rows, and ONE all-reduce per sweep of the [k][5] per-column table gives every rank the same integers,
+        from which every rank replays the same accept / skip / stop decisions (replay_sweep)."""
         _native.require_gpu()
+        if self.k > self.U.shape[1]:                                              # U[:, idx] in AssoIter.py:85-86
+            raise IndexError("index (%d) out of range" % (self.k - 1))
+        trace = _Trace()
+        self._dev_trace = trace
         m, n = self.m, self.n
         size = m * n
         w_fp = self.w_fp
         w_fn = 1 - self.w_fp if self.w_fn is None else self.w_fn
         iw = integer_weights(float(w_fp), float(w_fn))
         wa, wb, _s = iw if iw else (0, 0, 0)
-        X = device.to_csr_pattern(self.X_train)
-        sum_x = int(X.nnz)
-        x_bits = U_._bits_on_device(X)
+        plan, r0, r1, x_bits = _local_rows(self.X_train)
+        m_loc = r1 - r0
         words = device.words_for(n)
+        trace.mark("upload_pack")
         kU = self.U.shape[1]
-        uw, kw = U_._factor_words(U_._pattern(self.U))
+        uw, kw = U_._factor_words(U_._pattern(self.U)[r0:r1])
         vt = U_._bits_on_device(U_._pattern(self.V).T.tocsr())
-        counts = device.zeros((3,), torch.int64)
-        _native.call("bmf_confusion_factors", x_bits, m, words, uw, kw, vt, kU, sum_x, counts, None, None)
-        tp, fp, _fn = (int(v) for v in counts.cpu().numpy())
+        trace.mark("usage_words")
+        counts = device.zeros((3,), torch.int64)                                  # TP, FP, FN of this rank's rows
+        if m_loc > 0:
+            _native.call("bmf_confusion_factors", x_bits, m_loc, words, uw, kw, vt, kU, -1, counts, None, None)
+        tp, fp, fn = (int(v) for v in all_reduce_sum(counts).cpu().numpy())
+        sum_x = tp + fn
         best_score = -w_fp * np.array(fp, dtype=np.int64) + w_fn * np.array(tp, dtype=np.int64)   # AssoIter.py:52
-        best_error = U_.rates(tp, fp, sum_x - tp, size)["ERR"]
+        best_error = U_.rates(tp, fp, fn, size)["ERR"]
         n_stop = 0
         is_improving = True
-        # A sweep over the k columns is deterministic on the device (U[:, k] is ALWAYS replaced, AssoIter.py:60): all k
-        # refinements are enqueued back to back into a per-column table, read with one sync, and the accept / skip / stop
-        # bookkeeping is replayed on the host.  If the reference would have stopped in the middle of the sweep, the usage
-        # words are restored from the snapshot and the sweep is re-run up to that column.
+        # A sweep over the k columns is deterministic on the device (U[:, k] is ALWAYS replaced, AssoIter.py:60): one
+        # bmf_refine_sweep launch refines every column of the rank's rows and fills the per-column table, which is
+        # all-reduced and read with one sync, and the accept / skip / stop bookkeeping is replayed on the host.  If the
+        # reference would have stopped in the middle of the sweep, the usage words are restored from the snapshot and
+        # the sweep is re-run up to that column.
         table = device.zeros((max(self.k, 1), 5), torch.int64)
         with_splits = self.X_val is not None or self.X_test is not None
 
         def write_back():                                       # usage words -> the lil U the caller holds (in place: D7)
             # The reference assigns U[:, k] column by column on the SAME lil object the source model holds (AssoIter.py:28,
-            # 60); here all columns are rebuilt from the usage words at once and the object's row lists are replaced in
-            # place (a lil column assignment walks every row: 0.3 ms per column at 6040 rows).
-            dense = device.words_to_dense(uw.cpu().numpy(), kU)                   # [m, kU] uint8
+            # 60); here all columns are rebuilt from the usage words of every rank at once and the object's row lists are
+            # replaced in place (a lil column assignment walks every row: 0.3 ms per column at 6040 rows).
+            dense = device.words_to_dense(_gather_rows(uw, plan), kU)             # [m, kU] uint8
             new = _csr_to_lil_fast(csr_matrix(dense, dtype=self.U.dtype))
             if sp.isspmatrix_lil(self.U) and self.U.shape == new.shape:
                 self.U.rows[:] = new.rows
@@ -716,48 +785,44 @@ class AssoIter(Asso):
                     self.U[:, c] = _column(dense[:, c], m)
             self.__dict__.pop("X_pd", None)
 
-        def sweep(upto):
+        def run(upto):
             table.zero_()
-            for c in range(upto):
-                _native.call("bmf_refine_column", x_bits, m, n, words, uw, kw, vt, kU, c, wa, wb, float(w_fp),
-                             float(w_fn), table[c])
-            return table.cpu().numpy()
+            if upto > 0 and m_loc > 0:
+                _native.call("bmf_refine_sweep", x_bits, m_loc, n, words, uw, kw, vt, kU, 0, upto, wa, wb, float(w_fp),
+                             float(w_fn), table)
 
         while is_improving:
-            if self.k > kU:                                                       # U[:, idx] in AssoIter.py:85-86
-                raise IndexError("index (%d) out of range" % (self.k - 1))
             snapshot = uw.clone()
-            rows = sweep(self.k)
-            for k in range(self.k):
-                tp, fp = int(rows[k][0]), int(rows[k][1])
-                score = -w_fp * np.array(fp, dtype=np.int64) + w_fn * np.array(tp, dtype=np.int64)
-                fn = sum_x - tp
-                error = U_.rates(tp, fp, fn, size)["ERR"]
-                if error < best_error:
-                    _say("[I] Refined column i: {}, error: {:.4f} -> {:.4f}, score: {:.2f} -> {:.2f}.".format(
-                        k, best_error, error, float(best_score), float(score)))
-                    best_error, best_score = error, score
-                    self._dev_counts = (tp, fp, fn, size)
-                    if with_splits:                                               # val / test counts read self.U as of now
-                        now = uw.clone()
-                        uw.copy_(snapshot)
-                        sweep(k + 1)
-                        write_back()
-                        uw.copy_(now)
-                    self.evaluate(df_name="refinements", head_info={"k": k},
-                                  train_info={"score": best_score, "error": best_error})
-                    n_stop = 0
-                else:
-                    n_stop += 1
+            run(self.k)
+            rows = all_reduce_sum(table).cpu().numpy()
+            steps, stop, best_error, best_score, n_stop = replay_sweep(rows, self.k, sum_x, size, w_fp, w_fn, best_error,
+                                                                       best_score, n_stop)
+            for s in steps:
+                k = s["k"]
+                if not s["accepted"]:
                     _say("[I] Skipped column i: {}.".format(k))
-                    if n_stop == self.k:
-                        _say("[I] Error stops decreasing.")
-                        is_improving = False
-                        if k < self.k - 1:                                        # undo the columns the reference never reached
-                            uw.copy_(snapshot)
-                            sweep(k + 1)
-                        break
+                    continue
+                _say("[I] Refined column i: {}, error: {:.4f} -> {:.4f}, score: {:.2f} -> {:.2f}.".format(
+                    k, s["error_before"], s["error"], float(s["score_before"]), float(s["score"])))
+                self._dev_counts = (s["tp"], s["fp"], s["fn"], size)
+                if with_splits:                                                   # val / test counts read self.U as of now
+                    now = uw.clone()
+                    uw.copy_(snapshot)
+                    run(k + 1)
+                    write_back()
+                    uw.copy_(now)
+                self.evaluate(df_name="refinements", head_info={"k": k},
+                              train_info={"score": s["score"], "error": s["error"]})
+            if stop is not None:
+                _say("[I] Error stops decreasing.")
+                is_improving = False
+                if stop < self.k - 1:                                             # undo the columns the reference never reached
+                    uw.copy_(snapshot)
+                    run(stop + 1)
+        trace.mark("sweeps")
         write_back()
+        trace.mark("write_back")
+        trace.dump(dist_ctx()[0])
         self.__dict__.pop("_dev_counts", None)
 
 
@@ -806,21 +871,35 @@ class AssoOpt(Asso):
         BaseModel._init_factors(self)
 
     def optimal_rows(self, rows=None):
-        """argmax trial of every data row (or of `rows`) and its score: int64 [m], float64 [m]."""
+        """argmax trial of every data row (or of `rows`) and its score: int64 [m], float64 [m].
+
+        Without `rows` this is a collective under an initialised process group: each rank searches its ShardPlan rows and
+        one all-gather gives every rank all of them.  Explicit `rows` are searched locally, with no collective (of a
+        generate.DeviceBits input only this rank's rows can be asked for)."""
         _native.require_gpu()
-        X = device.to_csr_pattern(self.X_train)
-        if rows is not None:
-            X = X[np.asarray(rows, dtype=np.int64)]
-        m = X.shape[0]
-        x_bits = U_._bits_on_device(X)
         vt = U_._bits_on_device(U_._pattern(self.V).T.tocsr())
         if vt.shape[0] != self.k:
             raise ValueError("shapes (1,%d) and (%d,%d) not aligned" % (self.k, vt.shape[0], self.n))   # int2bin(j, k) @ V.T
+        X = self.X_train
+        plan = None
+        if rows is not None:
+            idx = np.asarray(rows, dtype=np.int64).reshape(-1)
+            if hasattr(X, "bits"):
+                assert ((idx >= X.r0) & (idx < X.r1)).all(), "DeviceBits holds rows [%d, %d) only" % (X.r0, X.r1)
+                x_bits = X.bits[torch.from_numpy(idx - X.r0).to(X.bits.device)]
+            else:
+                x_bits = U_._bits_on_device(device.to_csr_pattern(X)[idx])
+            m = len(idx)
+        else:
+            plan, r0, r1, x_bits = _local_rows(X)
+            m = r1 - r0
         best = device.zeros((max(m, 1),), torch.int64)
         score = device.zeros((max(m, 1),), torch.float64)
         if m > 0:
             _native.call("bmf_optimal_rows", x_bits, m, x_bits.shape[1], vt, self.k, float(self.w_fp), float(self.w_fn),
                          best, score)
+        if plan is not None:
+            return _gather_rows(best, plan), _gather_rows(score, plan)
         return best.cpu().numpy()[:m], score.cpu().numpy()[:m]
 
     def set_optimal_row(self, i):
