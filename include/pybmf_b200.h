@@ -313,7 +313,9 @@ int bmf_optimal_rows(const uint64_t* x_bits, int64_t m, int64_t words, const uin
  * bmf_random_bits: bits[r][.] = Bernoulli(p) for logical row row0 + r (pad bits 0).
  * bmf_noise_bits : add_noise -- ones dropped with probability p_pos, then entries set with probability p_neg.
  * bmf_transpose_bits: bits [rows][words] -> bits_t [ncols][words_t] (caller zero-fills bits_t's pad words), the X^T the
- * association needs when X never existed as a csr. */
+ * association needs when X never existed as a csr.  `words` and `words_t` are row strides, so a column window of bits
+ * (pointer advanced by whole words) or a word offset into bits_t can be passed; rows <= 4.19M per call.  Writes only
+ * bits_t[c][w] with c < ncols and 64 w < rows. */
 int bmf_random_bits(uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, int64_t row0, uint64_t seed,
                     uint64_t stream_id, double p, bmf_stream_t stream);
 int bmf_noise_bits(uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, int64_t row0, uint64_t seed, double p_pos,

@@ -2301,23 +2301,64 @@ __global__ void noise_bits_kernel(uint64_t* __restrict__ x, int64_t rows, int64_
     x[t] = v;
   }
 }
-// bit-matrix transpose: x [rows][words] -> xt [ncols][words_t] (bit r of xt row c = bit c of x row r); one CTA of 64
-// threads per 64 x 64 bit tile: thread t holds row t's word, ballots give the 64 column words
-__global__ void __launch_bounds__(64) transpose_bits_kernel(const uint64_t* __restrict__ x, int64_t rows, int64_t ncols,
-                                                            int64_t words, uint64_t* __restrict__ xt, int64_t words_t) {
-  __shared__ uint32_t half[64][2];
+// 64 x 64 bit-block transpose in registers: lane l holds rows l (a0) and l + 32 (a1) of the block and afterwards its
+// columns l and l + 32 as rows.  Six block-swap stages (Hacker's Delight, 7-3): 32 inside the thread, 16 .. 1 between
+// lanes by shuffles -- about 60 instructions per warp and block instead of 64 ballots per warp.
+__device__ __forceinline__ void transpose64_warp(uint64_t& a0, uint64_t& a1, int lane) {
+  {
+    const uint64_t t = ((a0 >> 32) ^ a1) & 0x00000000FFFFFFFFull;
+    a1 ^= t;
+    a0 ^= t << 32;
+  }
+  const uint64_t masks[5] = {0x0000FFFF0000FFFFull, 0x00FF00FF00FF00FFull, 0x0F0F0F0F0F0F0F0Full, 0x3333333333333333ull,
+                             0x5555555555555555ull};
+#pragma unroll
+  for (int s = 0; s < 5; ++s) {
+    const int j = 16 >> s;
+    const bool hi = lane & j;                                  // this lane holds row k | j of each swapped pair
+    const uint64_t p0 = __shfl_xor_sync(0xffffffffu, a0, j), p1 = __shfl_xor_sync(0xffffffffu, a1, j);
+    const uint64_t t0 = (((hi ? p0 : a0) >> j) ^ (hi ? a0 : p0)) & masks[s];
+    const uint64_t t1 = (((hi ? p1 : a1) >> j) ^ (hi ? a1 : p1)) & masks[s];
+    a0 ^= hi ? t0 : (t0 << j);
+    a1 ^= hi ? t1 : (t1 << j);
+  }
+}
+
+// bit-matrix transpose: x [rows][words] -> xt [ncols][words_t] (bit r of xt row c = bit c of x row r).  One CTA of 256
+// threads per 256-row x 512-column tile (4 x 8 blocks of 64 x 64), staged through shared memory so that the loads read
+// 64 B of every row and the stores write 32 B of every output row; each warp transposes 4 blocks in registers.  Only the
+// words xt[c][w] with c < ncols and 64 w < rows are written.
+constexpr int kTransposeRowBlocks = 4, kTransposeColWords = 8;
+__global__ void __launch_bounds__(256) transpose_bits_kernel(const uint64_t* __restrict__ x, int64_t rows, int64_t ncols,
+                                                             int64_t words, uint64_t* __restrict__ xt, int64_t words_t) {
+  constexpr int RB = kTransposeRowBlocks, CW = kTransposeColWords;
+  __shared__ uint64_t tin[RB * 64][CW + 1];                    // +1: the column reads below hit distinct banks
+  __shared__ uint64_t tout[CW * 64][RB + 1];
   const int t = threadIdx.x, lane = t & 31, wp = t >> 5;
-  const int64_t cb = blockIdx.x, rb = blockIdx.y;
-  const int64_t r = rb * 64 + t;
-  const uint64_t w = (r < rows) ? x[r * words + cb] : 0ull;
-#pragma unroll 8
-  for (int c = 0; c < 64; ++c) {
-    const uint32_t b = __ballot_sync(0xffffffffu, (w >> c) & 1ull);
-    if (lane == 0) half[c][wp] = b;
+  const int64_t w0 = (int64_t)blockIdx.x * CW, r0 = (int64_t)blockIdx.y * (RB * 64);
+  const int64_t wn = (ncols + 63) >> 6;                        // words of a row that hold columns < ncols
+#pragma unroll
+  for (int q = 0; q < RB * 64 * CW / 256; ++q) {
+    const int i = t + 256 * q, rr = i / CW, cw = i % CW;
+    const int64_t r = r0 + rr, w = w0 + cw;
+    tin[rr][cw] = (r < rows && w < wn) ? x[r * words + w] : 0ull;
   }
   __syncthreads();
-  const int64_t col = cb * 64 + t;
-  if (col < ncols) xt[col * words_t + rb] = (uint64_t)half[t][0] | ((uint64_t)half[t][1] << 32);
+#pragma unroll
+  for (int q = 0; q < RB * CW / 8; ++q) {
+    const int blk = wp + 8 * q, rb = blk % RB, cw = blk / RB;
+    uint64_t a0 = tin[rb * 64 + lane][cw], a1 = tin[rb * 64 + 32 + lane][cw];
+    transpose64_warp(a0, a1, lane);
+    tout[cw * 64 + lane][rb] = a0;
+    tout[cw * 64 + 32 + lane][rb] = a1;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int q = 0; q < CW * 64 * RB / 256; ++q) {
+    const int i = t + 256 * q, cc = i / RB, rb = i % RB;
+    const int64_t col = w0 * 64 + cc, wt = (int64_t)blockIdx.y * RB + rb;
+    if (col < ncols && wt * 64 < rows && wt < words_t) xt[col * words_t + wt] = tout[cc][rb];
+  }
 }
 
 static inline int row_stream_grid() { return num_sms() * 8; }
@@ -2930,9 +2971,9 @@ extern "C" int bmf_transpose_bits(const uint64_t* bits, int64_t rows, int64_t nc
                                   int64_t words_t, bmf_stream_t stream) {
   BMF_REQUIRE(bits && bits_t && rows > 0 && ncols > 0, "bmf_transpose_bits: bad arguments");
   BMF_REQUIRE(words * 64 >= ncols && words_t * 64 >= rows, "bmf_transpose_bits: word counts must cover the matrix");
-  dim3 grid((unsigned)ceil_div(ncols, 64), (unsigned)ceil_div(rows, 64));
-  BMF_REQUIRE(grid.y <= 65535u, "bmf_transpose_bits: more than 4.19M rows per call; transpose in row chunks");
-  transpose_bits_kernel<<<grid, 64, 0, as_stream(stream)>>>(bits, rows, ncols, words, bits_t, words_t);
+  BMF_REQUIRE(ceil_div(rows, 64) <= 65535, "bmf_transpose_bits: more than 4.19M rows per call; transpose in row chunks");
+  dim3 grid((unsigned)ceil_div(ceil_div(ncols, 64), kTransposeColWords), (unsigned)ceil_div(rows, 64 * kTransposeRowBlocks));
+  transpose_bits_kernel<<<grid, 256, 0, as_stream(stream)>>>(bits, rows, ncols, words, bits_t, words_t);
   BMF_LAUNCH_CHECK("bmf_transpose_bits");
   return 0;
 }

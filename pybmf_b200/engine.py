@@ -61,6 +61,18 @@ def dist_ctx():
     return 0, 1
 
 
+def local_plan(X):
+    """(plan, r0, r1): ShardPlan of X's rows over the ranks of the process group and this rank's rows.  A
+    generate.DeviceBits must hold exactly those rows, else ValueError (raised before any collective)."""
+    rank, world = dist_ctx()
+    plan = ShardPlan(X.shape[0], world)
+    r0, r1 = plan.rows(rank)
+    if hasattr(X, "bits") and (X.r0, X.r1) != (r0, r1):
+        raise ValueError("DeviceBits rows [%d, %d) must follow ShardPlan(m, world).rows(rank) = [%d, %d)"
+                         % (X.r0, X.r1, r0, r1))
+    return plan, r0, r1
+
+
 def all_reduce_sum(t):
     """In-place integer SUM across ranks (NCCL on GPU tensors, gloo on CPU tensors in tests)."""
     import torch.distributed as dist
@@ -102,8 +114,7 @@ class CoverEngine:
         self.trace = _Trace()
         self.rank, self.world = dist_ctx()
         self.m, self.n = X.shape
-        self.plan = ShardPlan(self.m, self.world)
-        r0, r1 = self.plan.rows(self.rank)
+        self.plan, r0, r1 = local_plan(X)
         self.r0, self.r1 = r0, r1
         self.m_loc = r1 - r0
         # Each rank takes only ITS rows (a view, no copy).  The packer ORs bits, so unsorted or duplicate column
@@ -113,7 +124,6 @@ class CoverEngine:
         self._ctor_args = (w_fp, w_fn, scorer, assoc, rescore)
         on_device = hasattr(X, "bits") and hasattr(X, "r0")     # generate.DeviceBits: this rank's rows are already bit rows
         if on_device:
-            assert (X.r0, X.r1) == (r0, r1), "DeviceBits rows must follow ShardPlan(m, world).rows(rank)"
             Xl = None
         else:
             Xl = device.csr_rows_view(X, r0, r1)

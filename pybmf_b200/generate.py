@@ -14,7 +14,7 @@ import scipy.sparse as sp
 import torch
 
 from . import _native, device
-from .engine import ShardPlan, dist_ctx
+from .engine import ShardPlan, dist_ctx, local_plan
 
 
 class DeviceBits:
@@ -75,12 +75,64 @@ def planted_bits(m, n, k_true, d_u, d_v, p_fn, p_fp, seed, rank=None, world=None
     return DeviceBits(bits, m, n, r0, r1)
 
 
+_TRANSPOSE_STEP = 64 * 65535                                    # rows per bmf_transpose_bits launch (grid.y limit)
+
+
+def _transpose_into(bits, rows, ncols, out, words_t):
+    """Transpose the bit rows [rows][ncols bits] (row stride bits.stride(0)) into the first words of the rows of `out`
+    (row stride words_t), in row chunks of _TRANSPOSE_STEP (a multiple of 64, so every chunk starts at a whole word)."""
+    for a in range(0, rows, _TRANSPOSE_STEP):
+        b = min(rows, a + _TRANSPOSE_STEP)
+        _native.call("bmf_transpose_bits", bits[a:b], b - a, ncols, bits.stride(0), out[:, a // 64:], words_t)
+
+
 def transpose_bits(bits, rows, ncols):
     """Bit matrix [rows][words(ncols)] -> its transpose [ncols][words(rows)] on the device."""
     words_t = device.words_for(rows)
     out = device.zeros((max(ncols, 1), words_t), torch.int64)
-    step = 64 * 65535                                           # rows per launch (grid.y limit), a multiple of 64
-    for a in range(0, rows, step):
-        b = min(rows, a + step)
-        _native.call("bmf_transpose_bits", bits[a:b], b - a, ncols, bits.shape[1], out[:, a // 64:], words_t)
+    _transpose_into(bits, rows, ncols, out, words_t)
     return out
+
+
+def transpose_slots(m, n, world):
+    """Layout of the one all-to-all exchange of `transpose` for an m x n matrix over `world` ranks (pure host logic).
+
+    Rank r holds rows rows[r] of X and receives rows cols[r] of X^T (both ShardPlan).  Every rank sends every rank s one
+    slot of slot_rows x slot_words int64 words: the transpose of its rows restricted to columns cols[s], which start at
+    word src_word[s] of its bit rows.  The slot rank s receives from rank r fills used_words[r] words of each of its X^T
+    rows (words_t words), starting at word dst_word[r].  Slots of a rank without rows or columns are sent all the same,
+    as zeros."""
+    rows, cols = ShardPlan(m, world).bounds, ShardPlan(n, world).bounds
+    for lo, hi in rows + cols:
+        assert lo % 64 == 0 or lo == hi, "the ranges of ranks that hold rows start at whole words"
+    used = [(r1 - r0 + 63) // 64 for r0, r1 in rows]
+    return {"rows": rows, "cols": cols, "slot_rows": max(c1 - c0 for c0, c1 in cols), "slot_words": max(used),
+            "src_word": [c0 // 64 for c0, _c1 in cols], "dst_word": [r0 // 64 for r0, _r1 in rows], "used_words": used,
+            "words_t": device.words_for(m)}
+
+
+def transpose(X: DeviceBits) -> DeviceBits:
+    """X^T of a row-sharded bit matrix, sharded the same way: this rank gets rows ShardPlan(n, world).rows(rank) of X^T,
+    whatever the number of ranks.  With several ranks this is a collective (ONE all_to_all_single of transpose_slots);
+    the send and the receive buffer take about m_loc * n / 8 bytes each."""
+    local_plan(X)
+    rank, world = dist_ctx()
+    if world == 1:
+        return DeviceBits(transpose_bits(X.bits, X.m, X.n), X.n, X.m, 0, X.n)
+    import torch.distributed as dist
+    L = transpose_slots(X.m, X.n, world)
+    sr, sw, wt = L["slot_rows"], L["slot_words"], L["words_t"]
+    send = device.zeros((world, sr, sw), torch.int64)
+    m_loc = X.r1 - X.r0
+    for s, (c0, c1) in enumerate(L["cols"]):
+        if m_loc > 0 and c1 > c0:
+            _transpose_into(X.bits[:, L["src_word"][s]:], m_loc, c1 - c0, send[s], sw)
+    recv = torch.empty_like(send)
+    dist.all_to_all_single(recv, send)
+    c0, c1 = L["cols"][rank]
+    out = device.zeros((max(c1 - c0, 1), wt), torch.int64)
+    for r in range(world):
+        w0, nw = L["dst_word"][r], L["used_words"][r]
+        if nw > 0 and c1 > c0:
+            out[: c1 - c0, w0:w0 + nw] = recv[r, : c1 - c0, :nw]
+    return DeviceBits(out, X.n, X.m, c0, c1)

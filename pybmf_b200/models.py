@@ -22,7 +22,7 @@ from scipy.sparse import csr_matrix, hstack, lil_matrix
 
 from . import _native, device
 from . import utils as U_
-from .engine import CoverEngine, ShardPlan, _Trace, all_reduce_sum, dist_ctx, integer_weights
+from .engine import CoverEngine, _Trace, all_reduce_sum, dist_ctx, integer_weights, local_plan
 
 CONFIG_KEYS = ("task", "seed", "display", "verbose", "scaling", "pixels", "show_logs", "save_model", "show_result")
 SILENT = bool(int(os.environ.get("PYBMF_B200_SILENT", "0")))
@@ -97,8 +97,8 @@ class BaseModel:
             _say("[W] Missing testing data.")
         # generate.DeviceBits (rows already bit-packed on the device) is passed through: Asso packs nothing and uploads nothing
         self.X_train = X_train if hasattr(X_train, "bits") else U_.to_sparse(X_train, "csr")
-        self.X_val = None if X_val is None else U_.to_sparse(X_val, "csr")
-        self.X_test = None if X_test is None else U_.to_sparse(X_test, "csr")
+        self.X_val = _split(self.X_train, X_val, getattr(self, "task", None))
+        self.X_test = _split(self.X_train, X_test, getattr(self, "task", None))
         self.m, self.n = self.X_train.shape
 
     def fit(self, X_train, X_val=None, X_test=None, **kwargs):
@@ -233,19 +233,13 @@ class BaseModel:
 
     def _split_counts(self, name):
         """(TP, FP, FN, size) of the current factors against X_<name> under self.task
-        (evaluate_utils.py:32-52); counts come from bmf_confusion_factors / _triplets."""
+        (evaluate_utils.py:32-52); counts come from bmf_confusion_factors / _triplets.  A generate.DeviceBits split is
+        counted on this rank's rows and summed over the ranks: a collective under an initialised process group."""
         X = getattr(self, "X_" + name)
+        if self.task == "reconstruction":                     # `self.task` unset -> AttributeError, as D6
+            return U_.factor_counts(X, self.U, self.V)
         Up, Vp = U_._pattern(self.U), U_._pattern(self.V)
         uw, kw = U_._factor_words(Up)
-        if self.task == "reconstruction":                     # `self.task` unset -> AttributeError, as D6
-            G = U_._pattern(X)
-            m, n = G.shape
-            counts = device.zeros((3,), torch.int64)
-            vt = U_._bits_on_device(Vp.T.tocsr())
-            _native.call("bmf_confusion_factors", U_._bits_on_device(G), m, device.words_for(n), uw, kw, vt,
-                         Up.shape[1], int(G.nnz), counts, None, None)
-            tp, fp, fn = (int(v) for v in counts.cpu().numpy())
-            return tp, fp, fn, m * n
         r, c, g = U_.to_triplet(X)
         vw, _ = U_._factor_words(Vp)
         counts = device.zeros((4,), torch.int64)
@@ -378,14 +372,28 @@ def _csr_to_lil_fast(A: csr_matrix) -> lil_matrix:
     return out
 
 
+def _split(X_train, X, task):
+    """A validation / test split as fit() keeps it: a host matrix becomes a csr; a generate.DeviceBits is passed through
+    once it is checked, on every rank and before any collective, to have X_train's shape and this rank's ShardPlan
+    rows.  task='prediction' counts stored entries (evaluate_utils.py:32-44), stored zeros included, which bit rows
+    cannot express."""
+    if X is None:
+        return None
+    if not hasattr(X, "bits"):
+        return U_.to_sparse(X, "csr")
+    if X.shape != X_train.shape:
+        raise ValueError("DeviceBits split of shape %s, X_train is %s" % (X.shape, X_train.shape))
+    local_plan(X)
+    if task == "prediction":
+        raise ValueError("task='prediction' counts stored entries; a DeviceBits split has none, use 'reconstruction'")
+    return X
+
+
 def _local_rows(X):
     """(plan, r0, r1, bit rows) of this rank's share of the training matrix under ShardPlan.  A generate.DeviceBits is
     used as it is; of a host csr only the rank's rows are packed, from a zero-copy row view."""
-    rank, world = dist_ctx()
-    plan = ShardPlan(X.shape[0], world)
-    r0, r1 = plan.rows(rank)
+    plan, r0, r1 = local_plan(X)
     if hasattr(X, "bits"):
-        assert (X.r0, X.r1) == (r0, r1), "DeviceBits rows must follow ShardPlan(m, world).rows(rank)"
         return plan, r0, r1, X.bits
     Xl = device.csr_rows_view(X, r0, r1)
     if device.has_stored_zeros(Xl):                             # the packer takes every STORED entry as a one
@@ -667,6 +675,11 @@ class Asso(BaseModel):
         # i.e. ones (TP / FN) and explicitly stored zeros (FP / TN) separately.
         cache = self.__dict__.setdefault("_dev_split_cache", {})
         key = (name, self.task)
+        if key not in cache and hasattr(X, "bits"):         # generate.DeviceBits: this rank's rows are already bit rows
+            ones = device.zeros((3,), torch.int64)
+            if dev.m_loc > 0:                                 # |split|: TP of the split against itself, once per fit
+                _native.call("bmf_confusion_bits", X.bits, X.bits, dev.m_loc, dev.words, -1, ones, None, None)
+            cache[key] = {"ones": X.bits, "n_ones": int(ones[0])}
         if key not in cache:
             Xl = device.csr_rows_view(X, dev.r0, dev.r1)
             # the common case stores no explicit zeros: then the stored pattern IS the set of ones (no 1e8-entry copies)
@@ -836,9 +849,18 @@ class TransposedModel(Asso):
         assert isinstance(self.model, BaseModel), "The model must be an instance of BaseModel."
 
     def fit(self, X_train, X_val=None, X_test=None, **kwargs):
-        X_train = X_train.T
-        X_val = X_val.T if X_val is not None else None
-        X_test = X_test.T if X_test is not None else None
+        if any(hasattr(X, "bits") for X in (X_train, X_val, X_test)):
+            # row-sharded bit rows: their X^T is re-sharded over the ranks by generate.transpose (a collective); the splits
+            # are checked first so that a bad split raises on every rank before any exchange
+            from . import generate
+            task = kwargs.get("task", getattr(self.model, "task", None))
+            X_val, X_test = _split(X_train, X_val, task), _split(X_train, X_test, task)
+            X_train, X_val, X_test = (X if X is None else generate.transpose(X) if hasattr(X, "bits") else X.T
+                                      for X in (X_train, X_val, X_test))
+        else:
+            X_train = X_train.T
+            X_val = X_val.T if X_val is not None else None
+            X_test = X_test.T if X_test is not None else None
         self.model.fit(X_train, X_val, X_test, **kwargs)
         self.U, self.V = self.model.V, self.model.U
 

@@ -114,6 +114,61 @@ def _factor_words(U: csr_matrix):
     return bits[:, :kw].contiguous(), kw
 
 
+def on_device(*mats):
+    """True when the given matrices (None skipped) are generate.DeviceBits, False when they are host matrices.  A mix is a
+    TypeError; a DeviceBits must hold this rank's ShardPlan rows (ValueError), so that a sum over the ranks counts every
+    row once."""
+    kinds = {hasattr(X, "bits") and hasattr(X, "r0") for X in mats if X is not None}
+    if len(kinds) > 1:
+        raise TypeError("cannot mix a generate.DeviceBits with a host matrix")
+    if kinds != {True}:
+        return False
+    from .engine import local_plan
+    for X in mats:
+        if X is not None:
+            local_plan(X)
+    return True
+
+
+def _bits_confusion(G, P):
+    """(TP, FP, FN) of two generate.DeviceBits with the same shape and rows, summed over the ranks (one all-reduce: a
+    collective under an initialised process group)."""
+    from .engine import all_reduce_sum
+    if G.shape != P.shape:
+        raise ValueError("shapes differ: %s and %s" % (G.shape, P.shape))
+    counts = device.zeros((3,), torch.int64)
+    if G.r1 > G.r0:
+        _native.call("bmf_confusion_bits", G.bits, P.bits, G.r1 - G.r0, G.bits.shape[1], -1, counts, None, None)
+    tp, fp, fn = (int(v) for v in all_reduce_sum(counts).cpu().numpy())
+    return tp, fp, fn
+
+
+def factor_counts(X, U, V):
+    """(TP, FP, FN, size) of X against the Boolean product U o V^T, by bmf_confusion_factors (the product is never formed).
+
+    X is a host matrix, or a generate.DeviceBits: then only this rank's rows of U are packed and the counts are summed
+    over the ranks (one all-reduce: a collective under an initialised process group)."""
+    Up, Vp = _pattern(U), _pattern(V)
+    vt = _bits_on_device(Vp.T.tocsr())
+    counts = device.zeros((3,), torch.int64)
+    if not on_device(X):
+        G = _pattern(X)
+        uw, kw = _factor_words(Up)
+        _native.call("bmf_confusion_factors", _bits_on_device(G), G.shape[0], device.words_for(G.shape[1]), uw, kw, vt,
+                     Up.shape[1], int(G.nnz), counts, None, None)
+        tp, fp, fn = (int(v) for v in counts.cpu().numpy())
+        return tp, fp, fn, G.shape[0] * G.shape[1]
+    from .engine import all_reduce_sum
+    if Up.shape[0] != X.m or Vp.shape[0] != X.n or Up.shape[1] != Vp.shape[1]:
+        raise ValueError("factors U %s and V %s do not fit X %s" % (Up.shape, Vp.shape, X.shape))
+    if X.r1 > X.r0:
+        uw, kw = _factor_words(Up[X.r0:X.r1])
+        _native.call("bmf_confusion_factors", X.bits, X.r1 - X.r0, X.bits.shape[1], uw, kw, vt, Up.shape[1], -1, counts,
+                     None, None)
+    tp, fp, fn = (int(v) for v in all_reduce_sum(counts).cpu().numpy())
+    return tp, fp, fn, X.m * X.n
+
+
 def _product_bits(U: csr_matrix, Vt: csr_matrix):
     """bits of (U o Vt) for U (m x k) and Vt (k x n) given as patterns."""
     m, k = U.shape
@@ -204,8 +259,13 @@ def get_residual(X, U, V):
 def confusion_counts(gt, pd, axis=None):
     """(TP, FP, FN) of PyBMF/utils/metrics.py:56-76 via bmf_confusion_bits.
 
-    axis=None -> three Python ints; axis=1 -> per-row int64 arrays; axis=0 -> per-column."""
+    axis=None -> three Python ints; axis=1 -> per-row int64 arrays; axis=0 -> per-column.  Two generate.DeviceBits are
+    counted on this rank's rows and summed over the ranks (axis=None only)."""
     _native.require_gpu()
+    if on_device(gt, pd):
+        if axis is not None:
+            raise NotImplementedError("per-row / per-column counts of a generate.DeviceBits are not supported")
+        return _bits_confusion(gt, pd)
     G, P = _pattern(gt), _pattern(pd)
     assert G.shape == P.shape, "U and V should have the same shape"
     if axis == 0:
@@ -319,9 +379,12 @@ def weighted_error(gt, pd, w_fp=0.5, w_fn=None, axis=None):
 
 
 def description_length(gt, U, V, pd=None, w_model=1.0, w_fp=1.0, w_fn=1.0):
-    """PyBMF/utils/metrics.py:173-179."""
-    pd = matmul(U, V.T, sparse=True, boolean=True) if pd is None else pd
-    _, fp, fn = confusion_counts(gt, pd, None)
+    """PyBMF/utils/metrics.py:173-179.  A generate.DeviceBits `gt` without `pd` is counted against the factors."""
+    if pd is None and on_device(gt):
+        _, fp, fn, _ = factor_counts(gt, U, V)
+    else:
+        pd = matmul(U, V.T, sparse=True, boolean=True) if pd is None else pd
+        _, fp, fn = confusion_counts(gt, pd, None)
     return w_model * (U.sum() + V.sum()) + w_fp * _as_count(fp) + w_fn * _as_count(fn)
 
 
@@ -340,7 +403,8 @@ def get_metrics(gt, pd, metrics, axis=None):
     """PyBMF/utils/metrics.py:8-53."""
     if axis is not None:
         raise NotImplementedError("get_metrics: only axis=None is supported")
-    if np.isnan(to_dense(pd, squeeze=True)).any() if not issparse(pd) else np.isnan(pd.data).any():
+    host_pd = not on_device(pd)                             # bit rows hold no NaN
+    if host_pd and (np.isnan(to_dense(pd, squeeze=True)).any() if not issparse(pd) else np.isnan(pd.data).any()):
         raise TypeError("NaN is found in prediction.")
     if isinstance(gt, np.ndarray) and gt.ndim == 1:        # triplet form of task='prediction'
         g = np.asarray(gt) != 0
@@ -353,12 +417,20 @@ def get_metrics(gt, pd, metrics, axis=None):
 
 def eval(metrics, task, X_gt, X_pd=None, U=None, V=None):
     """PyBMF/utils/evaluate_utils.py:12-54 -- counts on the GPU; for task='prediction' the
-    per-triplet Python loop (:41-44) becomes bmf_confusion_triplets."""
+    per-triplet Python loop (:41-44) becomes bmf_confusion_triplets.
+
+    A generate.DeviceBits `X_gt` is compared with factors `U`, `V` under task='reconstruction' only: this rank's rows
+    against this rank's rows of U, summed over the ranks (a collective under an initialised process group)."""
     using_matrix = X_pd is not None
     using_factors = U is not None and V is not None
     assert using_matrix or using_factors, "[E] User should provide either `U`, `V` or `X_pd`."
     assert task in ["prediction", "reconstruction"], "[E] Task should be either 'prediction' or 'reconstruction'."
     _native.require_gpu()
+    if on_device(X_gt):
+        if using_matrix:
+            raise TypeError("eval: a generate.DeviceBits X_gt is compared with factors U, V, not with X_pd")
+        if task != "reconstruction":
+            raise ValueError("eval: task='prediction' counts stored entries, which a generate.DeviceBits cannot hold")
     if not using_factors:
         if task == "reconstruction":
             return get_metrics(gt=to_sparse(X_gt, "csr"), pd=to_sparse(X_pd, "csr"), metrics=metrics)
@@ -366,17 +438,10 @@ def eval(metrics, task, X_gt, X_pd=None, U=None, V=None):
         P = csr_matrix(X_pd)
         pd_data = np.asarray(P[r, c]).ravel() if len(r) else np.zeros(0)
         return get_metrics(gt=g, pd=pd_data, metrics=metrics)
+    if task == "reconstruction":
+        return metrics_from_counts(metrics, *factor_counts(X_gt, U, V))
     Up, Vp = _pattern(U), _pattern(V)
     uw, kw = _factor_words(Up)
-    if task == "reconstruction":
-        G = _pattern(X_gt)
-        m, n = G.shape
-        counts = device.zeros((3,), torch.int64)
-        vt = _bits_on_device(Vp.T.tocsr())
-        _native.call("bmf_confusion_factors", _bits_on_device(G), m, device.words_for(n), uw, kw, vt, Up.shape[1],
-                     int(G.nnz), counts, None, None)
-        tp, fp, fn = (int(v) for v in counts.cpu().numpy())
-        return metrics_from_counts(metrics, tp, fp, fn, m * n)
     r, c, g = to_triplet(X_gt)
     vw, _ = _factor_words(Vp)
     counts = device.zeros((4,), torch.int64)
