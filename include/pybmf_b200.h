@@ -299,6 +299,33 @@ int bmf_confusion_triplets(const int32_t* rows, const int32_t* cols, const uint8
 int bmf_expand_scores(const uint64_t* x_bits, const uint64_t* old_bits, int64_t rows, int64_t words,
                       const uint64_t* pattern_bits, const uint64_t* exclude_bits, double w_fp, double w_fn,
                       double* delta, int64_t* best, bmf_stream_t stream);
+/* ---- GreConDPlus.expansion, PyBMF/models/GreConDPlus.py:207-264: the incremental, device-resident loop ----------
+ * Row layout only.  A rank holds rows [row0, row0 + rows) of x / old; u_bits (m bits) and v_bits (n bits) are the whole,
+ * replicated pattern.
+ * bmf_expand_init: one pass over the rows.  row_cnt[i][0..3] = (TP_old, FP_old, P, N) of local row i (int32, written)
+ * with P = |x & ~old & v|, N = |~x & ~old & v|; col_cnt[k][j] (int64 [4][n], written) = this rank's share of column j's
+ * TP_old, FP_old, and over the rows in u, P = |x & ~old| and N = |~x & ~old| (pad bits masked).  Column counts are
+ * summed over the ranks by the caller.
+ * One iteration = bmf_expand_step_rows, a SUM of xbuf over the ranks (nothing with one rank), bmf_expand_step_decide.
+ * state[8] (int64, caller-initialised to {0, -1, -1, 0, 0, 0, 0, 0}) = (stopped, row chosen last or -1, column chosen
+ * last or -1, iterations logged, two block counters).  partials: 4 * 1024 int64 scratch.  xbuf: 2 * world + 2 * words
+ * int64 = world slots (bits of the rank's max row delta, its logical row or -1) then the words of the row chosen last
+ * (x & ~old, then ~x & ~old masked to n), filled by its owner and 0 elsewhere.  step_rows applies a column chosen last to
+ * P / N of the rows and fills xbuf; step_decide applies the row in xbuf to the column counts, merges the slots (max, then
+ * the lowest row), takes the max and FIRST argmax of the column deltas and applies the reference's rule: it sets the bit in
+ * u / v and appends (0 row | 1 column | 2 stop, index) to log[log_cap][2].  Once stopped, both are no-ops.
+ * bmf_expand_col_scores: _expansion(axis = 0) from summed column counts: delta[j], best as bmf_expand_scores. */
+int bmf_expand_init(const uint64_t* x_bits, const uint64_t* old_bits, int64_t rows, int64_t n, int64_t words, int64_t row0,
+                    const uint64_t* u_bits, const uint64_t* v_bits, int32_t* row_cnt, int64_t* col_cnt,
+                    bmf_stream_t stream);
+int bmf_expand_step_rows(const uint64_t* x_bits, const uint64_t* old_bits, int64_t rows, int64_t n, int64_t words,
+                         int64_t row0, const uint64_t* u_bits, int32_t* row_cnt, double w_fp, double w_fn, int64_t* state,
+                         int64_t* partials, int64_t* xbuf, int64_t world, int64_t rank, bmf_stream_t stream);
+int bmf_expand_step_decide(int64_t* col_cnt, int64_t n, int64_t words, uint64_t* u_bits, uint64_t* v_bits, double w_fp,
+                           double w_fn, int64_t* state, int64_t* partials, const int64_t* xbuf, int64_t world,
+                           int64_t* log, int64_t log_cap, bmf_stream_t stream);
+int bmf_expand_col_scores(const int64_t* col_cnt, int64_t n, const uint64_t* v_bits, double w_fp, double w_fn,
+                          double* delta, int64_t* best, bmf_stream_t stream);
 /* ---- AssoOpt.set_optimal_row, PyBMF/models/AssoOpt.py:69-80 (SURVEY section 8f rank 4) -------------------------
  * best_trial[i] = FIRST argmax over j in [0, 2^k) of (-w_fp) FP + w_fn TP of the OR of the V^T rows selected by j
  * (factor l = bit k-1-l of j, the MSB-first order of int2bin, AssoOpt.py:83-86) against data row i; best_score

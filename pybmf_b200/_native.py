@@ -59,7 +59,11 @@ SIGNATURES = {
     "bmf_cover_rescore_i8_general": [_p, _i64, _p, _i64, _i64, _p, _p, _p, _f64, _f64, _p, _i32, _p, _p, _p],
     "bmf_basis_threshold_rows": [_p, _i64, _i64, _i64, _i64, _i32, _f64, _p, _i64, _p, _p, _p],
     "bmf_expand_scores": [_p, _p, _i64, _i64, _p, _p, _f64, _f64, _p, _p, _p],
-    "bmf_optimal_rows": [_p, _i64, _i64, _p, _i64, _f64, _f64, _p, _p, _p],
+    "bmf_expand_init": [_p, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p],
+    "bmf_expand_step_rows": [_p, _p, _i64, _i64, _i64, _i64, _p, _p, _f64, _f64, _p, _p, _p, _i64, _i64, _p],
+    "bmf_expand_step_decide": [_p, _i64, _i64, _p, _p, _f64, _f64, _p, _p, _p, _i64, _p, _i64, _p],
+    "bmf_expand_col_scores": [_p, _i64, _p, _f64, _f64, _p, _p, _p],
+    "bmf_optimal_rows":[_p, _i64, _i64, _p, _i64, _f64, _f64, _p, _p, _p],
     "bmf_random_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, C.c_uint64, _f64, _p],
     "bmf_noise_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, _f64, _f64, _p],
     "bmf_transpose_bits": [_p, _i64, _i64, _i64, _p, _i64, _p],

@@ -2189,6 +2189,304 @@ __global__ void __launch_bounds__(1024) argmax_first_f64_kernel(const double* __
 }
 
 // =========================================================================================
+// Incremental GreConD+ expansion (GreConDPlus.py:207-264, `expansion`).  X_old is fixed for the whole loop, so the
+// per-row TP_old / FP_old and the per-column TP_old / FP_old never change, and one iteration changes the increments by
+// one bit per row (a column c joined v) or by one row's bits per column (a row r joined u).  One streaming pass
+// (expand_init_kernel) produces every count; an iteration then costs O(m + n) (expand_step_rows_kernel,
+// expand_step_decide_kernel), with the deltas evaluated from the same integers by the same fp64 expression as
+// expand_delta_kernel, so they are bit-identical.
+// =========================================================================================
+
+// (max, FIRST argmax) merge: a candidate with a lower index wins a tie; idx < 0 is "no candidate"
+__device__ __forceinline__ void better_first(double& best, long long& idx, double v, long long i) {
+  if (i >= 0 && (idx < 0 || v > best || (v == best && i < idx))) { best = v; idx = i; }
+}
+
+// block-wide better_first (every thread returns the block's result); blockDim.x = 256
+__device__ __forceinline__ void block_first_max(double& best, long long& idx) {
+  __shared__ double s_val[8];
+  __shared__ long long s_idx[8];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1)
+    better_first(best, idx, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, idx, o));
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  __syncthreads();
+  if (lane == 0) { s_val[warp] = best; s_idx[warp] = idx; }
+  __syncthreads();
+  best = s_val[0];
+  idx = s_idx[0];
+  for (int q = 1; q < 8; ++q) better_first(best, idx, s_val[q], s_idx[q]);
+}
+
+// Every block stores its (max, argmax) in partials[blockIdx.x]; the block that arrives last returns true with the
+// grid's result in (best, idx) and re-arms the counter for the next launch.
+__device__ __forceinline__ bool grid_first_max(double& best, long long& idx, long long* __restrict__ partials,
+                                               unsigned long long* counter) {
+  __shared__ int s_last;
+  block_first_max(best, idx);
+  if (threadIdx.x == 0) {
+    partials[2 * blockIdx.x] = __double_as_longlong(best);
+    partials[2 * blockIdx.x + 1] = idx;
+    __threadfence();
+    s_last = atomicAdd(counter, 1ull) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!s_last) return false;
+  __threadfence();
+  best = 0.0;
+  idx = -1;
+  for (int b = threadIdx.x; b < (int)gridDim.x; b += blockDim.x)
+    better_first(best, idx, __longlong_as_double(__ldcg(partials + 2 * b)), __ldcg(partials + 2 * b + 1));
+  block_first_max(best, idx);
+  if (threadIdx.x == 0) *counter = 0ull;
+  return true;
+}
+
+// Bit-sliced (positional) counter of 64 columns: value of column c = sum_b bit c of plane b * 2^b.  Eight one-bit
+// inputs enter a carry-save tree (ones / twos / fours, Harley-Seal); its carry of weight 8 ripples into the planes hi.
+constexpr int kExpandHiPlanes = 8;                                   // <= 255 groups of 8 rows between two flushes
+constexpr int kExpandRowsPerWarp = 1024;
+struct PosCount {
+  uint64_t ones, twos, fours, hi[kExpandHiPlanes];
+  __device__ __forceinline__ void clear() {
+    ones = twos = fours = 0ull;
+#pragma unroll
+    for (int b = 0; b < kExpandHiPlanes; ++b) hi[b] = 0ull;
+  }
+  __device__ __forceinline__ void add8(const uint64_t (&a)[8]) {
+    uint64_t tA, tB, fA, fB, e;
+    csa64(tA, ones, ones, a[0], a[1]);
+    csa64(tB, ones, ones, a[2], a[3]);
+    csa64(fA, twos, twos, tA, tB);
+    csa64(tA, ones, ones, a[4], a[5]);
+    csa64(tB, ones, ones, a[6], a[7]);
+    csa64(fB, twos, twos, tA, tB);
+    csa64(e, fours, fours, fA, fB);
+#pragma unroll
+    for (int b = 0; b < kExpandHiPlanes; ++b) {
+      const uint64_t c = hi[b] & e;
+      hi[b] ^= e;
+      e = c;
+    }
+  }
+  __device__ __forceinline__ unsigned value(int c) const {
+    unsigned v = (unsigned)((ones >> c) & 1ull) | ((unsigned)((twos >> c) & 1ull) << 1) |
+                 ((unsigned)((fours >> c) & 1ull) << 2);
+#pragma unroll
+    for (int b = 0; b < kExpandHiPlanes; ++b) v |= (unsigned)((hi[b] >> c) & 1ull) << (3 + b);
+    return v;
+  }
+};
+
+// One pass over rows [0, rows) of x / old (logical rows row0 + i).  Block (bx, by) covers words [32 bx, 32 bx + 32) of
+// rows [8 rpw by, 8 rpw (by + 1)); warp q of the block the rows [rpw q, rpw (q + 1)) of that range, lane l word 32 bx + l.
+//   row_cnt[i] = (TP_old, FP_old, P, N) += this window's share (two 64-bit atomics per row and window), P / N against v;
+//   col_cnt[k][j] += counter k of column j over the block's rows: TP_old (x & old), FP_old (~x & old), and over the rows in
+//   u: P (x & ~old), N (~x & ~old, pad bits masked).  Lanes count their 64 columns in PosCount registers, flush them
+//   into the block's shared table once per warp and the block adds the table to col_cnt once.
+__global__ void __launch_bounds__(256)
+expand_init_kernel(const uint64_t* __restrict__ xb, const uint64_t* __restrict__ ob, int64_t rows, int64_t n,
+                   int64_t words, int64_t row0, const uint64_t* __restrict__ u, const uint64_t* __restrict__ v,
+                   int32_t* __restrict__ row_cnt, unsigned long long* __restrict__ col_cnt, int64_t rpw) {
+  __shared__ unsigned s_cnt[4][64][32];                             // [counter][bit][lane]: conflict-free flushes
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t w0 = (int64_t)blockIdx.x * 32, w = w0 + lane;
+  const bool active = w < words;
+  const int64_t valid_bits = n - w * 64;
+  const uint64_t colmask = !active || valid_bits <= 0 ? 0ull : valid_bits >= 64 ? ~0ull : (1ull << valid_bits) - 1ull;
+  const uint64_t vw = active ? v[w] : 0ull;
+  for (int e = threadIdx.x; e < 4 * 64 * 32; e += 256) (&s_cnt[0][0][0])[e] = 0u;
+  __syncthreads();
+  const int64_t rb = ((int64_t)blockIdx.y * 8 + warp) * rpw;
+  const int64_t re = rb + rpw < rows ? rb + rpw : rows;
+  if (rb < re) {
+    PosCount ctp, cfp, cP, cN;
+    ctp.clear(); cfp.clear(); cP.clear(); cN.clear();
+    for (int64_t i0 = rb; i0 < re; i0 += 8) {
+      uint64_t xw[8], ow[8], um[8];
+#pragma unroll
+      for (int q = 0; q < 8; ++q) {
+        const int64_t i = i0 + q;
+        const bool ok = i < re;
+        xw[q] = ok && active ? __ldg(xb + i * words + w) : 0ull;
+        ow[q] = ok && active ? __ldg(ob + i * words + w) : 0ull;
+        const int64_t g = row0 + i;
+        um[q] = ok ? 0ull - ((__ldg(u + (g >> 6)) >> (g & 63)) & 1ull) : 0ull;
+      }
+#pragma unroll
+      for (int q = 0; q < 8; ++q) {
+        unsigned t = (unsigned)__popcll(xw[q] & ow[q]) | ((unsigned)__popcll(~xw[q] & ow[q]) << 16);
+        unsigned p = (unsigned)__popcll(xw[q] & ~ow[q] & vw) | ((unsigned)__popcll(~xw[q] & ~ow[q] & vw) << 16);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          t += __shfl_xor_sync(0xffffffffu, t, o);
+          p += __shfl_xor_sync(0xffffffffu, p, o);
+        }
+        const int64_t i = i0 + q;
+        if (lane == 0 && i < re) {                                   // (TP, FP) and (P, N): one 64-bit add each
+          unsigned long long* rc = reinterpret_cast<unsigned long long*>(row_cnt + 4 * i);
+          if (t) atomicAdd(rc, (unsigned long long)(t & 0xffffu) | ((unsigned long long)(t >> 16) << 32));
+          if (p) atomicAdd(rc + 1, (unsigned long long)(p & 0xffffu) | ((unsigned long long)(p >> 16) << 32));
+        }
+      }
+      uint64_t a[8];
+#pragma unroll
+      for (int q = 0; q < 8; ++q) a[q] = xw[q] & ow[q];
+      ctp.add8(a);
+#pragma unroll
+      for (int q = 0; q < 8; ++q) a[q] = ~xw[q] & ow[q];
+      cfp.add8(a);
+#pragma unroll
+      for (int q = 0; q < 8; ++q) a[q] = xw[q] & ~ow[q] & um[q];
+      cP.add8(a);
+#pragma unroll
+      for (int q = 0; q < 8; ++q) a[q] = ~xw[q] & ~ow[q] & um[q] & colmask;
+      cN.add8(a);
+    }
+    if (active) {
+      for (int c = 0; c < 64; ++c) {
+        unsigned val;
+        if ((val = ctp.value(c))) atomicAdd(&s_cnt[0][c][lane], val);
+        if ((val = cfp.value(c))) atomicAdd(&s_cnt[1][c][lane], val);
+        if ((val = cP.value(c))) atomicAdd(&s_cnt[2][c][lane], val);
+        if ((val = cN.value(c))) atomicAdd(&s_cnt[3][c][lane], val);
+      }
+    }
+  }
+  __syncthreads();
+  for (int e = threadIdx.x; e < 4 * 64 * 32; e += 256) {
+    const int k = e >> 11, c = (e >> 5) & 63, l = e & 31;
+    const int64_t j = (w0 + l) * 64 + c;
+    const unsigned val = s_cnt[k][c][l];
+    if (val && j < n) atomicAdd(col_cnt + k * n + j, (unsigned long long)val);
+  }
+}
+
+// Iteration, part 1 (grid over the rank's rows).  A column c chosen by the previous decision adds bit c of x & ~old /
+// ~x & ~old to every row's P / N; every row's delta is evaluated (+0.0 in u) and the last block writes the exchange
+// buffer: slot `rank` = (bits of the local max, its logical row), every other slot 0, and the words of the row r chosen by
+// the previous decision (x & ~old, ~x & ~old masked to n) if this rank owns r, else 0.  No-op but for zeroing the buffer
+// once state[0] (stopped) is set.
+__global__ void __launch_bounds__(256)
+expand_step_rows_kernel(const uint64_t* __restrict__ xb, const uint64_t* __restrict__ ob, int64_t rows, int64_t n,
+                        int64_t words, int64_t row0, const uint64_t* __restrict__ u, int32_t* __restrict__ row_cnt,
+                        double neg_w_fp, double w_fn, long long* __restrict__ state, long long* __restrict__ partials,
+                        long long* __restrict__ xbuf, int64_t world, int64_t rank) {
+  const int64_t buf_len = 2 * world + 2 * words;
+  if (state[0]) {
+    if (blockIdx.x == 0)
+      for (int64_t e = threadIdx.x; e < buf_len; e += blockDim.x) xbuf[e] = 0;
+    return;
+  }
+  const long long c = state[2];
+  double best = 0.0;
+  long long idx = -1;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < rows; i += (int64_t)gridDim.x * blockDim.x) {
+    int4 cnt = reinterpret_cast<const int4*>(row_cnt)[i];
+    if (c >= 0) {
+      const uint64_t bit = 1ull << (c & 63);
+      const uint64_t xw = xb[i * words + (c >> 6)], ow = ob[i * words + (c >> 6)];
+      if (!(ow & bit)) {
+        if (xw & bit) row_cnt[4 * i + 2] = ++cnt.z;
+        else row_cnt[4 * i + 3] = ++cnt.w;
+      }
+    }
+    const int64_t g = row0 + i;
+    double d = 0.0;
+    if (!((u[g >> 6] >> (g & 63)) & 1ull)) {
+      const double s_old = cover_score_f64(neg_w_fp, w_fn, cnt.y, cnt.x);
+      const double s_new = cover_score_f64(neg_w_fp, w_fn, cnt.y + cnt.w, cnt.x + cnt.z);
+      d = __dsub_rn(s_new, s_old);
+    }
+    better_first(best, idx, d, g);
+  }
+  if (!grid_first_max(best, idx, partials, reinterpret_cast<unsigned long long*>(state + 4))) return;
+  const long long r = state[1];
+  const bool own = r >= row0 && r < row0 + rows;
+  for (int64_t e = threadIdx.x; e < buf_len; e += blockDim.x) {
+    long long val = 0;
+    if (e == 2 * rank) val = __double_as_longlong(best);
+    else if (e == 2 * rank + 1) val = idx;
+    else if (e >= 2 * world && own) {
+      const int64_t wq = (e - 2 * world) % words;
+      const uint64_t xw = xb[(r - row0) * words + wq], ow = ob[(r - row0) * words + wq];
+      const int64_t valid_bits = n - wq * 64;
+      const uint64_t mask = valid_bits <= 0 ? 0ull : valid_bits >= 64 ? ~0ull : (1ull << valid_bits) - 1ull;
+      val = (long long)(e < 2 * world + words ? xw & ~ow : ~xw & ~ow & mask);
+    }
+    xbuf[e] = val;
+  }
+}
+
+// Iteration, part 2 (grid over the columns; after the buffers of all ranks were summed).  The row r chosen by the
+// previous decision adds its words to every column's P / N; every column's delta is evaluated (+0.0 in v); the last block
+// merges the rank slots (max, then the lowest logical row) and applies the reference's rule (GreConDPlus.py:221-236):
+// a row if r_score > c_score and r_score > 0, a column if c_score > r_score and c_score > 0, else stop.  It sets the bit
+// in u / v, appends (0 row | 1 column | 2 stop, index) to the log and updates state.
+__global__ void __launch_bounds__(256)
+expand_step_decide_kernel(long long* __restrict__ col_cnt, int64_t n, int64_t words, uint64_t* __restrict__ u,
+                          uint64_t* __restrict__ v, double neg_w_fp, double w_fn, long long* __restrict__ state,
+                          long long* __restrict__ partials, const long long* __restrict__ xbuf, int64_t world,
+                          long long* __restrict__ log, int64_t log_cap) {
+  if (state[0]) return;
+  const long long r = state[1];
+  const uint64_t* rp = reinterpret_cast<const uint64_t*>(xbuf + 2 * world);
+  const uint64_t* rn = rp + words;
+  double best = 0.0;
+  long long idx = -1;
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+    const long long tp = col_cnt[j], fp = col_cnt[n + j];
+    long long P = col_cnt[2 * n + j], N = col_cnt[3 * n + j];
+    if (r >= 0) {
+      if ((rp[j >> 6] >> (j & 63)) & 1ull) col_cnt[2 * n + j] = ++P;
+      if ((rn[j >> 6] >> (j & 63)) & 1ull) col_cnt[3 * n + j] = ++N;
+    }
+    double d = 0.0;
+    if (!((v[j >> 6] >> (j & 63)) & 1ull)) {
+      const double s_old = cover_score_f64(neg_w_fp, w_fn, (int)fp, (int)tp);
+      const double s_new = cover_score_f64(neg_w_fp, w_fn, (int)(fp + N), (int)(tp + P));
+      d = __dsub_rn(s_new, s_old);
+    }
+    better_first(best, idx, d, j);
+  }
+  if (!grid_first_max(best, idx, partials, reinterpret_cast<unsigned long long*>(state + 5))) return;
+  if (threadIdx.x != 0) return;
+  double r_score = 0.0;
+  long long r_index = -1;
+  for (int64_t q = 0; q < world; ++q) better_first(r_score, r_index, __longlong_as_double(xbuf[2 * q]), xbuf[2 * q + 1]);
+  const long long t = state[3];
+  long long kind = 2, at = -1;
+  if (r_score > best && r_score > 0.0) {
+    kind = 0; at = r_index;
+    u[r_index >> 6] |= 1ull << (r_index & 63);
+    state[1] = r_index; state[2] = -1;
+  } else if (best > r_score && best > 0.0) {
+    kind = 1; at = idx;
+    v[idx >> 6] |= 1ull << (idx & 63);
+    state[1] = -1; state[2] = idx;
+  } else {
+    state[0] = 1;
+  }
+  if (t < log_cap) { log[2 * t] = kind; log[2 * t + 1] = at; }
+  state[3] = t + 1;
+}
+
+// column deltas of _expansion(axis = 0) from the column counts: delta[j] = +0.0 for j in v
+__global__ void __launch_bounds__(256)
+expand_col_delta_kernel(const long long* __restrict__ col_cnt, int64_t n, const uint64_t* __restrict__ v, double neg_w_fp,
+                        double w_fn, double* __restrict__ delta) {
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+    double d = 0.0;
+    if (!((v[j >> 6] >> (j & 63)) & 1ull)) {
+      const long long tp = col_cnt[j], fp = col_cnt[n + j], P = col_cnt[2 * n + j], N = col_cnt[3 * n + j];
+      d = __dsub_rn(cover_score_f64(neg_w_fp, w_fn, (int)(fp + N), (int)(tp + P)),
+                    cover_score_f64(neg_w_fp, w_fn, (int)fp, (int)tp));
+    }
+    delta[j] = d;
+  }
+}
+
+// =========================================================================================
 // AssoOpt.set_optimal_row (PyBMF/models/AssoOpt.py:69-80): for data row i try all 2^k usage vectors, the score of trial
 // j is (-w_fp) FP + w_fn TP of  OR_{l in bits(j)} V^T_l  against x_i, and the FIRST maximum wins (np.argmax).
 // int2bin (AssoOpt.py:83-86) writes j MSB first, so factor l is bit (k - 1 - l) of j.
@@ -2913,6 +3211,78 @@ extern "C" int bmf_expand_scores(const uint64_t* x_bits, const uint64_t* old_bit
     argmax_first_f64_kernel<<<1, 1024, 0, as_stream(stream)>>>(delta, rows, reinterpret_cast<long long*>(best));
     BMF_LAUNCH_CHECK("bmf_expand_scores");
   }
+  return 0;
+}
+
+static constexpr int64_t kExpandMaxBlocks = 1024;                   // grid of the step kernels (partials: 2 x 1024 pairs)
+
+extern "C" int bmf_expand_init(const uint64_t* x_bits, const uint64_t* old_bits, int64_t rows, int64_t n, int64_t words,
+                               int64_t row0, const uint64_t* u_bits, const uint64_t* v_bits, int32_t* row_cnt,
+                               int64_t* col_cnt, bmf_stream_t stream) {
+  BMF_REQUIRE(u_bits && v_bits && col_cnt && (rows == 0 || (x_bits && old_bits && row_cnt)), "bmf_expand_init: null pointer");
+  BMF_REQUIRE(rows >= 0 && n > 0 && words * 64 >= n && words % 2 == 0 && row0 >= 0 && row0 + rows < (1ll << 31),
+              "bmf_expand_init: bad shape");
+  cudaStream_t s = as_stream(stream);
+  int rc = check_cuda(cudaMemsetAsync(col_cnt, 0, (size_t)(4 * n) * sizeof(int64_t), s), "bmf_expand_init");
+  if (rc || rows == 0) return rc;
+  rc = check_cuda(cudaMemsetAsync(row_cnt, 0, (size_t)(4 * rows) * sizeof(int32_t), s), "bmf_expand_init");
+  if (rc) return rc;
+  // rows per warp: about four blocks per SM in all, at most kExpandRowsPerWarp (the PosCount planes' range)
+  const int64_t windows = ceil_div(words, 32);
+  int64_t rpw = ceil_div(ceil_div(rows * windows, (int64_t)num_sms() * 4 * 8), 8) * 8;
+  rpw = rpw < 8 ? 8 : rpw > kExpandRowsPerWarp ? kExpandRowsPerWarp : rpw;
+  const int64_t row_blocks = ceil_div(rows, 8 * rpw);
+  BMF_REQUIRE(windows <= 0x7fffffff && row_blocks <= 65535, "bmf_expand_init: matrix too large for one launch");
+  dim3 grid((unsigned)windows, (unsigned)row_blocks);
+  expand_init_kernel<<<grid, 256, 0, s>>>(x_bits, old_bits, rows, n, words, row0, u_bits, v_bits, row_cnt,
+                                          reinterpret_cast<unsigned long long*>(col_cnt), rpw);
+  BMF_LAUNCH_CHECK("bmf_expand_init");
+  return 0;
+}
+
+extern "C" int bmf_expand_step_rows(const uint64_t* x_bits, const uint64_t* old_bits, int64_t rows, int64_t n,
+                                    int64_t words, int64_t row0, const uint64_t* u_bits, int32_t* row_cnt, double w_fp,
+                                    double w_fn, int64_t* state, int64_t* partials, int64_t* xbuf, int64_t world,
+                                    int64_t rank, bmf_stream_t stream) {
+  BMF_REQUIRE(u_bits && state && partials && xbuf && (rows == 0 || (x_bits && old_bits && row_cnt)),
+              "bmf_expand_step_rows: null pointer");
+  BMF_REQUIRE(rows >= 0 && n > 0 && words * 64 >= n && world >= 1 && rank >= 0 && rank < world,
+              "bmf_expand_step_rows: bad arguments");
+  int64_t blocks = ceil_div(rows, 256);
+  blocks = blocks < 1 ? 1 : blocks > kExpandMaxBlocks ? kExpandMaxBlocks : blocks;
+  expand_step_rows_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(
+      x_bits, old_bits, rows, n, words, row0, u_bits, row_cnt, -w_fp, w_fn, reinterpret_cast<long long*>(state),
+      reinterpret_cast<long long*>(partials), reinterpret_cast<long long*>(xbuf), world, rank);
+  BMF_LAUNCH_CHECK("bmf_expand_step_rows");
+  return 0;
+}
+
+extern "C" int bmf_expand_step_decide(int64_t* col_cnt, int64_t n, int64_t words, uint64_t* u_bits, uint64_t* v_bits,
+                                      double w_fp, double w_fn, int64_t* state, int64_t* partials, const int64_t* xbuf,
+                                      int64_t world, int64_t* log, int64_t log_cap, bmf_stream_t stream) {
+  BMF_REQUIRE(col_cnt && u_bits && v_bits && state && partials && xbuf && log, "bmf_expand_step_decide: null pointer");
+  BMF_REQUIRE(n > 0 && words * 64 >= n && world >= 1 && log_cap >= 0, "bmf_expand_step_decide: bad arguments");
+  int64_t blocks = ceil_div(n, 256);
+  blocks = blocks > kExpandMaxBlocks ? kExpandMaxBlocks : blocks;
+  expand_step_decide_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(
+      reinterpret_cast<long long*>(col_cnt), n, words, u_bits, v_bits, -w_fp, w_fn, reinterpret_cast<long long*>(state),
+      reinterpret_cast<long long*>(partials) + 2 * kExpandMaxBlocks, reinterpret_cast<const long long*>(xbuf), world,
+      reinterpret_cast<long long*>(log), log_cap);
+  BMF_LAUNCH_CHECK("bmf_expand_step_decide");
+  return 0;
+}
+
+extern "C" int bmf_expand_col_scores(const int64_t* col_cnt, int64_t n, const uint64_t* v_bits, double w_fp, double w_fn,
+                                     double* delta, int64_t* best, bmf_stream_t stream) {
+  BMF_REQUIRE(col_cnt && v_bits && delta && best, "bmf_expand_col_scores: null pointer");
+  BMF_REQUIRE(n > 0, "bmf_expand_col_scores: bad shape");
+  int64_t blocks = ceil_div(n, 256);
+  if (blocks > row_stream_grid()) blocks = row_stream_grid();
+  expand_col_delta_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(reinterpret_cast<const long long*>(col_cnt), n,
+                                                                         v_bits, -w_fp, w_fn, delta);
+  BMF_LAUNCH_CHECK("bmf_expand_col_scores");
+  argmax_first_f64_kernel<<<1, 1024, 0, as_stream(stream)>>>(delta, n, reinterpret_cast<long long*>(best));
+  BMF_LAUNCH_CHECK("bmf_expand_col_scores");
   return 0;
 }
 
