@@ -280,6 +280,15 @@ int bmf_confusion_factors(const uint64_t* gt_bits, int64_t m, int64_t words, con
 int bmf_confusion_bits(const uint64_t* gt_bits, const uint64_t* pd_bits, int64_t m, int64_t words,
                        int64_t gt_ones, int64_t* counts, int32_t* row_tp, int32_t* row_fp,
                        bmf_stream_t stream);
+/* Stored-entry counts of evaluate_utils.py:32-44 (task='prediction') in ONE pass: ones = the stored non-zeros, zeros
+ * (nullable) = the explicitly stored zeros, both [m][words] like pd_bits; counts[0..3] = (|ones & pd|, |zeros & pd|,
+ * |ones|, |zeros|) (overwritten), so TP = counts[0], FP = counts[1], FN = counts[2] - TP, size = counts[2] + counts[3].
+ * _factors computes the product of the factors once for both streams (panel-list form for k <= 64, row stream above). */
+int bmf_confusion_entries_bits(const uint64_t* ones, const uint64_t* zeros, const uint64_t* pd_bits, int64_t m,
+                               int64_t words, int64_t* counts, bmf_stream_t stream);
+int bmf_confusion_entries_factors(const uint64_t* ones, const uint64_t* zeros, int64_t m, int64_t words,
+                                  const uint64_t* u_words, int64_t kw, const uint64_t* vt_bits, int64_t k,
+                                  int64_t* counts, bmf_stream_t stream);
 /* add(boolean=True) / multiply(boolean=True), PyBMF/utils/boolean_utils.py:87-107 / 6-33, and the
  * residual X AND NOT C of get_residual (PyBMF/utils/common.py:154-160):
  * out = a OR b (op 0), a AND b (op 1), a AND NOT b (op 2) on [rows][words] bit matrices. */
@@ -349,6 +358,16 @@ int bmf_noise_bits(uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, i
                    double p_neg, bmf_stream_t stream);
 int bmf_transpose_bits(const uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, uint64_t* bits_t,
                        int64_t words_t, bmf_stream_t stream);
+/* bmf_split_bits: generate.ratio_split in one pass over x (rows [row0, row0 + rows) of an ncols-column matrix).  A one at
+ * global bit index b = (row * ceil(ncols / 64) + w) * 64 + bit draws u = 32-bit half (b & 1) of
+ * splitmix64(key(seed, stream_ones) + b / 2), the draw of bmf_random_bits, and goes to val ones if u < t_v, to test ones
+ * if u < t_v + t_t, else to train; a zero inside the ncols columns draws from stream_zeros and becomes a val zero if
+ * u < q_v, a test zero if u < q_v + q_t, else nothing.  Thresholds are 32-bit (p * 2^32, as bmf_random_bits).  out_bits
+ * = 5 consecutive [rows][words] matrices: train, val ones, val zeros, test ones, test zeros; every word is written and
+ * pad bits are zero. */
+int bmf_split_bits(const uint64_t* x_bits, int64_t rows, int64_t ncols, int64_t words, int64_t row0, uint64_t seed,
+                   uint64_t stream_ones, uint64_t stream_zeros, uint64_t t_v, uint64_t t_t, uint64_t q_v, uint64_t q_t,
+                   uint64_t* out_bits, bmf_stream_t stream);
 
 /* ---- measurement aid (bench.py): tensor-pipe ceiling measured on the box -----------------------------------
  * One launch in which a CTA pair per TPC issues iters x 4 back-to-back tcgen05.mma instructions of the production shape

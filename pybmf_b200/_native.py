@@ -46,6 +46,8 @@ SIGNATURES = {
     "bmf_bool_product": [_p, _i64, _i64, _p, _i64, _i64, _p, _p],
     "bmf_confusion_factors": [_p, _i64, _i64, _p, _i64, _p, _i64, _i64, _p, _p, _p, _p],
     "bmf_confusion_bits": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p],
+    "bmf_confusion_entries_bits": [_p, _p, _p, _i64, _i64, _p, _p],
+    "bmf_confusion_entries_factors": [_p, _p, _i64, _i64, _p, _i64, _p, _i64, _p, _p],
     "bmf_bits_combine": [_p, _p, _i64, _i64, C.c_int, _p, _p],
     "bmf_confusion_triplets": [_p, _p, _p, _i64, _p, _i64, _p, _p, _p],
     "bmf_greedy_select": [_p, _p, _p, _p, _p, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _p, _p, _p, _p, _p, _p],
@@ -67,6 +69,8 @@ SIGNATURES = {
     "bmf_random_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, C.c_uint64, _f64, _p],
     "bmf_noise_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, _f64, _f64, _p],
     "bmf_transpose_bits": [_p, _i64, _i64, _i64, _p, _i64, _p],
+    "bmf_split_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64,
+                       C.c_uint64, _p, _p],
     "bmf_probe_mma_rate": [_i32, _i32, _p, _p],
     "bmf_refine_column": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
     "bmf_refine_sweep": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],

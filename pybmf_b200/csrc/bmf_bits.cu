@@ -1086,27 +1086,37 @@ bool_product_kernel(const uint64_t* __restrict__ u_words, int64_t m, int64_t kw,
 // (the number of stored ones, free on the host) or counted (COUNT_GT).  The integer (POPC/ALU) pipe is
 // the busiest unit of this kernel, so the main loop runs without bounds checks on whole groups of
 // 4 x 32 pairs with pointer increments, and a checked tail handles the last < 128 pairs of a row.
-template <bool FROM_FACTORS, bool COUNT_GT>
+// ENTRIES (stored-entry counts, task='prediction'): gt holds the stored ones and zt (nullable) the explicitly stored
+// zeros; counts[0..3] += (|gt & pd|, |zt & pd|, |gt|, |zt|) in the same single pass (COUNT_GT must be set).
+template <bool FROM_FACTORS, bool COUNT_GT, bool ENTRIES = false>
 __global__ void __launch_bounds__(256)
-confusion_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ pd_bits, int64_t m,
-                 int64_t words, const uint64_t* __restrict__ u_words, int64_t kw,
+confusion_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ zt, const uint64_t* __restrict__ pd_bits,
+                 int64_t m, int64_t words, const uint64_t* __restrict__ u_words, int64_t kw,
                  const uint64_t* __restrict__ vt, unsigned long long* __restrict__ counts,
                  int32_t* __restrict__ row_tp, int32_t* __restrict__ row_fp) {
+  static_assert(!ENTRIES || COUNT_GT, "stored-entry counts count |gt|");
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
   const int64_t pairs = words >> 1;
   const int64_t full = pairs / (32 * PU);                    // unchecked groups per row
-  long long t_tp = 0, t_pd = 0, t_gt = 0;
+  const bool has_z = ENTRIES && zt != nullptr;
+  long long t_tp = 0, t_pd = 0, t_gt = 0, t_z = 0;
   for (int64_t i = warp0; i < m; i += nwarps) {
-    int tp = 0, np = 0, ng = 0;
+    int tp = 0, np = 0, ng = 0, nz = 0;
     const ulonglong2* gp = reinterpret_cast<const ulonglong2*>(gt + i * words) + lane;
+    const ulonglong2* zp = has_z ? reinterpret_cast<const ulonglong2*>(zt + i * words) + lane : nullptr;
     const ulonglong2* dp = FROM_FACTORS ? nullptr : reinterpret_cast<const ulonglong2*>(pd_bits + i * words) + lane;
     const uint64_t* uw = FROM_FACTORS ? u_words + i * kw : nullptr;
     for (int64_t it = 0; it < full; ++it) {
-      ulonglong2 g[PU], d[PU];
+      ulonglong2 g[PU], d[PU], z[PU];
 #pragma unroll
       for (int u = 0; u < PU; ++u) g[u] = __ldcs(gp + 32 * u);
+      if (has_z) {
+#pragma unroll
+        for (int u = 0; u < PU; ++u) z[u] = __ldcs(zp + 32 * u);
+        zp += 32 * PU;
+      }
       if (!FROM_FACTORS) {
 #pragma unroll
         for (int u = 0; u < PU; ++u) d[u] = __ldcs(dp + 32 * u);
@@ -1133,21 +1143,27 @@ confusion_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ p
 #pragma unroll
       for (int u = 0; u < PU; ++u) {
         tp += __popcll(g[u].x & d[u].x) + __popcll(g[u].y & d[u].y);
-        np += __popcll(d[u].x) + __popcll(d[u].y);
+        if (!ENTRIES) np += __popcll(d[u].x) + __popcll(d[u].y);
         if (COUNT_GT) ng += __popcll(g[u].x) + __popcll(g[u].y);
+        if (has_z) {
+          np += __popcll(z[u].x & d[u].x) + __popcll(z[u].y & d[u].y);
+          nz += __popcll(z[u].x) + __popcll(z[u].y);
+        }
       }
     }
     {                                                         // checked tail
       const int64_t p0 = full * (32 * PU) + lane;
       if (full * (32 * PU) < pairs) {
-        ulonglong2 g[PU], d[PU];
+        ulonglong2 g[PU], d[PU], z[PU];
 #pragma unroll
         for (int u = 0; u < PU; ++u) {
           const int64_t p = p0 + 32 * u;
           g[u] = make_ulonglong2(0ull, 0ull);
           d[u] = make_ulonglong2(0ull, 0ull);
+          z[u] = make_ulonglong2(0ull, 0ull);
           if (p < pairs) {
             g[u] = __ldcs(reinterpret_cast<const ulonglong2*>(gt + i * words + 2 * p));
+            if (has_z) z[u] = __ldcs(reinterpret_cast<const ulonglong2*>(zt + i * words + 2 * p));
             if (!FROM_FACTORS) d[u] = __ldcs(reinterpret_cast<const ulonglong2*>(pd_bits + i * words + 2 * p));
           }
         }
@@ -1155,18 +1171,23 @@ confusion_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ p
 #pragma unroll
         for (int u = 0; u < PU; ++u) {
           tp += __popcll(g[u].x & d[u].x) + __popcll(g[u].y & d[u].y);
-          np += __popcll(d[u].x) + __popcll(d[u].y);
+          if (!ENTRIES) np += __popcll(d[u].x) + __popcll(d[u].y);
           if (COUNT_GT) ng += __popcll(g[u].x) + __popcll(g[u].y);
+          if (has_z) {
+            np += __popcll(z[u].x & d[u].x) + __popcll(z[u].y & d[u].y);
+            nz += __popcll(z[u].x) + __popcll(z[u].y);
+          }
         }
       }
     }
     tp = warp_sum(tp);
     np = warp_sum(np);
     if (COUNT_GT) ng = warp_sum(ng);
+    if (has_z) nz = warp_sum(nz);
     if (lane == 0) {
       if (row_tp != nullptr) row_tp[i] = tp;
       if (row_fp != nullptr) row_fp[i] = np - tp;
-      t_tp += tp; t_pd += np; t_gt += ng;
+      t_tp += tp; t_pd += np; t_gt += ng; t_z += nz;
     }
   }
   if (lane == 0 && (t_pd | t_gt)) {
@@ -1174,6 +1195,7 @@ confusion_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ p
     atomicAdd(counts + 1, (unsigned long long)t_pd);
     if (COUNT_GT) atomicAdd(counts + 2, (unsigned long long)t_gt);
   }
+  if (ENTRIES && lane == 0 && t_z) atomicAdd(counts + 3, (unsigned long long)t_z);
 }
 
 // =========================================================================================
@@ -1596,11 +1618,18 @@ bool_product_panel_kernel(const uint64_t* __restrict__ u_words, int64_t m, const
 }
 
 // The selection-list forms of the two panel kernels (see pack_selection above): same grid, same ring, same results.
-template <bool COUNT_GT, int MODE>
+// ENTRIES (stored-entry counts, task='prediction'): gt holds the stored ones and zt (nullable) the explicitly stored
+// zeros, counts[0..3] += (|gt & pd|, |zt & pd|, |gt|, |zt|), the product computed once for both.  A row's zeros segment
+// takes the ring slot after its ones segment (RING_DEPTH >= 2), so the bytes in flight per warp are those of the plain
+// form.  COUNT_GT must be set; MODE applies to |gt & pd|, and |zt & pd| goes through POPC.
+template <bool COUNT_GT, int MODE, bool ENTRIES = false>
 __global__ void __launch_bounds__(PANEL_THREADS, 1)
-confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t words,
+confusion_panel_list_kernel(const uint64_t* __restrict__ gt, const uint64_t* __restrict__ zt, int64_t m, int64_t words,
                             const uint64_t* __restrict__ u_words, const uint64_t* __restrict__ vt, int64_t k,
                             int panel_chunks, int RING_DEPTH, const PanelGrid pg, unsigned long long* __restrict__ counts) {
+  static_assert(!ENTRIES || COUNT_GT, "stored-entry counts count |gt|");
+  const bool has_z = ENTRIES && zt != nullptr;
+  const int segs = has_z ? 2 : 1;                                 // ring slots per row
   extern __shared__ __align__(128) uint8_t panel_smem[];
   const int panel_pairs = panel_chunks * CH_PAIRS;
   const int row_bytes = panel_pairs * 16;
@@ -1638,23 +1667,27 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
     const int64_t last_block = gw + (int64_t)(my_blocks - 1) * nwarps;
     last_rows = (int)((m - last_block * 32) < 32 ? (m - last_block * 32) : 32);
   }
-  int to_issue = my_blocks > 0 ? (my_blocks - 1) * 32 + last_rows : 0;
+  int to_issue = my_blocks > 0 ? ((my_blocks - 1) * 32 + last_rows) * segs : 0;   // segments not yet requested
   const uint64_t* iss_ptr = gt + 2 * pair0 + gw * 32 * words;
   const int64_t step_block = (nwarps * 32 - 31) * words;
   int iss_r = 0, iss_slot = 0;
+  bool iss_z = false;                                              // next segment is the zeros half of the row
   auto issue = [&]() {
+    const uint64_t* src = (ENTRIES && iss_z) ? zt + (iss_ptr - gt) : iss_ptr;
     mbar_expect_tx(bar0 + 8u * iss_slot, seg_bytes);
-    bulk_load(ring0 + (uint32_t)(iss_slot * row_bytes), iss_ptr, seg_bytes, bar0 + 8u * iss_slot);
+    bulk_load(ring0 + (uint32_t)(iss_slot * row_bytes), src, seg_bytes, bar0 + 8u * iss_slot);
     iss_slot = iss_slot == RING_DEPTH - 1 ? 0 : iss_slot + 1;
-    if (++iss_r == 32) { iss_r = 0; iss_ptr += step_block; } else { iss_ptr += words; }
     --to_issue;
+    if (ENTRIES && has_z && !iss_z) { iss_z = true; return; }
+    iss_z = false;
+    if (++iss_r == 32) { iss_r = 0; iss_ptr += step_block; } else { iss_ptr += words; }
   };
   if (lane == 0)
     for (int d = 0; d < RING_DEPTH && to_issue > 0; ++d) issue();
 
-  HarleySeal8 hs_tp, hs_pd, hs_gt;
+  HarleySeal8 hs_tp, hs_pd, hs_gt, hs_z;
   HarleySeal4 h4_tp;
-  bool sec_tp = false, sec_pd = false, sec_gt = false;
+  bool sec_tp = false, sec_pd = false, sec_gt = false, sec_z = false;
   long long n_pd = 0, n_tp = 0;
   int slot = 0;
   uint32_t phase = 0;
@@ -1667,7 +1700,7 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
     u_next = (blk + 1 < my_blocks && (gw + (int64_t)(blk + 1) * nwarps) * 32 + lane < m) ? __ldg(u_ptr) : 0ull;
     const uint64_t list = pack_selection(u_cur);                 // this lane's row, scanned once
     const uint32_t list_lo = (uint32_t)list, list_hi = (uint32_t)(list >> 32);
-    int blk_pd = (list_hi >> 24) == 1u ? pop_v[list_lo & 0xffu] : 0, blk_tp = 0;
+    int blk_pd = (!ENTRIES && (list_hi >> 24) == 1u) ? pop_v[list_lo & 0xffu] : 0, blk_tp = 0;
     const int nrows = blk + 1 < my_blocks ? 32 : last_rows;
     for (int r = 0; r < nrows; ++r) {
       const uint32_t lo = __shfl_sync(0xffffffffu, list_lo, r);
@@ -1675,10 +1708,16 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
       const int cnt = (int)(hi >> 24);
       const ulonglong2* seg = reinterpret_cast<const ulonglong2*>(ring + (size_t)slot * row_bytes);
       mbar_wait(bar0 + 8u * slot, phase);
+      const ulonglong2* zseg = nullptr;
+      if (has_z) {                                               // the zeros half sits in the next slot
+        if (++slot == RING_DEPTH) { slot = 0; phase ^= 1u; }
+        zseg = reinterpret_cast<const ulonglong2*>(ring + (size_t)slot * row_bytes);
+        mbar_wait(bar0 + 8u * slot, phase);
+      }
       if (COUNT_GT || cnt != 0) {                                // a row that uses no factor predicts nothing
         for (int c = 0; c < nch; ++c) {
           const int slot0 = c * CH_PAIRS + lane;
-          ulonglong2 g[4], d[4];
+          ulonglong2 g[4], d[4], z[4];
           uint64_t w[8];
 #pragma unroll
           for (int u = 0; u < 4; ++u) g[u] = seg[slot0 + 32 * u];
@@ -1687,6 +1726,12 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
             for (int u = 0; u < 4; ++u) { w[2 * u] = g[u].x; w[2 * u + 1] = g[u].y; }
             if (!sec_gt) hs_gt.add8_first(w); else hs_gt.add8_second(w);
             sec_gt = !sec_gt;
+          }
+          if (has_z) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) { z[u] = zseg[slot0 + 32 * u]; w[2 * u] = z[u].x; w[2 * u + 1] = z[u].y; }
+            if (!sec_z) hs_z.add8_first(w); else hs_z.add8_second(w);
+            sec_z = !sec_z;
           }
           if (cnt != 0) {
             if (cnt <= 7) {
@@ -1709,7 +1754,12 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
               if (!sec_tp) hs_tp.add8_first(w); else hs_tp.add8_second(w);
               sec_tp = !sec_tp;
             }
-            if (cnt != 1) {                                      // one factor: |prediction| came from pop_v
+            if (ENTRIES) {
+              if (has_z) {
+#pragma unroll
+                for (int u = 0; u < 4; ++u) blk_pd += __popcll(z[u].x & d[u].x) + __popcll(z[u].y & d[u].y);
+              }
+            } else if (cnt != 1) {                               // one factor: |prediction| came from pop_v
               if (MODE == 0) {
 #pragma unroll
                 for (int u = 0; u < 4; ++u) { w[2 * u] = d[u].x; w[2 * u + 1] = d[u].y; }
@@ -1724,7 +1774,8 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
         }
       }
       __syncwarp();
-      if (lane == 0 && to_issue > 0) issue();
+      if (lane == 0)                                             // refill the slot(s) of this row
+        for (int q = 0; q < segs && to_issue > 0; ++q) issue();
       if (++slot == RING_DEPTH) { slot = 0; phase ^= 1u; }
     }
     n_pd += blk_pd;
@@ -1737,6 +1788,10 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, int64_t m, int64_t 
     atomicAdd(counts + 0, (unsigned long long)t_tp);
     atomicAdd(counts + 1, (unsigned long long)t_pd);
     if (COUNT_GT) atomicAdd(counts + 2, (unsigned long long)t_gt);
+  }
+  if (has_z) {
+    const long long t_z = warp_sum_ll(hs_z.total());
+    if (lane == 0 && t_z) atomicAdd(counts + 3, (unsigned long long)t_z);
   }
 }
 
@@ -2599,6 +2654,58 @@ __global__ void noise_bits_kernel(uint64_t* __restrict__ x, int64_t rows, int64_
     x[t] = v;
   }
 }
+// ratio_split on bit rows (generate.ratio_split): every one of x draws u from stream s_ones and goes to val (u < t_v), test
+// (u < t_v + t_t) or train; every zero inside the ncols columns draws from stream s_zeros and becomes a stored zero of val
+// (u < q_v), of test (u < q_v + q_t) or stays unstored.  u is the 32-bit half of bernoulli_word's hash for the global bit
+// index, so the result depends on (seed, i, j) only.  out = 5 matrices [rows][words] (train, val ones, val zeros, test
+// ones, test zeros), every word written, pad bits zero.
+__device__ __forceinline__ uint32_t draw32(uint64_t key, uint64_t bit) {
+  const uint64_t h = splitmix64(key + (bit >> 1));
+  return (bit & 1) ? (uint32_t)(h >> 32) : (uint32_t)h;
+}
+__global__ void __launch_bounds__(256)
+split_bits_kernel(const uint64_t* __restrict__ x, int64_t rows, int64_t ncols, int64_t words, int64_t row0, uint64_t seed,
+                  uint64_t s_ones, uint64_t s_zeros, uint64_t t_v, uint64_t t_vt, uint64_t q_v, uint64_t q_vt,
+                  uint64_t* __restrict__ out) {
+  const int64_t total = rows * words;
+  const int64_t cw = (ncols + 63) >> 6;
+  const uint64_t k1 = seed * 0x9E3779B97F4A7C15ull + s_ones * 0xD1B54A32D192ED03ull;
+  const uint64_t k0 = seed * 0x9E3779B97F4A7C15ull + s_zeros * 0xD1B54A32D192ED03ull;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = t / words, w = t - r * words;
+    uint64_t tr = 0, v1 = 0, v0 = 0, s1 = 0, s0 = 0;
+    if (w < cw) {
+      const int64_t left = ncols - w * 64;
+      const uint64_t valid = left < 64 ? (1ull << left) - 1ull : ~0ull;
+      const uint64_t xv = __ldcs(x + t) & valid;
+      const uint64_t base = (uint64_t)((row0 + r) * cw + w) * 64ull;
+      uint64_t ones = xv;
+      while (ones) {                                              // a sparse X: few ones per word
+        const int b = __ffsll((long long)ones) - 1;
+        ones &= ones - 1;
+        const uint64_t u = draw32(k1, base + b), bit = 1ull << b;
+        if (u < t_v) v1 |= bit; else if (u < t_vt) s1 |= bit; else tr |= bit;
+      }
+      if (q_vt > 0) {
+        const uint64_t zeros = ~xv & valid;
+#pragma unroll 4
+        for (int q = 0; q < 32; ++q) {                            // one hash serves two neighbouring bits
+          if (((zeros >> (2 * q)) & 3ull) == 0) continue;
+          const uint64_t h = splitmix64(k0 + (base >> 1) + (uint64_t)q);
+          const uint64_t ua = (uint32_t)h, ub = (uint32_t)(h >> 32);
+          const uint64_t ba = 1ull << (2 * q), bb = ba << 1;
+          if (zeros & ba) { if (ua < q_v) v0 |= ba; else if (ua < q_vt) s0 |= ba; }
+          if (zeros & bb) { if (ub < q_v) v0 |= bb; else if (ub < q_vt) s0 |= bb; }
+        }
+      }
+    }
+    out[t] = tr;
+    out[total + t] = v1;
+    out[2 * total + t] = v0;
+    out[3 * total + t] = s1;
+    out[4 * total + t] = s0;
+  }
+}
 // 64 x 64 bit-block transpose in registers: lane l holds rows l (a0) and l + 32 (a1) of the block and afterwards its
 // columns l and l + 32 as rows.  Six block-swap stages (Hacker's Delight, 7-3): 32 inside the thread, 16 .. 1 between
 // lanes by shuffles -- about 60 instructions per warp and block instead of 64 ballots per warp.
@@ -3066,7 +3173,7 @@ static int launch_confusion(const uint64_t* gt_bits, const uint64_t* pd_bits, in
     rc = check_cuda(cudaFuncSetAttribute(confusion_panel_list_kernel<CG, MD>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                          (int)smem), who);                                                                \
     if (rc) return rc;                                                                                                    \
-    confusion_panel_list_kernel<CG, MD><<<ctas, PANEL_THREADS, smem, st>>>(gt_bits, m, words, u_words, vt_bits, k, chunks,  \
+    confusion_panel_list_kernel<CG, MD><<<ctas, PANEL_THREADS, smem, st>>>(gt_bits, nullptr, m, words, u_words, vt_bits, k, chunks,  \
                                                                            depth, pg, c);                                 \
   } while (0)
       if (panel_lists()) {
@@ -3093,10 +3200,10 @@ static int launch_confusion(const uint64_t* gt_bits, const uint64_t* pd_bits, in
   int64_t blocks = ceil_div(m, 8);
   if (blocks > row_stream_grid()) blocks = row_stream_grid();
   if (gt_ones >= 0)
-    confusion_kernel<FROM_FACTORS, false><<<(unsigned)blocks, 256, 0, st>>>(gt_bits, pd_bits, m, words, u_words, kw,
+    confusion_kernel<FROM_FACTORS, false><<<(unsigned)blocks, 256, 0, st>>>(gt_bits, nullptr, pd_bits, m, words, u_words, kw,
                                                                           vt_bits, c, row_tp, row_fp);
   else
-    confusion_kernel<FROM_FACTORS, true><<<(unsigned)blocks, 256, 0, st>>>(gt_bits, pd_bits, m, words, u_words, kw,
+    confusion_kernel<FROM_FACTORS, true><<<(unsigned)blocks, 256, 0, st>>>(gt_bits, nullptr, pd_bits, m, words, u_words, kw,
                                                                          vt_bits, c, row_tp, row_fp);
   rc = check_cuda(cudaGetLastError(), who);
   if (rc) return rc;
@@ -3119,6 +3226,56 @@ extern "C" int bmf_confusion_bits(const uint64_t* gt_bits, const uint64_t* pd_bi
   BMF_REQUIRE(gt_bits && pd_bits && counts && m > 0 && words > 0 && words % 2 == 0, "bmf_confusion_bits: bad arguments");
   return launch_confusion<false>(gt_bits, pd_bits, m, words, nullptr, 0, nullptr, 0, gt_ones, counts, row_tp, row_fp,
                                  as_stream(stream), "bmf_confusion_bits");
+}
+
+// Stored-entry counts (task='prediction'): counts[0..3] = (|ones & pd|, |zeros & pd|, |ones|, |zeros|) in ONE pass,
+// against a materialised prediction (FROM_FACTORS false) or the product of the factors.  The panel-list form serves
+// k <= 64 when its ring holds the two segments of a row, the row-stream form everything else.
+template <bool FROM_FACTORS>
+static int launch_confusion_entries(const uint64_t* ones, const uint64_t* zeros, const uint64_t* pd_bits, int64_t m,
+                                    int64_t words, const uint64_t* u_words, int64_t kw, const uint64_t* vt_bits, int64_t k,
+                                    int64_t* counts, cudaStream_t st, const char* who) {
+  int rc = check_cuda(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), st), who);
+  if (rc) return rc;
+  unsigned long long* c = reinterpret_cast<unsigned long long*>(counts);
+  if (FROM_FACTORS && !panel_disabled()) {
+    const int chunks = panel_chunks_for(k, kw, words);
+    const int depth = chunks > 0 ? confusion_ring_depth(k, chunks) : 0;
+    if (chunks > 0 && depth >= 2) {
+      const size_t smem = confusion_panel_smem(k, chunks, depth);
+      const int64_t max_splits = ceil_div(ceil_div(m, 32), PANEL_WARPS);
+      int ctas = 0;
+      const PanelGrid pg = make_panel_grid(words >> 1, chunks * CH_PAIRS, max_splits, &ctas);
+      rc = check_cuda(cudaFuncSetAttribute(confusion_panel_list_kernel<true, 3, true>,
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), who);
+      if (rc) return rc;
+      confusion_panel_list_kernel<true, 3, true><<<ctas, PANEL_THREADS, smem, st>>>(ones, zeros, m, words, u_words, vt_bits,
+                                                                                 k, chunks, depth, pg, c);
+      return check_cuda(cudaGetLastError(), who);
+    }
+  }
+  int64_t blocks = ceil_div(m, 8);
+  if (blocks > row_stream_grid()) blocks = row_stream_grid();
+  confusion_kernel<FROM_FACTORS, true, true><<<(unsigned)blocks, 256, 0, st>>>(ones, zeros, pd_bits, m, words, u_words, kw,
+                                                                             vt_bits, c, nullptr, nullptr);
+  return check_cuda(cudaGetLastError(), who);
+}
+
+extern "C" int bmf_confusion_entries_bits(const uint64_t* ones, const uint64_t* zeros, const uint64_t* pd_bits, int64_t m,
+                                          int64_t words, int64_t* counts, bmf_stream_t stream) {
+  BMF_REQUIRE(ones && pd_bits && counts && m > 0 && words > 0 && words % 2 == 0, "bmf_confusion_entries_bits: bad arguments");
+  return launch_confusion_entries<false>(ones, zeros, pd_bits, m, words, nullptr, 0, nullptr, 0, counts, as_stream(stream),
+                                         "bmf_confusion_entries_bits");
+}
+
+extern "C" int bmf_confusion_entries_factors(const uint64_t* ones, const uint64_t* zeros, int64_t m, int64_t words,
+                                             const uint64_t* u_words, int64_t kw, const uint64_t* vt_bits, int64_t k,
+                                             int64_t* counts, bmf_stream_t stream) {
+  BMF_REQUIRE(ones && u_words && counts && m > 0 && kw > 0 && k >= 0 && k <= kw * 64,
+              "bmf_confusion_entries_factors: bad arguments");
+  BMF_REQUIRE(words > 0 && words % 2 == 0 && (k == 0 || vt_bits), "bmf_confusion_entries_factors: bad words / vt_bits");
+  return launch_confusion_entries<true>(ones, zeros, nullptr, m, words, u_words, kw, vt_bits, k, counts, as_stream(stream),
+                                        "bmf_confusion_entries_factors");
 }
 
 extern "C" int bmf_bits_combine(const uint64_t* a_bits, const uint64_t* b_bits, int64_t rows, int64_t words, int op,
@@ -3334,6 +3491,21 @@ extern "C" int bmf_noise_bits(uint64_t* bits, int64_t rows, int64_t ncols, int64
   noise_bits_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(bits, rows, ncols, words, row0, seed,
                                                                    bernoulli_threshold(p_pos), bernoulli_threshold(p_neg));
   BMF_LAUNCH_CHECK("bmf_noise_bits");
+  return 0;
+}
+
+extern "C" int bmf_split_bits(const uint64_t* x_bits, int64_t rows, int64_t ncols, int64_t words, int64_t row0, uint64_t seed,
+                              uint64_t stream_ones, uint64_t stream_zeros, uint64_t t_v, uint64_t t_t, uint64_t q_v,
+                              uint64_t q_t, uint64_t* out_bits, bmf_stream_t stream) {
+  BMF_REQUIRE(x_bits && out_bits && rows >= 0 && ncols > 0 && words * 64 >= ncols && row0 >= 0, "bmf_split_bits: bad arguments");
+  BMF_REQUIRE(t_v <= 0xFFFFFFFFull && t_t <= 0xFFFFFFFFull && q_v <= 0xFFFFFFFFull && q_t <= 0xFFFFFFFFull,
+              "bmf_split_bits: thresholds are 32-bit");
+  if (rows == 0) return 0;
+  int64_t blocks = ceil_div(rows * words, 256);
+  if (blocks > (int64_t)num_sms() * 32) blocks = (int64_t)num_sms() * 32;
+  split_bits_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(x_bits, rows, ncols, words, row0, seed, stream_ones,
+                                                                   stream_zeros, t_v, t_v + t_t, q_v, q_v + q_t, out_bits);
+  BMF_LAUNCH_CHECK("bmf_split_bits");
   return 0;
 }
 

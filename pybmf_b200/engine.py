@@ -63,12 +63,12 @@ def dist_ctx():
 
 def local_plan(X):
     """(plan, r0, r1): ShardPlan of X's rows over the ranks of the process group and this rank's rows.  A
-    generate.DeviceBits must hold exactly those rows, else ValueError (raised before any collective)."""
+    generate.DeviceBits or DeviceEntries must hold exactly those rows, else ValueError (raised before any collective)."""
     rank, world = dist_ctx()
     plan = ShardPlan(X.shape[0], world)
     r0, r1 = plan.rows(rank)
-    if hasattr(X, "bits") and (X.r0, X.r1) != (r0, r1):
-        raise ValueError("DeviceBits rows [%d, %d) must follow ShardPlan(m, world).rows(rank) = [%d, %d)"
+    if hasattr(X, "r0") and (X.r0, X.r1) != (r0, r1):
+        raise ValueError("device rows [%d, %d) must follow ShardPlan(m, world).rows(rank) = [%d, %d)"
                          % (X.r0, X.r1, r0, r1))
     return plan, r0, r1
 

@@ -30,6 +30,57 @@ class DeviceBits:
         return _bits_to_csr(self.bits, self.r1 - self.r0, self.n)
 
 
+class DeviceEntries:
+    """The device form of a split with stored entries (task='prediction', evaluate_utils.py:32-44): `ones` holds the
+    stored non-zeros and `zeros` the explicitly stored zeros of rows [r0, r1) of a logical m x n matrix, both
+    DeviceBits over the same shape and the same ShardPlan rows.  The two must be disjoint (not checked: the producers
+    here, entries_from_host and ratio_split, guarantee it)."""
+
+    def __init__(self, ones: DeviceBits, zeros: DeviceBits):
+        if ones.shape != zeros.shape or (ones.r0, ones.r1) != (zeros.r0, zeros.r1):
+            raise ValueError("DeviceEntries: ones %s rows [%d, %d) and zeros %s rows [%d, %d) differ"
+                             % (ones.shape, ones.r0, ones.r1, zeros.shape, zeros.r0, zeros.r1))
+        local_plan(ones)
+        self.ones, self.zeros = ones, zeros
+        self.shape, self.m, self.n, self.r0, self.r1 = ones.shape, ones.m, ones.n, ones.r0, ones.r1
+
+    def to_csr(self) -> sp.csr_matrix:
+        """This rank's rows as a host csr int64 with the zeros stored explicitly (for cross-checks)."""
+        ones = self.ones.to_csr().tocoo()
+        zeros = self.zeros.to_csr().tocoo()
+        rows = np.concatenate([ones.row, zeros.row])
+        cols = np.concatenate([ones.col, zeros.col])
+        data = np.concatenate([np.ones(ones.nnz, np.int64), np.zeros(zeros.nnz, np.int64)])
+        order = np.lexsort((cols, rows))
+        indptr = np.searchsorted(rows[order], np.arange(self.r1 - self.r0 + 1))
+        return sp.csr_matrix((data[order], cols[order], indptr), shape=(self.r1 - self.r0, self.n))
+
+
+def bits_from_host(X) -> DeviceBits:
+    """This rank's ShardPlan rows of a host csr / ndarray as a DeviceBits; stored zeros are dropped."""
+    from .utils import _bits_on_device, to_sparse
+    X = X if sp.isspmatrix_csr(X) else to_sparse(X, "csr")
+    _plan, r0, r1 = local_plan(X)
+    Xl = device.csr_rows_view(X, r0, r1)
+    if device.has_stored_zeros(Xl):                             # the packer takes every STORED entry as a one
+        Xl = device.drop_stored_zeros(Xl)
+    return DeviceBits(_bits_on_device(Xl), X.shape[0], X.shape[1], r0, r1)
+
+
+def entries_from_host(X) -> DeviceEntries:
+    """This rank's ShardPlan rows of a host matrix as a DeviceEntries: stored non-zeros into `ones`, explicitly stored
+    zeros into `zeros` (an ndarray, converted to csr like everywhere else, stores none)."""
+    from .utils import _bits_on_device, to_sparse
+    X = X if sp.isspmatrix_csr(X) else to_sparse(X, "csr")
+    _plan, r0, r1 = local_plan(X)
+    Xl = device.csr_rows_view(X, r0, r1)
+    zeros = Xl.copy()
+    zeros.data = (zeros.data == 0).astype(np.int8)
+    zeros.eliminate_zeros()
+    m, n = X.shape
+    return DeviceEntries(bits_from_host(X), DeviceBits(_bits_on_device(zeros), m, n, r0, r1))
+
+
 def _rows_of(m, rank=None, world=None):
     if rank is None or world is None:
         rank, world = dist_ctx()
@@ -136,3 +187,64 @@ def transpose(X: DeviceBits) -> DeviceBits:
         if nw > 0 and c1 > c0:
             out[: c1 - c0, w0:w0 + nw] = recv[r, : c1 - c0, :nw]
     return DeviceBits(out, X.n, X.m, c0, c1)
+
+
+SPLIT_STREAMS = (5, 6)                                          # counter streams of ratio_split: ones, zeros
+
+
+def _threshold(p):
+    """bmf_random_bits' probability -> 32-bit threshold (bernoulli_threshold in bmf_bits.cu)."""
+    if not p > 0.0:
+        return 0
+    if p >= 1.0:
+        return 0xFFFFFFFF
+    return int(p * 4294967296.0)
+
+
+def split_thresholds(ones, m, n, val_size, test_size, neg_ratio=1.0):
+    """The thresholds of ratio_split (pure host logic): (t_v, t_t, q_v, q_t).  A one draws u and goes to val below t_v,
+    to test below t_v + t_t; a zero becomes a stored zero of val below q_v, of test below q_v + q_t, where
+    q_s = thr(neg_ratio * s_size * ones / (m * n - ones)).  Bad sizes, or too few zeros, raise ValueError."""
+    for name, v in (("val_size", val_size), ("test_size", test_size)):
+        if not 0.0 <= v <= 1.0:
+            raise ValueError("%s must be in [0, 1], got %r" % (name, v))
+    if val_size + test_size > 1.0:
+        raise ValueError("val_size + test_size must not exceed 1, got %r" % (val_size + test_size))
+    if not neg_ratio >= 0.0:
+        raise ValueError("neg_ratio must be >= 0, got %r" % (neg_ratio,))
+    zeros = m * n - ones
+    need = neg_ratio * (val_size + test_size) * ones
+    if need > 0 and (zeros == 0 or need / zeros > 1.0):
+        raise ValueError("neg_ratio %r asks for %.0f negatives, the matrix has %d zeros" % (neg_ratio, need, zeros))
+    q_v = neg_ratio * val_size * ones / zeros if zeros else 0.0
+    q_t = neg_ratio * test_size * ones / zeros if zeros else 0.0
+    return _threshold(val_size), _threshold(test_size), _threshold(q_v), _threshold(q_t)
+
+
+def ratio_split(X: DeviceBits, val_size, test_size, neg_ratio=1.0, seed=0):
+    """Split the ones of a row-sharded bit matrix into train / val / test and sample stored zeros (negatives) for val and
+    test: returns (X_train: DeviceBits, X_val: DeviceEntries, X_test: DeviceEntries) on this rank's rows.
+
+    Every one at (i, j) draws a 32-bit uniform number from the counter scheme of random_bits (stream SPLIT_STREAMS[0],
+    global bit index as random_bits) and goes to val with probability val_size, to test with probability test_size,
+    else to train.  Every zero draws from stream SPLIT_STREAMS[1] and becomes a stored zero of val (test) with probability
+    neg_ratio * val_size (test_size) * |X| / (m n - |X|): about neg_ratio negatives per positive in each split.  The result
+    depends on (seed, i, j) only, not on the number of ranks.  This is this project's own recipe: it does not reproduce
+    the random draws of the reference's RatioSplit.
+
+    A collective under an initialised process group (ONE all-reduce of |X|); bad sizes raise ValueError on every rank."""
+    from .engine import all_reduce_sum
+    local_plan(X)
+    _native.require_gpu()
+    rows, words = X.r1 - X.r0, X.bits.shape[1]
+    ones = device.zeros((3,), torch.int64)
+    if rows > 0:
+        _native.call("bmf_confusion_bits", X.bits, X.bits, rows, words, -1, ones, None, None)
+    total = int(all_reduce_sum(ones)[0])
+    t_v, t_t, q_v, q_t = split_thresholds(total, X.m, X.n, val_size, test_size, neg_ratio)
+    out = device.zeros((5, max(rows, 1), words), torch.int64)
+    if rows > 0:
+        _native.call("bmf_split_bits", X.bits, rows, X.n, words, X.r0, int(seed), SPLIT_STREAMS[0], SPLIT_STREAMS[1],
+                     t_v, t_t, q_v, q_t, out)
+    part = [DeviceBits(out[i], X.m, X.n, X.r0, X.r1) for i in range(5)]
+    return part[0], DeviceEntries(part[1], part[2]), DeviceEntries(part[3], part[4])

@@ -20,7 +20,7 @@ import scipy.sparse as sp
 import torch
 from scipy.sparse import csr_matrix, hstack, lil_matrix
 
-from . import _native, device
+from . import _native, device, generate
 from . import utils as U_
 from .engine import CoverEngine, _Trace, all_reduce_sum, dist_ctx, integer_weights, local_plan
 
@@ -95,8 +95,9 @@ class BaseModel:
             _say("[I] Missing validation data.")
         if X_test is None:
             _say("[W] Missing testing data.")
-        # generate.DeviceBits (rows already bit-packed on the device) is passed through: Asso packs nothing and uploads nothing
-        self.X_train = X_train if hasattr(X_train, "bits") else U_.to_sparse(X_train, "csr")
+        # generate.DeviceBits / DeviceEntries (rows already bit-packed on the device) are passed through: Asso packs nothing
+        # and uploads nothing
+        self.X_train = X_train if hasattr(X_train, "r0") else U_.to_sparse(X_train, "csr")
         self.X_val = _split(self.X_train, X_val, getattr(self, "task", None))
         self.X_test = _split(self.X_train, X_test, getattr(self, "task", None))
         self.m, self.n = self.X_train.shape
@@ -233,11 +234,15 @@ class BaseModel:
 
     def _split_counts(self, name):
         """(TP, FP, FN, size) of the current factors against X_<name> under self.task
-        (evaluate_utils.py:32-52); counts come from bmf_confusion_factors / _triplets.  A generate.DeviceBits split is
-        counted on this rank's rows and summed over the ranks: a collective under an initialised process group."""
+        (evaluate_utils.py:32-52); counts come from bmf_confusion_factors / _entries_factors / _triplets.  A
+        generate.DeviceBits or DeviceEntries split is counted on this rank's rows and summed over the ranks: a collective
+        under an initialised process group.  Under 'reconstruction' a DeviceEntries counts as its ones, as a host csr
+        with stored zeros does; under 'prediction' a DeviceBits (an X_train) stores its ones and no zeros."""
         X = getattr(self, "X_" + name)
         if self.task == "reconstruction":                     # `self.task` unset -> AttributeError, as D6
-            return U_.factor_counts(X, self.U, self.V)
+            return U_.factor_counts(_ones(X), self.U, self.V)
+        if hasattr(X, "r0"):
+            return U_.entry_counts(X, self.U, self.V)
         Up, Vp = U_._pattern(self.U), U_._pattern(self.V)
         uw, kw = U_._factor_words(Up)
         r, c, g = U_.to_triplet(X)
@@ -373,32 +378,36 @@ def _csr_to_lil_fast(A: csr_matrix) -> lil_matrix:
 
 
 def _split(X_train, X, task):
-    """A validation / test split as fit() keeps it: a host matrix becomes a csr; a generate.DeviceBits is passed through
-    once it is checked, on every rank and before any collective, to have X_train's shape and this rank's ShardPlan
-    rows.  task='prediction' counts stored entries (evaluate_utils.py:32-44), stored zeros included, which bit rows
-    cannot express."""
+    """A validation / test split as fit() keeps it: a host matrix becomes a csr; a generate.DeviceBits or DeviceEntries
+    is passed through once it is checked, on every rank and before any collective, to have X_train's shape and this
+    rank's ShardPlan rows.  task='prediction' counts stored entries (evaluate_utils.py:32-44), stored zeros included,
+    which a DeviceEntries holds and plain bit rows cannot express."""
     if X is None:
         return None
-    if not hasattr(X, "bits"):
+    if not hasattr(X, "r0"):
         return U_.to_sparse(X, "csr")
     if X.shape != X_train.shape:
-        raise ValueError("DeviceBits split of shape %s, X_train is %s" % (X.shape, X_train.shape))
+        raise ValueError("device split of shape %s, X_train is %s" % (X.shape, X_train.shape))
     local_plan(X)
-    if task == "prediction":
-        raise ValueError("task='prediction' counts stored entries; a DeviceBits split has none, use 'reconstruction'")
+    if task == "prediction" and not hasattr(X, "zeros"):
+        raise ValueError("task='prediction' counts stored entries; a DeviceBits split has none, use a DeviceEntries "
+                         "or 'reconstruction'")
     return X
+
+
+def _ones(X):
+    """The stored ones of a generate.DeviceEntries (what a fit trains on and 'reconstruction' counts), else X."""
+    return X.ones if hasattr(X, "zeros") else X
 
 
 def _local_rows(X):
     """(plan, r0, r1, bit rows) of this rank's share of the training matrix under ShardPlan.  A generate.DeviceBits is
-    used as it is; of a host csr only the rank's rows are packed, from a zero-copy row view."""
+    used as it is (a DeviceEntries by its ones); of a host csr only the rank's rows are packed (generate.bits_from_host)."""
+    X = _ones(X)
     plan, r0, r1 = local_plan(X)
-    if hasattr(X, "bits"):
-        return plan, r0, r1, X.bits
-    Xl = device.csr_rows_view(X, r0, r1)
-    if device.has_stored_zeros(Xl):                             # the packer takes every STORED entry as a one
-        Xl = device.drop_stored_zeros(Xl)
-    return plan, r0, r1, U_._bits_on_device(Xl)
+    if not hasattr(X, "bits"):
+        X = generate.bits_from_host(X)
+    return plan, r0, r1, X.bits
 
 
 def _gather_rows(local, plan):
@@ -568,7 +577,7 @@ class Asso(BaseModel):
     def init_model(self):
         super().init_model()
         w_fn = 1 - self.w_fp if self.w_fn is None else self.w_fn
-        self._dev = CoverEngine(self.X_train, self.w_fp, w_fn, scorer=self._scorer, assoc=self._assoc_kernel,
+        self._dev = CoverEngine(_ones(self.X_train), self.w_fp, w_fn, scorer=self._scorer, assoc=self._assoc_kernel,
                                 rescore=self.__dict__.get("_rescore", "auto"))
         self._dev.trace.rows.insert(0, ("before_engine", self._dev.trace.t0 - self.__dict__.get("_dev_t0", self._dev.trace.t0)))
         self.rescore_ = self._dev.rescore                      # 'incremental' or 'full' (what this fit really runs)
@@ -670,16 +679,20 @@ class Asso(BaseModel):
         if dev is None or "_dev_counts" not in self.__dict__ or X.shape != (self.m, self.n):
             return super()._split_counts(name)
         # During a fit the cover U o V^T of this rank's rows IS dev.c_bits: the split is packed once per fit and every
-        # step costs one or two streaming passes (no factor materialisation, no re-upload).
+        # step costs one streaming pass (no factor materialisation, no re-upload).
         # reconstruction: counts over the whole matrix; prediction: over the STORED entries (evaluate_utils.py:32-44),
-        # i.e. ones (TP / FN) and explicitly stored zeros (FP / TN) separately.
+        # i.e. ones (TP / FN) and explicitly stored zeros (FP / TN), both in one bmf_confusion_entries_bits pass.
         cache = self.__dict__.setdefault("_dev_split_cache", {})
         key = (name, self.task)
-        if key not in cache and hasattr(X, "bits"):         # generate.DeviceBits: this rank's rows are already bit rows
-            ones = device.zeros((3,), torch.int64)
-            if dev.m_loc > 0:                                 # |split|: TP of the split against itself, once per fit
-                _native.call("bmf_confusion_bits", X.bits, X.bits, dev.m_loc, dev.words, -1, ones, None, None)
-            cache[key] = {"ones": X.bits, "n_ones": int(ones[0])}
+        if key not in cache and hasattr(X, "r0"):           # generate.DeviceBits / DeviceEntries: already bit rows
+            ones = _ones(X).bits
+            if self.task == "prediction":                    # a DeviceBits (an X_train) stores its ones and no zeros
+                cache[key] = {"ones": ones, "zeros": X.zeros.bits if hasattr(X, "zeros") else None}
+            else:
+                n_ones = device.zeros((3,), torch.int64)
+                if dev.m_loc > 0:                             # |split|: TP of the split against itself, once per fit
+                    _native.call("bmf_confusion_bits", ones, ones, dev.m_loc, dev.words, -1, n_ones, None, None)
+                cache[key] = {"ones": ones, "n_ones": int(n_ones[0])}
         if key not in cache:
             Xl = device.csr_rows_view(X, dev.r0, dev.r1)
             # the common case stores no explicit zeros: then the stored pattern IS the set of ones (no 1e8-entry copies)
@@ -696,22 +709,20 @@ class Asso(BaseModel):
                     zeros.data = (zeros.data == 0).astype(np.int8)
                     zeros.eliminate_zeros()
                     entry["zeros"] = U_._bits_on_device(zeros) if dev.m_loc > 0 else None
-                entry["n_stored"] = int(Xl.nnz)
             cache[key] = entry
         e = cache[key]
-        counts = device.zeros((6,), torch.int64)
+        counts = device.zeros((4,), torch.int64)
         if dev.m_loc > 0:
-            _native.call("bmf_confusion_bits", e["ones"], dev.c_bits, dev.m_loc, dev.words, e["n_ones"], counts[:3], None, None)
-            if self.task == "prediction" and e["zeros"] is not None:
-                _native.call("bmf_confusion_bits", e["zeros"], dev.c_bits, dev.m_loc, dev.words, -1, counts[3:], None, None)
-        stored = torch.tensor([e.get("n_stored", 0)], dtype=torch.int64, device=counts.device)
-        both = torch.cat([counts, stored])
-        all_reduce_sum(both)
-        c = both.cpu().numpy()
+            if self.task == "reconstruction":
+                _native.call("bmf_confusion_bits", e["ones"], dev.c_bits, dev.m_loc, dev.words, e["n_ones"], counts[:3],
+                             None, None)
+            else:
+                _native.call("bmf_confusion_entries_bits", e["ones"], e["zeros"], dev.c_bits, dev.m_loc, dev.words, counts)
+        c = all_reduce_sum(counts).cpu().numpy()
         if self.task == "reconstruction":
             return int(c[0]), int(c[1]), int(c[2]), self.m * self.n
-        # ones: TP = |G1 & C|, FN = |G1 \ C|; stored zeros: FP = |G0 & C| (the TP slot of the second pass)
-        return int(c[0]), int(c[3]), int(c[2]), int(c[6])
+        # (|G1 & C|, |G0 & C|, |G1|, |G0|): TP, FP, FN = |G1| - TP, size = |G1| + |G0|
+        return int(c[0]), int(c[1]), int(c[2] - c[0]), int(c[2] + c[3])
 
 
 class AssoIter(Asso):
@@ -849,20 +860,27 @@ class TransposedModel(Asso):
         assert isinstance(self.model, BaseModel), "The model must be an instance of BaseModel."
 
     def fit(self, X_train, X_val=None, X_test=None, **kwargs):
-        if any(hasattr(X, "bits") for X in (X_train, X_val, X_test)):
-            # row-sharded bit rows: their X^T is re-sharded over the ranks by generate.transpose (a collective); the splits
-            # are checked first so that a bad split raises on every rank before any exchange
-            from . import generate
+        if any(hasattr(X, "r0") for X in (X_train, X_val, X_test)):
+            # row-sharded bit rows: their X^T is re-sharded over the ranks by generate.transpose (a collective; both parts
+            # of a DeviceEntries); the splits are checked first so that a bad split raises on every rank before any exchange
             task = kwargs.get("task", getattr(self.model, "task", None))
             X_val, X_test = _split(X_train, X_val, task), _split(X_train, X_test, task)
-            X_train, X_val, X_test = (X if X is None else generate.transpose(X) if hasattr(X, "bits") else X.T
-                                      for X in (X_train, X_val, X_test))
+            X_train, X_val, X_test = (_transposed(X) for X in (X_train, X_val, X_test))
         else:
             X_train = X_train.T
             X_val = X_val.T if X_val is not None else None
             X_test = X_test.T if X_test is not None else None
         self.model.fit(X_train, X_val, X_test, **kwargs)
         self.U, self.V = self.model.V, self.model.U
+
+
+def _transposed(X):
+    """X^T of a fit input: generate.transpose of a DeviceBits and of both parts of a DeviceEntries, `.T` of a host matrix."""
+    if X is None:
+        return None
+    if hasattr(X, "zeros"):
+        return generate.DeviceEntries(generate.transpose(X.ones), generate.transpose(X.zeros))
+    return generate.transpose(X) if hasattr(X, "bits") else X.T
 
 
 class AssoOpt(Asso):

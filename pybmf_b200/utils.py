@@ -114,15 +114,18 @@ def _factor_words(U: csr_matrix):
     return bits[:, :kw].contiguous(), kw
 
 
-def on_device(*mats):
-    """True when the given matrices (None skipped) are generate.DeviceBits, False when they are host matrices.  A mix is a
-    TypeError; a DeviceBits must hold this rank's ShardPlan rows (ValueError), so that a sum over the ranks counts every
-    row once."""
-    kinds = {hasattr(X, "bits") and hasattr(X, "r0") for X in mats if X is not None}
+def on_device(*mats, entries=False):
+    """True when the given matrices (None skipped) are generate.DeviceBits (or DeviceEntries), False when they are host
+    matrices.  A mix is a TypeError; a DeviceEntries is a TypeError unless `entries` is set (only eval takes one); a
+    device matrix must hold this rank's ShardPlan rows (ValueError), so that a sum over the ranks counts every row once."""
+    given = [X for X in mats if X is not None]
+    kinds = {(hasattr(X, "bits") or hasattr(X, "zeros")) and hasattr(X, "r0") for X in given}
     if len(kinds) > 1:
-        raise TypeError("cannot mix a generate.DeviceBits with a host matrix")
+        raise TypeError("cannot mix a generate.DeviceBits / DeviceEntries with a host matrix")
     if kinds != {True}:
         return False
+    if not entries and any(hasattr(X, "zeros") for X in given):
+        raise TypeError("a generate.DeviceEntries is taken by eval(X_gt=, U=, V=) only")
     from .engine import local_plan
     for X in mats:
         if X is not None:
@@ -167,6 +170,24 @@ def factor_counts(X, U, V):
                      None, None)
     tp, fp, fn = (int(v) for v in all_reduce_sum(counts).cpu().numpy())
     return tp, fp, fn, X.m * X.n
+
+
+def entry_counts(X, U, V):
+    """(TP, FP, FN, size) over the STORED entries (evaluate_utils.py:32-44) of a generate.DeviceEntries -- or of a
+    DeviceBits, whose stored entries are its ones -- against U o V^T, in one bmf_confusion_entries_factors pass over this
+    rank's rows, summed over the ranks (one all-reduce: a collective under an initialised process group)."""
+    from .engine import all_reduce_sum
+    Up, Vp = _pattern(U), _pattern(V)
+    if Up.shape[0] != X.m or Vp.shape[0] != X.n or Up.shape[1] != Vp.shape[1]:
+        raise ValueError("factors U %s and V %s do not fit X %s" % (Up.shape, Vp.shape, X.shape))
+    ones, zeros = (X.ones.bits, X.zeros.bits) if hasattr(X, "zeros") else (X.bits, None)
+    counts = device.zeros((4,), torch.int64)
+    if X.r1 > X.r0:
+        uw, kw = _factor_words(Up[X.r0:X.r1])
+        _native.call("bmf_confusion_entries_factors", ones, zeros, X.r1 - X.r0, ones.shape[1], uw, kw,
+                     _bits_on_device(Vp.T.tocsr()), Up.shape[1], counts)
+    tp, fp, n1, n0 = (int(v) for v in all_reduce_sum(counts).cpu().numpy())
+    return tp, fp, n1 - tp, n1 + n0
 
 
 def _product_bits(U: csr_matrix, Vt: csr_matrix):
@@ -419,16 +440,21 @@ def eval(metrics, task, X_gt, X_pd=None, U=None, V=None):
     """PyBMF/utils/evaluate_utils.py:12-54 -- counts on the GPU; for task='prediction' the
     per-triplet Python loop (:41-44) becomes bmf_confusion_triplets.
 
-    A generate.DeviceBits `X_gt` is compared with factors `U`, `V` under task='reconstruction' only: this rank's rows
-    against this rank's rows of U, summed over the ranks (a collective under an initialised process group)."""
+    A generate.DeviceBits `X_gt` is compared with factors `U`, `V` under task='reconstruction' only, a
+    generate.DeviceEntries under both tasks ('reconstruction' counts its ones, as of a host csr with stored zeros): this
+    rank's rows against this rank's rows of U, summed over the ranks (a collective under an initialised process group)."""
     using_matrix = X_pd is not None
     using_factors = U is not None and V is not None
     assert using_matrix or using_factors, "[E] User should provide either `U`, `V` or `X_pd`."
     assert task in ["prediction", "reconstruction"], "[E] Task should be either 'prediction' or 'reconstruction'."
     _native.require_gpu()
-    if on_device(X_gt):
+    if on_device(X_gt, X_pd, entries=True):
         if using_matrix:
-            raise TypeError("eval: a generate.DeviceBits X_gt is compared with factors U, V, not with X_pd")
+            raise TypeError("eval: a generate.DeviceBits / DeviceEntries X_gt is compared with factors U, V, not with X_pd")
+        if hasattr(X_gt, "zeros"):
+            if task == "reconstruction":
+                return metrics_from_counts(metrics, *factor_counts(X_gt.ones, U, V))
+            return metrics_from_counts(metrics, *entry_counts(X_gt, U, V))
         if task != "reconstruction":
             raise ValueError("eval: task='prediction' counts stored entries, which a generate.DeviceBits cannot hold")
     if not using_factors:
