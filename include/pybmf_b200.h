@@ -269,6 +269,10 @@ int bmf_basis_threshold_rows(const int32_t* cnt_rows, int64_t ldc, int64_t n, in
  * pd_bits[i] = OR_{l in U_i} vt_bits[l]. */
 int bmf_bool_product(const uint64_t* u_words, int64_t m, int64_t kw, const uint64_t* vt_bits,
                      int64_t k, int64_t words, uint64_t* pd_bits, bmf_stream_t stream);
+/* get_residual, PyBMF/utils/common.py:154-160: out[i] = x[i] AND NOT (OR_{l in U_i} vt_bits[l]) in one pass.
+ * Same u_words / vt_bits layout as bmf_bool_product; k = 0 copies x; out must not alias x. */
+int bmf_residual_factors(const uint64_t* x_bits, int64_t m, int64_t words, const uint64_t* u_words, int64_t kw,
+                         const uint64_t* vt_bits, int64_t k, uint64_t* out_bits, bmf_stream_t stream);
 /* TP/FP/FN of PyBMF/utils/metrics.py:56-76 against the product computed on the fly
  * (never materialised).  counts[0..2] = (TP, FP, FN) (overwritten); row_tp/row_fp nullable int32[m].
  * gt_ones = number of ones in gt_bits when the caller knows it (the csr nnz), which saves the
@@ -289,8 +293,7 @@ int bmf_confusion_entries_bits(const uint64_t* ones, const uint64_t* zeros, cons
 int bmf_confusion_entries_factors(const uint64_t* ones, const uint64_t* zeros, int64_t m, int64_t words,
                                   const uint64_t* u_words, int64_t kw, const uint64_t* vt_bits, int64_t k,
                                   int64_t* counts, bmf_stream_t stream);
-/* add(boolean=True) / multiply(boolean=True), PyBMF/utils/boolean_utils.py:87-107 / 6-33, and the
- * residual X AND NOT C of get_residual (PyBMF/utils/common.py:154-160):
+/* add(boolean=True) / multiply(boolean=True), PyBMF/utils/boolean_utils.py:87-107 / 6-33:
  * out = a OR b (op 0), a AND b (op 1), a AND NOT b (op 2) on [rows][words] bit matrices. */
 int bmf_bits_combine(const uint64_t* a_bits, const uint64_t* b_bits, int64_t rows, int64_t words, int op,
                      uint64_t* out_bits, bmf_stream_t stream);

@@ -44,6 +44,7 @@ SIGNATURES = {
     "bmf_select_first_max": [_p, _p, _p, _i64, _i32, _i32, _i64, _f64, _f64, _f64, _i64, _i64, _f64, _p, _p],
     "bmf_cover_apply": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _i32, _f64, _f64, _p, _i64, _i8, _p, _p, _p],
     "bmf_bool_product": [_p, _i64, _i64, _p, _i64, _i64, _p, _p],
+    "bmf_residual_factors": [_p, _i64, _i64, _p, _i64, _p, _i64, _p, _p],
     "bmf_confusion_factors": [_p, _i64, _i64, _p, _i64, _p, _i64, _i64, _p, _p, _p, _p],
     "bmf_confusion_bits": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p],
     "bmf_confusion_entries_bits": [_p, _p, _p, _i64, _i64, _p, _p],

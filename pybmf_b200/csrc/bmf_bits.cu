@@ -1060,9 +1060,13 @@ __device__ __forceinline__ void product_quad(const uint64_t* __restrict__ uw, in
   }
 }
 
+// RESIDUAL (get_residual): x holds X with the layout of pd, and pd receives x AND NOT (the product).  The x pairs are
+// loaded before the OR chain, so their latency overlaps the V^T reads; a row that uses no factor stores x unchanged.
+template <bool RESIDUAL = false>
 __global__ void __launch_bounds__(256)
 bool_product_kernel(const uint64_t* __restrict__ u_words, int64_t m, int64_t kw,
-                    const uint64_t* __restrict__ vt, int64_t words, uint64_t* __restrict__ pd) {
+                    const uint64_t* __restrict__ vt, int64_t words, const uint64_t* __restrict__ x,
+                    uint64_t* __restrict__ pd) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
@@ -1070,11 +1074,19 @@ bool_product_kernel(const uint64_t* __restrict__ u_words, int64_t m, int64_t kw,
   for (int64_t i = warp0; i < m; i += nwarps) {
     const uint64_t* uw = u_words + i * kw;
     for (int64_t p0 = lane; p0 < pairs; p0 += 32 * PU) {
-      ulonglong2 acc[PU];
+      ulonglong2 xv[PU], acc[PU];
+      if (RESIDUAL) {
+#pragma unroll
+        for (int u = 0; u < PU; ++u) {
+          const int64_t p = p0 + 32 * u;
+          xv[u] = p < pairs ? ld_words2(x + i * words + 2 * p) : make_ulonglong2(0ull, 0ull);
+        }
+      }
       product_quad(uw, kw, vt, words, p0, pairs, -1, acc);
 #pragma unroll
       for (int u = 0; u < PU; ++u) {
         const int64_t p = p0 + 32 * u;
+        if (RESIDUAL) acc[u] = make_ulonglong2(xv[u].x & ~acc[u].x, xv[u].y & ~acc[u].y);
         if (p < pairs) __stcs(reinterpret_cast<ulonglong2*>(pd + i * words + 2 * p), acc[u]);   // 128-bit streaming store
       }
     }
@@ -1287,20 +1299,31 @@ struct HarleySeal8 {
   }
 };
 
+__device__ __forceinline__ ulonglong2 or2(const ulonglong2 a, const ulonglong2 b) {
+  return make_ulonglong2(a.x | b.x, a.y | b.y);
+}
+__device__ __forceinline__ ulonglong2 or3(const ulonglong2 a, const ulonglong2 b, const ulonglong2 c) {
+  return make_ulonglong2(a.x | b.x | c.x, a.y | b.y | c.y);
+}
+
 // d = OR of the V^T rows selected by `sel` (warp-uniform) at the lane's four pair slots; the common cases of one and
-// two selected rows are straight-line code (sel comes from a shuffle, so the branch never diverges)
+// two selected rows are straight-line code (sel comes from a shuffle, so the branch never diverges).
+// SEED: d enters with a value and the rows are ORed into it.
+template <bool SEED = false>
 __device__ __forceinline__ void panel_or_fast(const ulonglong2* Vs, int panel_pairs, uint64_t sel, int slot0,
                                               ulonglong2 (&d)[4]) {
   if (sel == 0) {
+    if (!SEED) {
 #pragma unroll
-    for (int u = 0; u < 4; ++u) d[u] = make_ulonglong2(0ull, 0ull);
+      for (int u = 0; u < 4; ++u) d[u] = make_ulonglong2(0ull, 0ull);
+    }
     return;
   }
   const int l0 = __ffsll((long long)sel) - 1;
   sel &= sel - 1;
   const ulonglong2* v0 = Vs + l0 * panel_pairs + slot0;
 #pragma unroll
-  for (int u = 0; u < 4; ++u) d[u] = v0[32 * u];
+  for (int u = 0; u < 4; ++u) d[u] = SEED ? or2(d[u], v0[32 * u]) : v0[32 * u];
   while (sel) {
     const int l = __ffsll((long long)sel) - 1;
     sel &= sel - 1;
@@ -1331,31 +1354,28 @@ __device__ __forceinline__ uint64_t pack_selection(uint64_t u) {
   }
   return p;
 }
-__device__ __forceinline__ ulonglong2 or2(const ulonglong2 a, const ulonglong2 b) {
-  return make_ulonglong2(a.x | b.x, a.y | b.y);
-}
-__device__ __forceinline__ ulonglong2 or3(const ulonglong2 a, const ulonglong2 b, const ulonglong2 c) {
-  return make_ulonglong2(a.x | b.x | c.x, a.y | b.y | c.y);
-}
-// d = OR of the cnt (1..7) V^T rows named by the list bytes (lo = bytes 0..3, hi = bytes 4..6), at the lane's four pair slots
+// d = OR of the cnt (1..7) V^T rows named by the list bytes (lo = bytes 0..3, hi = bytes 4..6), at the lane's four pair
+// slots; SEED: d enters with a value and the rows are ORed into it
+template <bool SEED = false>
 __device__ __forceinline__ void panel_or_list(const ulonglong2* Vs, int panel_pairs, uint32_t lo, uint32_t hi, int cnt,
                                               int slot0, ulonglong2 (&d)[4]) {
   const ulonglong2* base = Vs + slot0;
   const ulonglong2* r0 = base + __byte_perm(lo, 0u, 0x4440u) * panel_pairs;
   if (cnt == 1) {
 #pragma unroll
-    for (int u = 0; u < 4; ++u) d[u] = r0[32 * u];
+    for (int u = 0; u < 4; ++u) d[u] = SEED ? or2(d[u], r0[32 * u]) : r0[32 * u];
     return;
   }
   const ulonglong2* r1 = base + __byte_perm(lo, 0u, 0x4441u) * panel_pairs;
   if (cnt == 2) {
 #pragma unroll
-    for (int u = 0; u < 4; ++u) d[u] = or2(r0[32 * u], r1[32 * u]);
+    for (int u = 0; u < 4; ++u) d[u] = SEED ? or3(d[u], r0[32 * u], r1[32 * u]) : or2(r0[32 * u], r1[32 * u]);
     return;
   }
   const ulonglong2* r2 = base + __byte_perm(lo, 0u, 0x4442u) * panel_pairs;
 #pragma unroll
-  for (int u = 0; u < 4; ++u) d[u] = or3(r0[32 * u], r1[32 * u], r2[32 * u]);
+  for (int u = 0; u < 4; ++u)
+    d[u] = SEED ? or2(d[u], or3(r0[32 * u], r1[32 * u], r2[32 * u])) : or3(r0[32 * u], r1[32 * u], r2[32 * u]);
   if (cnt == 3) return;
   const ulonglong2* r3 = base + (lo >> 24) * panel_pairs;
   if (cnt == 4) {
@@ -1800,11 +1820,16 @@ confusion_panel_list_kernel(const uint64_t* __restrict__ gt, const uint64_t* __r
 // average out of 4.3 M elapsed -- SMs drain their stores at different rates, and the early finishers idle for a sixth of
 // the kernel.  The counter is read two blocks ahead (atomic for block i+2 and the usage words of block i+1 are in flight
 // while block i is written), so its latency is never waited for.
-template <bool DYNAMIC>
+// RESIDUAL (get_residual): pd receives x AND NOT (the product), x with the layout of pd.  Each lane loads its four x
+// pairs of the segment before the OR chain, so the load latency overlaps the panel reads, and seeds the chain with ~x:
+// the store of ~(~x | product) needs no registers beyond d's (x and d held apart spill at 64 registers).  A row that uses
+// no factor stores x unchanged.
+template <bool DYNAMIC, bool RESIDUAL = false>
 __global__ void __launch_bounds__(PRODUCT_THREADS, 1)
 bool_product_panel_list_kernel(const uint64_t* __restrict__ u_words, int64_t m, const uint64_t* __restrict__ vt,
                                int64_t k, int64_t words, int panel_chunks, int store_mode, const PanelGrid pg,
-                               unsigned int* __restrict__ sched, uint64_t* __restrict__ pd) {
+                               unsigned int* __restrict__ sched, const uint64_t* __restrict__ x,
+                               uint64_t* __restrict__ pd) {
   extern __shared__ __align__(128) uint8_t panel_smem[];
   ulonglong2* Vs = reinterpret_cast<ulonglong2*>(panel_smem);
   const int panel_pairs = panel_chunks * CH_PAIRS;
@@ -1846,18 +1871,30 @@ bool_product_panel_list_kernel(const uint64_t* __restrict__ u_words, int64_t m, 
         const int slot0 = c * CH_PAIRS + lane;
         if (c * CH_PAIRS >= valid_pairs) break;
         ulonglong2 d[4];
-        if (cnt == 0) {
+        if (RESIDUAL) {
+          // x at out's offset, derived rather than carried (a second row pointer spills at 64 registers)
+          const ulonglong2* xin = reinterpret_cast<const ulonglong2*>(x) + (out - reinterpret_cast<ulonglong2*>(pd));
 #pragma unroll
-          for (int u = 0; u < 4; ++u) d[u] = make_ulonglong2(0ull, 0ull);
+          for (int u = 0; u < 4; ++u) {
+            const ulonglong2 xv = slot0 + 32 * u < valid_pairs ? __ldg(xin + slot0 + 32 * u) : make_ulonglong2(0ull, 0ull);
+            d[u] = make_ulonglong2(~xv.x, ~xv.y);
+          }
+        }
+        if (cnt == 0) {
+          if (!RESIDUAL) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) d[u] = make_ulonglong2(0ull, 0ull);
+          }
         } else if (cnt <= 7) {
-          panel_or_list(Vs, panel_pairs, lo, hi, cnt, slot0, d);
+          panel_or_list<RESIDUAL>(Vs, panel_pairs, lo, hi, cnt, slot0, d);
         } else {
           const uint64_t sel = ((uint64_t)__shfl_sync(0xffffffffu, (uint32_t)(u_cur >> 32), r) << 32) |
                                __shfl_sync(0xffffffffu, (uint32_t)u_cur, r);
-          panel_or_fast(Vs, panel_pairs, sel, slot0, d);
+          panel_or_fast<RESIDUAL>(Vs, panel_pairs, sel, slot0, d);
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
+          if (RESIDUAL) d[u] = make_ulonglong2(~d[u].x, ~d[u].y);       // ~(~x | product) = x AND NOT product
           if (slot0 + 32 * u < valid_pairs) {
             ulonglong2* dst = out + slot0 + 32 * u;
             if (store_mode == 0) __stcs(dst, d[u]);
@@ -3097,12 +3134,47 @@ extern "C" int bmf_expand_bits_pq(const uint64_t* x_bits, const uint64_t* c_bits
   return 0;
 }
 
+// The product (x == nullptr) or the residual x AND NOT product (RESIDUAL) in the panel-list form (chunks > 0: k <= 64,
+// kw == 1) or the row-stream form (chunks == 0).
+template <bool RESIDUAL>
+static int launch_product(const uint64_t* x, const uint64_t* u_words, int64_t m, int64_t kw, const uint64_t* vt_bits,
+                          int64_t k, int64_t words, int chunks, uint64_t* out, cudaStream_t st, const char* who) {
+  if (chunks == 0) {
+    int64_t blocks = ceil_div(m, 8);
+    if (blocks > row_stream_grid()) blocks = row_stream_grid();
+    bool_product_kernel<RESIDUAL><<<(unsigned)blocks, 256, 0, st>>>(u_words, m, kw, vt_bits, words, x, out);
+    return check_cuda(cudaGetLastError(), who);
+  }
+  const size_t smem = (size_t)k * chunks * CH_PAIRS * 16;
+  const int64_t max_splits = ceil_div(m, 32 * (PRODUCT_THREADS / 32));
+  int ctas = 0;
+  const PanelGrid pg = make_panel_grid(words >> 1, chunks * CH_PAIRS, max_splits, &ctas);
+  unsigned int* sched = (panel_dynamic() && pg.panels <= 64 && m < (1ll << 36)) ? stream_counters(st) : nullptr;
+  int rc = 0;
+  if (sched != nullptr) {
+    rc = check_cuda(cudaMemsetAsync(sched, 0, 64 * sizeof(unsigned int), st), who);
+    if (rc) return rc;
+    rc = check_cuda(cudaFuncSetAttribute(bool_product_panel_list_kernel<true, RESIDUAL>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), who);
+    if (rc) return rc;
+    bool_product_panel_list_kernel<true, RESIDUAL><<<ctas, PRODUCT_THREADS, smem, st>>>(
+        u_words, m, vt_bits, k, words, chunks, product_store_mode(), pg, sched, x, out);
+  } else {
+    rc = check_cuda(cudaFuncSetAttribute(bool_product_panel_list_kernel<false, RESIDUAL>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), who);
+    if (rc) return rc;
+    bool_product_panel_list_kernel<false, RESIDUAL><<<ctas, PRODUCT_THREADS, smem, st>>>(
+        u_words, m, vt_bits, k, words, chunks, product_store_mode(), pg, nullptr, x, out);
+  }
+  return check_cuda(cudaGetLastError(), who);
+}
+
 extern "C" int bmf_bool_product(const uint64_t* u_words, int64_t m, int64_t kw, const uint64_t* vt_bits,
                                 int64_t k, int64_t words, uint64_t* pd_bits, bmf_stream_t stream) {
   BMF_REQUIRE(u_words && pd_bits && m > 0 && kw > 0 && k >= 0 && k <= kw * 64, "bmf_bool_product: bad arguments");
   BMF_REQUIRE(words > 0 && words % 2 == 0 && (k == 0 || vt_bits), "bmf_bool_product: bad words / vt_bits");
   const int chunks = panel_disabled() ? 0 : panel_chunks_for(k, kw, words);
-  if (chunks > 0) {
+  if (chunks > 0 && !(panel_lists() && panel_rowmap() == 0)) {
     const int panel_pairs = chunks * CH_PAIRS;
     const size_t smem = (size_t)k * panel_pairs * 16;
     const int64_t max_splits = ceil_div(m, 32 * (PRODUCT_THREADS / 32));
@@ -3111,36 +3183,25 @@ extern "C" int bmf_bool_product(const uint64_t* u_words, int64_t m, int64_t kw, 
     int rc = check_cuda(cudaFuncSetAttribute(bool_product_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)smem), "bmf_bool_product");
     if (rc) return rc;
-    if (panel_lists() && panel_rowmap() == 0) {
-      unsigned int* sched = (panel_dynamic() && pg.panels <= 64 && m < (1ll << 36)) ? stream_counters(as_stream(stream)) : nullptr;
-      if (sched != nullptr) {
-        rc = check_cuda(cudaMemsetAsync(sched, 0, 64 * sizeof(unsigned int), as_stream(stream)), "bmf_bool_product");
-        if (rc) return rc;
-        rc = check_cuda(cudaFuncSetAttribute(bool_product_panel_list_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)smem), "bmf_bool_product");
-        if (rc) return rc;
-        bool_product_panel_list_kernel<true><<<ctas, PRODUCT_THREADS, smem, as_stream(stream)>>>(
-            u_words, m, vt_bits, k, words, chunks, product_store_mode(), pg, sched, pd_bits);
-      } else {
-        rc = check_cuda(cudaFuncSetAttribute(bool_product_panel_list_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)smem), "bmf_bool_product");
-        if (rc) return rc;
-        bool_product_panel_list_kernel<false><<<ctas, PRODUCT_THREADS, smem, as_stream(stream)>>>(
-            u_words, m, vt_bits, k, words, chunks, product_store_mode(), pg, nullptr, pd_bits);
-      }
-    } else {
-      bool_product_panel_kernel<<<ctas, PRODUCT_THREADS, smem, as_stream(stream)>>>(u_words, m, vt_bits, k, words, chunks,
-                                                                                  panel_rowmap(), product_store_mode(), pg,
-                                                                                  pd_bits);
-    }
+    bool_product_panel_kernel<<<ctas, PRODUCT_THREADS, smem, as_stream(stream)>>>(u_words, m, vt_bits, k, words, chunks,
+                                                                                panel_rowmap(), product_store_mode(), pg,
+                                                                                pd_bits);
     BMF_LAUNCH_CHECK("bmf_bool_product");
     return 0;
   }
-  int64_t blocks = ceil_div(m, 8);
-  if (blocks > row_stream_grid()) blocks = row_stream_grid();
-  bool_product_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(u_words, m, kw, vt_bits, words, pd_bits);
-  BMF_LAUNCH_CHECK("bmf_bool_product");
-  return 0;
+  return launch_product<false>(nullptr, u_words, m, kw, vt_bits, k, words, chunks, pd_bits, as_stream(stream),
+                               "bmf_bool_product");
+}
+
+extern "C" int bmf_residual_factors(const uint64_t* x_bits, int64_t m, int64_t words, const uint64_t* u_words, int64_t kw,
+                                    const uint64_t* vt_bits, int64_t k, uint64_t* out_bits, bmf_stream_t stream) {
+  BMF_REQUIRE(x_bits && u_words && out_bits && m > 0 && kw > 0 && k >= 0 && k <= kw * 64,
+              "bmf_residual_factors: bad arguments");
+  BMF_REQUIRE(words > 0 && words % 2 == 0 && (k == 0 || vt_bits), "bmf_residual_factors: bad words / vt_bits");
+  BMF_REQUIRE(out_bits != x_bits, "bmf_residual_factors: out_bits must not alias x_bits");
+  const int chunks = panel_disabled() ? 0 : panel_chunks_for(k, kw, words);
+  return launch_product<true>(x_bits, u_words, m, kw, vt_bits, k, words, chunks, out_bits, as_stream(stream),
+                              "bmf_residual_factors");
 }
 
 template <bool FROM_FACTORS>

@@ -126,6 +126,26 @@ def planted_bits(m, n, k_true, d_u, d_v, p_fn, p_fp, seed, rank=None, world=None
     return DeviceBits(bits, m, n, r0, r1)
 
 
+def prediction(U, V, rank=None, world=None) -> DeviceBits:
+    """The device form of utils.get_prediction: this rank's ShardPlan rows of the Boolean product U o V^T (m = U.shape[0],
+    n = V.shape[0]) as a DeviceBits, from host factors (lil, csr or ndarray).  One bmf_bool_product launch on this rank's
+    rows of U, no collective; the result does not depend on the number of ranks.  A factor column mismatch raises
+    ValueError."""
+    from .utils import _bits_on_device, _factor_words, _pattern
+    _native.require_gpu()
+    Up, Vp = _pattern(U), _pattern(V)
+    if Up.shape[1] != Vp.shape[1]:
+        raise ValueError("factors U %s and V %s should have the same number of columns" % (Up.shape, Vp.shape))
+    (m, k), n = Up.shape, Vp.shape[0]
+    r0, r1 = _rows_of(m, rank, world)
+    words = device.words_for(n)
+    bits = device.zeros((max(r1 - r0, 1), words), torch.int64)
+    if r1 > r0:
+        uw, kw = _factor_words(Up[r0:r1])
+        _native.call("bmf_bool_product", uw, r1 - r0, kw, _bits_on_device(Vp.T.tocsr()), k, words, bits)
+    return DeviceBits(bits, m, n, r0, r1)
+
+
 _TRANSPOSE_STEP = 64 * 65535                                    # rows per bmf_transpose_bits launch (grid.y limit)
 
 

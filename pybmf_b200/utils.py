@@ -233,7 +233,7 @@ def get_prediction(U, V, boolean=True, sparse=True):
 
 
 def _elementwise(X, Y, op):
-    """Bit-packed OR / AND / AND-NOT on the device (bmf_bits_combine); returns (bits, m, n)."""
+    """Bit-packed OR / AND on the device (bmf_bits_combine); returns (bits, m, n)."""
     _native.require_gpu()
     Xp, Yp = _pattern(X), _pattern(Y)
     assert Xp.shape == Yp.shape, "U and V should have the same shape"
@@ -241,7 +241,7 @@ def _elementwise(X, Y, op):
     out = device.zeros((max(m, 1), device.words_for(n)), torch.int64)
     if m > 0:
         _native.call("bmf_bits_combine", _bits_on_device(Xp), _bits_on_device(Yp), m, out.shape[1],
-                     {"or": 0, "and": 1, "andnot": 2}[op], out)
+                     {"or": 0, "and": 1}[op], out)
     return out, m, n
 
 
@@ -267,10 +267,34 @@ def multiply(U, V, sparse=None, boolean=False):
     return check_sparse(device.bits_to_host(bits, n)[:m].astype(int), sparse=sparse)
 
 
+def _residual_bits(x_bits, rows, U: csr_matrix, vt):
+    """bits of (x AND NOT (U o V^T)) for `rows` bit rows x_bits and the rows of U, by one bmf_residual_factors launch
+    (the product is never formed)."""
+    out = device.zeros((max(rows, 1), x_bits.shape[1]), torch.int64)
+    if rows > 0:
+        uw, kw = _factor_words(U)
+        _native.call("bmf_residual_factors", x_bits, rows, x_bits.shape[1], uw, kw, vt, U.shape[1], out)
+    return out
+
+
 def get_residual(X, U, V):
-    """`X AND NOT (U o V^T)` -- PyBMF/utils/common.py:154-160 (returns lil like the reference)."""
-    pattern = get_prediction(U, V, boolean=True)
-    bits, m, n = _elementwise(X, pattern, "andnot")
+    """`X AND NOT (U o V^T)` -- PyBMF/utils/common.py:154-160 (returns lil like the reference).
+
+    A generate.DeviceBits X gives a DeviceBits with the same shape and rows: this rank's rows of the residual, from this
+    rank's rows of U (no collective)."""
+    _native.require_gpu()
+    Up, Vp = _pattern(U), _pattern(V)
+    if on_device(X):
+        if Up.shape[0] != X.m or Vp.shape[0] != X.n or Up.shape[1] != Vp.shape[1]:
+            raise ValueError("factors U %s and V %s do not fit X %s" % (Up.shape, Vp.shape, X.shape))
+        from .generate import DeviceBits
+        bits = _residual_bits(X.bits, X.r1 - X.r0, Up[X.r0:X.r1], _bits_on_device(Vp.T.tocsr()))
+        return DeviceBits(bits, X.m, X.n, X.r0, X.r1)
+    assert Up.shape[1] == Vp.shape[1], "U and V should be multiplicable"
+    Xp = _pattern(X)
+    assert Xp.shape == (Up.shape[0], Vp.shape[0]), "U and V should have the same shape"
+    m, n = Xp.shape
+    bits = _residual_bits(_bits_on_device(Xp), m, Up, _bits_on_device(Vp.T.tocsr()))
     return lil_matrix(_bits_to_csr(bits, m, n, dtype=sp.csr_matrix(X).dtype))
 
 
