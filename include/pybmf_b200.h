@@ -172,6 +172,45 @@ int bmf_cover_apply_f4(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int6
                        int32_t* fp_old, int32_t wa, int32_t wb, uint8_t* rows_plane, int64_t ld_bytes,
                        int32_t covered_code, uint64_t* u_bits, int64_t* totals, bmf_stream_t stream);
 
+/* ---- block-sparse FP4 scoring (integer weights, zero-dominant encoding) ----
+ * Both planes may hold their K columns in an order sigma and the candidate plane its rows in an order pi: column k of X
+ * is element col_pos[k] (col_pos = sigma^-1, int32 [ncols]) and candidate plane row p holds basis row row_src[p] = pi[p]
+ * (int32 [rows]).  A common K permutation leaves every dot product unchanged; the scorer's epilogue writes the gain of
+ * plane row p to gain[cand_id[p]] and reads the bias from cand_pop[cand_id[p]] (cand_id int32 [cand_pad], padding rows
+ * map to themselves), so gains stay indexed by the original candidate.  The plain entry points above are these with
+ * null maps.  Mapped expansion needs zero == 0 and ld_bytes <= 204800.
+ * kb_table (int32, nullable = dense walk): [mt_total + 1] exclusive prefix sums of the per-candidate-tile counts of K
+ * blocks (256 candidates x 256 columns) that hold a nonzero, then [mt_total][kb_total] the ascending K-block lists
+ * (mt_total = cand_pad / 256, kb_total = ld_bytes / 128).  Blocks left out must be all zero in the candidate plane: they
+ * add exactly 0 to the integer D.  With a table the (data-row super tile, candidate tile) units are walked super tile
+ * outer and split over the CTA pairs by equal K-block cost.
+ * bmf_bits_first_set: row_first[j] = lowest set column of bit row j (ncols when empty), col_first[k] = min row_rank[j]
+ * over the rows holding column k (caller-filled with INT_MAX); both outputs nullable. */
+int bmf_expand_bits_f4_mapped(const uint64_t* bits, const uint64_t* mask_bits, int64_t rows, int64_t ncols, int64_t words,
+                              int32_t one, int32_t zero, int32_t masked, const int32_t* row_src, const int32_t* col_pos,
+                              uint8_t* plane, int64_t rows_pad, int64_t ld_bytes, bmf_stream_t stream);
+int bmf_cover_apply_f4_mapped(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
+                              const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner, int32_t* tp_old,
+                              int32_t* fp_old, int32_t wa, int32_t wb, uint8_t* rows_plane, int64_t ld_bytes,
+                              int32_t covered_code, const int32_t* col_pos, uint64_t* u_bits, int64_t* totals,
+                              bmf_stream_t stream);
+int bmf_cover_apply_compact_mapped(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
+                                   const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner, int32_t* tp_old,
+                                   int32_t* fp_old, int32_t wa, int32_t wb, int32_t kind, int32_t v_one, int32_t v_zero,
+                                   int32_t v_covered, uint8_t* comp_old, uint8_t* comp_new, int64_t comp_ld,
+                                   int64_t comp_cap, int32_t tile_rows, int32_t* nused, uint64_t* u_bits,
+                                   uint64_t* u_words, int64_t kw, int32_t factor_bit, uint64_t* vt_row,
+                                   const int32_t* col_pos, int64_t* totals, bmf_stream_t stream);
+int bmf_cover_score_f4_blocks(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* rows_plane, int64_t rows_pad,
+                              int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale, const int32_t* kb_table,
+                              const int32_t* cand_id, int64_t* gain, bmf_stream_t stream);
+int bmf_cover_rescore_f4_blocks(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* compact_plane,
+                                int64_t rows_cap, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
+                                const int32_t* kb_table, const int32_t* cand_id, const int32_t* dyn_rows,
+                                int32_t gain_sign, int64_t* gain, bmf_stream_t stream);
+int bmf_bits_first_set(const uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, const int32_t* row_rank,
+                       int32_t* row_first, int32_t* col_first, bmf_stream_t stream);
+
 /* argmax of Asso.py:94: first j (lowest index) among alive candidates whose score is
  * strictly greater than `best_score` and than every earlier score.
  * integer mode: score_j = (double)(base_int + gain_p[j]) * scale

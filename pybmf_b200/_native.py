@@ -72,6 +72,14 @@ SIGNATURES = {
     "bmf_transpose_bits": [_p, _i64, _i64, _i64, _p, _i64, _p],
     "bmf_split_bits": [_p, _i64, _i64, _i64, _i64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64,
                        C.c_uint64, _p, _p],
+    "bmf_expand_bits_f4_mapped": [_p, _p, _i64, _i64, _i64, _i32, _i32, _i32, _p, _p, _p, _i64, _i64, _p],
+    "bmf_cover_apply_f4_mapped": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _i32, _p, _i64, _i32, _p, _p, _p,
+                                  _p],
+    "bmf_cover_apply_compact_mapped": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p,
+                                       _p, _i64, _i64, _i32, _p, _p, _p, _i64, _i32, _p, _p, _p, _p],
+    "bmf_cover_score_f4_blocks": [_p, _i64, _p, _i64, _i64, _p, _i32, _p, _p, _p, _p],
+    "bmf_cover_rescore_f4_blocks": [_p, _i64, _p, _i64, _i64, _p, _i32, _p, _p, _p, _i32, _p, _p],
+    "bmf_bits_first_set": [_p, _i64, _i64, _i64, _p, _p, _p, _p],
     "bmf_probe_mma_rate": [_i32, _i32, _p, _p],
     "bmf_refine_column": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
     "bmf_refine_sweep": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],

@@ -4,6 +4,8 @@
 // pipe (POPC); rows are 16-byte aligned so every row stream uses 128-bit loads.
 #include <stdlib.h>
 
+#include <algorithm>
+#include <climits>
 #include <map>
 #include <mutex>
 #include <utility>
@@ -150,6 +152,83 @@ expand_bits_f4_kernel(const uint64_t* __restrict__ bits, const uint64_t* __restr
         dst[q] = f4_codes32((uint32_t)(bw[u] >> sh), (uint32_t)(kw[u] >> sh), valid[u], one, zero, masked);
       }
     }
+  }
+}
+
+// Codes of one 64-column bit word at mapped plane positions: `masked` where c is set, else `one` where x is set (the zero
+// code is 0, so only set bits cost work).  Element e of a row is nibble e % 8 of 32-bit word e / 8; lanes may share a
+// word, hence the atomics.  col_pos == nullptr is the identity map.
+__device__ __forceinline__ void f4_scatter64(uint32_t* row, uint64_t x, uint64_t c, uint64_t valid, int64_t col0,
+                                             const int32_t* __restrict__ col_pos, uint32_t one, uint32_t masked) {
+  uint64_t s = (x | c) & valid;
+  while (s) {
+    const int t = __ffsll((long long)s) - 1;
+    s &= s - 1;
+    const uint32_t code = ((c >> t) & 1ull) ? masked : one;
+    if (code) {
+      const int64_t e = col_pos != nullptr ? (int64_t)col_pos[col0 + t] : col0 + t;
+      atomicOr(row + (e >> 3), code << ((e & 7) * 4));
+    }
+  }
+}
+
+// bmf_expand_bits_f4 with maps (the block-sparse scorer's operand order): plane row r < rows holds bit row row_src[r], and
+// column k of it lands on element col_pos[k].  One warp per plane row: the row is built in a zeroed shared-memory copy by
+// f4_scatter64 and written with coalesced 128-bit stores.
+__global__ void __launch_bounds__(256)
+expand_bits_f4_mapped_kernel(const uint64_t* __restrict__ bits, const uint64_t* __restrict__ mask, int64_t rows,
+                             int64_t ncols, int64_t words, uint32_t one, uint32_t masked, const int32_t* __restrict__ row_src,
+                             const int32_t* __restrict__ col_pos, uint8_t* __restrict__ plane, int64_t rows_pad,
+                             int64_t ld_bytes) {
+  extern __shared__ uint4 expand_smem[];
+  const int lane = threadIdx.x & 31;
+  const int64_t n16 = ld_bytes >> 4;
+  uint4* buf = expand_smem + (threadIdx.x >> 5) * n16;
+  const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t r = warp0; r < rows_pad; r += nwarps) {
+    for (int64_t q = lane; q < n16; q += 32) buf[q] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+    if (r < rows) {
+      const int64_t src = row_src != nullptr ? (int64_t)row_src[r] : r;
+      for (int64_t w = lane; w < words && w * 64 < ncols; w += 32) {
+        const int64_t left = ncols - w * 64;
+        const uint64_t valid = left >= 64 ? ~0ull : ((1ull << left) - 1ull);
+        f4_scatter64(reinterpret_cast<uint32_t*>(buf), bits[src * words + w], mask != nullptr ? mask[src * words + w] : 0ull,
+                     valid, w * 64, col_pos, one, masked);
+      }
+    }
+    __syncwarp();
+    uint4* dst = reinterpret_cast<uint4*>(plane + r * ld_bytes);
+    for (int64_t q = lane; q < n16; q += 32) dst[q] = buf[q];
+    __syncwarp();
+  }
+}
+
+// Per bit row j: row_first[j] = its lowest set column (ncols when the row is empty); col_first[k] = min of row_rank[j] over
+// the rows j that hold column k (the caller fills col_first with INT_MAX first).  Either output is nullable.  One warp per row.
+__global__ void __launch_bounds__(256)
+bits_first_set_kernel(const uint64_t* __restrict__ bits, int64_t rows, int64_t ncols, int64_t words,
+                      const int32_t* __restrict__ row_rank, int32_t* __restrict__ row_first, int32_t* __restrict__ col_first) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t j = warp0; j < rows; j += nwarps) {
+    const int rank = col_first != nullptr ? row_rank[j] : 0;
+    int first = INT_MAX;
+    for (int64_t w = lane; w < words && w * 64 < ncols; w += 32) {
+      const int64_t left = ncols - w * 64;
+      uint64_t b = bits[j * words + w] & (left >= 64 ? ~0ull : ((1ull << left) - 1ull));
+      if (b != 0ull && first == INT_MAX) first = (int)(w * 64) + __ffsll((long long)b) - 1;
+      if (col_first != nullptr)
+        while (b) {
+          const int t = __ffsll((long long)b) - 1;
+          b &= b - 1;
+          atomicMin(col_first + w * 64 + t, rank);
+        }
+    }
+    first = (int)__reduce_min_sync(0xffffffffu, (unsigned)first);
+    if (row_first != nullptr && lane == 0) row_first[j] = first == INT_MAX ? (int)ncols : first;
   }
 }
 
@@ -739,7 +818,23 @@ struct ApplyExtra {
   int32_t* comp_fp_old;
   int32_t* comp_tp_new;
   int32_t* comp_fp_new;
+  // packed E2M1 planes in a column order (the block-sparse scorer's): column k of X is element col_pos[k] of the rows plane
+  // patch (pq_layout 2) and of the compacted rows (kind 1); nullptr = natural order
+  const int32_t* col_pos;
 };
+
+// The E2M1 rows-plane patch of newly covered columns s (64 columns from col0) at mapped positions: the nibble becomes `code`
+__device__ __forceinline__ void f4_patch64(uint32_t* row, uint64_t s, int64_t col0, const int32_t* __restrict__ col_pos,
+                                           uint32_t code) {
+  while (s) {
+    const int t = __ffsll((long long)s) - 1;
+    s &= s - 1;
+    const int64_t e = col_pos[col0 + t];
+    const int sh = (int)(e & 7) * 4;
+    atomicAnd(row + (e >> 3), ~(0xFu << sh));
+    atomicOr(row + (e >> 3), code << sh);
+  }
+}
 
 // The update of ONE data row that uses the winner (warp-collective; P / N = the row's new true / false positives, tpo / fpo
 // its counters before): usage bit, cover OR, counters, the operand-plane patch and the compacted before / after rows.
@@ -757,6 +852,14 @@ __device__ __forceinline__ void apply_used_row(const uint64_t* __restrict__ xb, 
     s0 = __shfl_sync(0xffffffffu, s0, 0);
     slot = s0 < ex.comp_cap ? s0 : -1;                                // capacity = all rows: never exceeded
   }
+  const bool mapped = ex.col_pos != nullptr;
+  if (slot >= 0 && ex.comp_kind == 1 && mapped) {                     // mapped compact rows are scattered into zeroed rows
+    for (int64_t q = lane; q < (ex.comp_ld >> 4); q += 32) {
+      reinterpret_cast<uint4*>(ex.comp_old + slot * ex.comp_ld)[q] = make_uint4(0u, 0u, 0u, 0u);
+      reinterpret_cast<uint4*>(ex.comp_new + slot * ex.comp_ld)[q] = make_uint4(0u, 0u, 0u, 0u);
+    }
+    __syncwarp();
+  }
   for (int64_t p = lane; p < pairs; p += 32) {
     ulonglong2* cp = reinterpret_cast<ulonglong2*>(cb + i * words + 2 * p);
     ulonglong2 c = *cp;
@@ -773,7 +876,12 @@ __device__ __forceinline__ void apply_used_row(const uint64_t* __restrict__ xb, 
         const int64_t col0 = (2 * p + h) * 64;
         const int64_t left = n - col0;
         const uint64_t valid = left >= 64 ? ~0ull : (left <= 0 ? 0ull : ((1ull << left) - 1ull));
-        if (kind == 1 || kind == 3) {                                 // 64 bits -> 32 bytes of packed E2M1
+        if (kind == 1 && mapped) {
+          f4_scatter64(reinterpret_cast<uint32_t*>(ex.comp_old + prow * ex.comp_ld), xw[h], cw[h], valid, col0, ex.col_pos,
+                       ex.v_one, ex.v_cov);
+          f4_scatter64(reinterpret_cast<uint32_t*>(ex.comp_new + prow * ex.comp_ld), xw[h], nw[h], valid, col0, ex.col_pos,
+                       ex.v_one, ex.v_cov);
+        } else if (kind == 1 || kind == 3) {                          // 64 bits -> 32 bytes of packed E2M1
           uint4* o = reinterpret_cast<uint4*>(ex.comp_old + prow * ex.comp_ld + (2 * p + h) * 32);
           uint4* q = reinterpret_cast<uint4*>(ex.comp_new + prow * ex.comp_ld + (2 * p + h) * 32);
 #pragma unroll
@@ -816,6 +924,10 @@ __device__ __forceinline__ void apply_used_row(const uint64_t* __restrict__ xb, 
         int8_t* rowp = rows_plane + i * ld + p * 128;
         while (s0) { const int k = __ffsll((long long)s0) - 1; s0 &= s0 - 1; rowp[k] = (int8_t)covered_value; }
         while (s1) { const int k = __ffsll((long long)s1) - 1; s1 &= s1 - 1; rowp[64 + k] = (int8_t)covered_value; }
+      } else if (pq_layout == 2 && mapped) {
+        uint32_t* roww = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(rows_plane) + i * ld);
+        f4_patch64(roww, s0, p * 128, ex.col_pos, (uint32_t)covered_value & 0xFu);
+        f4_patch64(roww, s1, p * 128 + 64, ex.col_pos, (uint32_t)covered_value & 0xFu);
       } else if (pq_layout == 2) {                                     // packed E2M1 plane: rewrite the nibble
         uint8_t* rowp = reinterpret_cast<uint8_t*>(rows_plane) + i * ld + p * 64;
         const uint32_t code = (uint32_t)covered_value & 0xFu;
@@ -2989,14 +3101,17 @@ extern "C" int bmf_greedy_select(const int64_t* gain_p, const int64_t* gain_n, c
   return 0;
 }
 
-extern "C" int bmf_cover_apply_compact(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
-                                       const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner,
-                                       int32_t* tp_old, int32_t* fp_old, int32_t wa, int32_t wb, int32_t kind,
-                                       int32_t v_one, int32_t v_zero, int32_t v_covered, uint8_t* comp_old,
-                                       uint8_t* comp_new, int64_t comp_ld, int64_t comp_cap, int32_t tile_rows,
-                                       int32_t* nused, uint64_t* u_bits, uint64_t* u_words, int64_t kw,
-                                       int32_t factor_bit, uint64_t* vt_row, int64_t* totals, bmf_stream_t stream) {
+extern "C" int bmf_cover_apply_compact_mapped(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
+                                              const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner,
+                                              int32_t* tp_old, int32_t* fp_old, int32_t wa, int32_t wb, int32_t kind,
+                                              int32_t v_one, int32_t v_zero, int32_t v_covered, uint8_t* comp_old,
+                                              uint8_t* comp_new, int64_t comp_ld, int64_t comp_cap, int32_t tile_rows,
+                                              int32_t* nused, uint64_t* u_bits, uint64_t* u_words, int64_t kw,
+                                              int32_t factor_bit, uint64_t* vt_row, const int32_t* col_pos, int64_t* totals,
+                                              bmf_stream_t stream) {
   BMF_REQUIRE((wa | wb) != 0, "bmf_cover_apply_compact: integer weights only");
+  BMF_REQUIRE(col_pos == nullptr || (kind == 1 && v_zero == 0),
+              "bmf_cover_apply_compact: a column map needs kind 1 (E2M1) and a zero code of 0");
   BMF_REQUIRE(kind == 0 || ((kind == 1 || kind == 2) && comp_old && comp_new && nused && comp_cap > 0 && tile_rows > 0),
               "bmf_cover_apply_compact: kind 1 (E2M1) / 2 (int8) needs the compact planes and the counter");
   BMF_REQUIRE(kind == 0 || (comp_ld % 128 == 0 && comp_ld * (kind == 1 ? 2 : 1) >= words * 64),
@@ -3008,12 +3123,25 @@ extern "C" int bmf_cover_apply_compact(const uint64_t* x_bits, uint64_t* c_bits,
   ex.comp_old = comp_old; ex.comp_new = comp_new; ex.comp_ld = comp_ld; ex.comp_cap = comp_cap; ex.nused = nused;
   ex.comp_kind = kind; ex.v_one = v_one; ex.v_zero = v_zero; ex.v_cov = v_covered;
   ex.u_words = u_words; ex.kw = kw; ex.factor_bit = factor_bit; ex.vt_row = vt_row;
+  ex.col_pos = col_pos;
   int rc = launch_cover_apply(x_bits, c_bits, m, n, words, basis_bits, alive, winner, tp_old, fp_old, wa, wb, 0.0, 0.0,
                               nullptr, 0, 0, 0, u_bits, totals, stream, ex);
   if (rc || kind == 0) return rc;
   compact_tail_zero_kernel<<<64, 256, 0, as_stream(stream)>>>(comp_old, comp_new, comp_ld, comp_cap, nused, tile_rows);
   BMF_LAUNCH_CHECK("bmf_cover_apply_compact");
   return 0;
+}
+
+extern "C" int bmf_cover_apply_compact(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
+                                       const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner,
+                                       int32_t* tp_old, int32_t* fp_old, int32_t wa, int32_t wb, int32_t kind,
+                                       int32_t v_one, int32_t v_zero, int32_t v_covered, uint8_t* comp_old,
+                                       uint8_t* comp_new, int64_t comp_ld, int64_t comp_cap, int32_t tile_rows,
+                                       int32_t* nused, uint64_t* u_bits, uint64_t* u_words, int64_t kw,
+                                       int32_t factor_bit, uint64_t* vt_row, int64_t* totals, bmf_stream_t stream) {
+  return bmf_cover_apply_compact_mapped(x_bits, c_bits, m, n, words, basis_bits, alive, winner, tp_old, fp_old, wa, wb, kind,
+                                        v_one, v_zero, v_covered, comp_old, comp_new, comp_ld, comp_cap, tile_rows, nused,
+                                        u_bits, u_words, kw, factor_bit, vt_row, nullptr, totals, stream);
 }
 
 extern "C" int bmf_cover_apply_compact_general(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
@@ -3059,14 +3187,25 @@ extern "C" int bmf_cover_apply_general(const uint64_t* x_bits, uint64_t* c_bits,
                             w_fn, pq_plane, ld, 0, 1, u_bits, totals, stream);
 }
 
+extern "C" int bmf_cover_apply_f4_mapped(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
+                                         const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner, int32_t* tp_old,
+                                         int32_t* fp_old, int32_t wa, int32_t wb, uint8_t* rows_plane, int64_t ld_bytes,
+                                         int32_t covered_code, const int32_t* col_pos, uint64_t* u_bits, int64_t* totals,
+                                         bmf_stream_t stream) {
+  BMF_REQUIRE(rows_plane != nullptr && covered_code >= 0 && covered_code <= 7, "bmf_cover_apply_f4: bad plane / code");
+  BMF_REQUIRE((wa | wb) != 0, "bmf_cover_apply_f4: integer weights only");
+  ApplyExtra ex = {};
+  ex.col_pos = col_pos;
+  return launch_cover_apply(x_bits, c_bits, m, n, words, basis_bits, alive, winner, tp_old, fp_old, wa, wb, 0.0, 0.0,
+                            reinterpret_cast<int8_t*>(rows_plane), ld_bytes, covered_code, 2, u_bits, totals, stream, ex);
+}
+
 extern "C" int bmf_cover_apply_f4(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
                                   const uint64_t* basis_bits, uint8_t* alive, const int64_t* winner, int32_t* tp_old,
                                   int32_t* fp_old, int32_t wa, int32_t wb, uint8_t* rows_plane, int64_t ld_bytes,
                                   int32_t covered_code, uint64_t* u_bits, int64_t* totals, bmf_stream_t stream) {
-  BMF_REQUIRE(rows_plane != nullptr && covered_code >= 0 && covered_code <= 7, "bmf_cover_apply_f4: bad plane / code");
-  BMF_REQUIRE((wa | wb) != 0, "bmf_cover_apply_f4: integer weights only");
-  return launch_cover_apply(x_bits, c_bits, m, n, words, basis_bits, alive, winner, tp_old, fp_old, wa, wb, 0.0, 0.0,
-                            reinterpret_cast<int8_t*>(rows_plane), ld_bytes, covered_code, 2, u_bits, totals, stream);
+  return bmf_cover_apply_f4_mapped(x_bits, c_bits, m, n, words, basis_bits, alive, winner, tp_old, fp_old, wa, wb, rows_plane,
+                                   ld_bytes, covered_code, nullptr, u_bits, totals, stream);
 }
 
 extern "C" int bmf_cover_apply_f4_general(const uint64_t* x_bits, uint64_t* c_bits, int64_t m, int64_t n, int64_t words,
@@ -3104,19 +3243,56 @@ extern "C" int bmf_e2m1_code(int32_t value) {
   }
 }
 
-extern "C" int bmf_expand_bits_f4(const uint64_t* bits, const uint64_t* mask_bits, int64_t rows, int64_t ncols,
-                                  int64_t words, int32_t one, int32_t zero, int32_t masked, uint8_t* plane,
-                                  int64_t rows_pad, int64_t ld_bytes, bmf_stream_t stream) {
+extern "C" int bmf_expand_bits_f4_mapped(const uint64_t* bits, const uint64_t* mask_bits, int64_t rows, int64_t ncols,
+                                         int64_t words, int32_t one, int32_t zero, int32_t masked, const int32_t* row_src,
+                                         const int32_t* col_pos, uint8_t* plane, int64_t rows_pad, int64_t ld_bytes,
+                                         bmf_stream_t stream) {
   BMF_REQUIRE(bits && plane, "bmf_expand_bits_f4: null pointer");
   BMF_REQUIRE(ld_bytes % 128 == 0 && ld_bytes * 2 >= ncols && rows_pad >= rows && rows >= 0, "bmf_expand_bits_f4: bad ld / rows_pad");
   BMF_REQUIRE(((one | zero | masked) & ~7) == 0, "bmf_expand_bits_f4: codes must be non-negative E2M1 bit patterns (0..7)");
   if (rows_pad == 0) return 0;
+  if (row_src != nullptr || col_pos != nullptr) {
+    BMF_REQUIRE(zero == 0, "bmf_expand_bits_f4_mapped: the zero code must be 0");
+    constexpr int64_t kSmemBudget = 200 * 1024;
+    BMF_REQUIRE(ld_bytes <= kSmemBudget, "bmf_expand_bits_f4_mapped: a plane row must fit in shared memory (ld_bytes <= 204800)");
+    const int64_t warps = std::min<int64_t>(8, kSmemBudget / ld_bytes);
+    const int smem = (int)(warps * ld_bytes);
+    int rc = check_cuda(cudaFuncSetAttribute(expand_bits_f4_mapped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+                        "bmf_expand_bits_f4_mapped");
+    if (rc) return rc;
+    int64_t blocks = ceil_div(rows_pad, warps);
+    if (blocks > (int64_t)num_sms() * 8) blocks = (int64_t)num_sms() * 8;
+    expand_bits_f4_mapped_kernel<<<(unsigned)blocks, (unsigned)(32 * warps), smem, as_stream(stream)>>>(
+        bits, mask_bits, rows, ncols, words, (uint32_t)one, (uint32_t)masked, row_src, col_pos, plane, rows_pad, ld_bytes);
+    BMF_LAUNCH_CHECK("bmf_expand_bits_f4_mapped");
+    return 0;
+  }
   int64_t blocks = ceil_div(rows_pad, 8);
   if (blocks > (int64_t)num_sms() * 8) blocks = (int64_t)num_sms() * 8;
   expand_bits_f4_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(bits, mask_bits, rows, ncols, words, (uint32_t)one,
                                                                        (uint32_t)zero, (uint32_t)masked, plane, rows_pad,
                                                                        ld_bytes);
   BMF_LAUNCH_CHECK("bmf_expand_bits_f4");
+  return 0;
+}
+
+extern "C" int bmf_expand_bits_f4(const uint64_t* bits, const uint64_t* mask_bits, int64_t rows, int64_t ncols,
+                                  int64_t words, int32_t one, int32_t zero, int32_t masked, uint8_t* plane,
+                                  int64_t rows_pad, int64_t ld_bytes, bmf_stream_t stream) {
+  return bmf_expand_bits_f4_mapped(bits, mask_bits, rows, ncols, words, one, zero, masked, nullptr, nullptr, plane, rows_pad,
+                                   ld_bytes, stream);
+}
+
+extern "C" int bmf_bits_first_set(const uint64_t* bits, int64_t rows, int64_t ncols, int64_t words, const int32_t* row_rank,
+                                  int32_t* row_first, int32_t* col_first, bmf_stream_t stream) {
+  BMF_REQUIRE(bits && rows >= 0 && ncols >= 0 && words * 64 >= ncols, "bmf_bits_first_set: bad bits / shape");
+  BMF_REQUIRE(col_first == nullptr || row_rank != nullptr, "bmf_bits_first_set: col_first needs row_rank");
+  if (rows == 0) return 0;
+  int64_t blocks = ceil_div(rows, 8);
+  if (blocks > row_stream_grid()) blocks = row_stream_grid();
+  bits_first_set_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(bits, rows, ncols, words, row_rank, row_first,
+                                                                        col_first);
+  BMF_LAUNCH_CHECK("bmf_bits_first_set");
   return 0;
 }
 

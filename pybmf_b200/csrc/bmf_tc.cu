@@ -62,6 +62,9 @@ struct EpiArgs {
                                    // shrinks to ceil(*dyn_rows / tile) row tiles (nullable: all rows_pad rows are walked)
   int gain_sign;                   // EPI_GAIN: gain[j] += gain_sign * sum relu (-1 retracts the used rows' old contribution)
   int symmetric;                   // EPI_STORE (X^T X): row tiles entirely below the diagonal are skipped (C = C^T)
+  const int32_t* kb_table;         // EPI_GAIN, FP4 super tiles (nullable): per candidate tile the K blocks that hold a nonzero
+                                   // (layout in include/pybmf_b200.h, bmf_cover_score_f4_blocks)
+  const int32_t* cand_id;          // EPI_GAIN (nullable): candidate plane row -> index of its gain and cand_pop entry
 };
 struct __align__(16) RowState { double s_old; int tpo; int fpo; };
 
@@ -1098,6 +1101,66 @@ struct SuperTileIter {
   }
 };
 
+// Block-sparse walk (EPI_GAIN with a K-block table): the units are (super tile st, candidate tile mt) in st-major order, and
+// unit (st, mt) costs cnt[mt] = cum[mt + 1] - cum[mt] K blocks (per sub-tile).  With the candidates and columns reordered
+// most tiles hold few nonzero K blocks (2 to 36 of 70 at c4), so dealing tiles round-robin would leave pairs with several
+// times the work of others: pair p instead takes the units whose cost prefix st * C + cum[mt] lies in
+// [ceil(p T / P), ceil((p + 1) T / P)), T = st_total * C.  Super tiles outer keeps the nonzero candidate blocks (C x 32 KB)
+// resident in L2 while every pair streams its own data rows from DRAM about once.  Units of cost 0 (all-zero candidate
+// tiles: relu(0 - bias) = 0) are skipped.  All three warp roles build the same walk.
+struct SparseWalk {
+  const int32_t* cum;
+  int mt_total, st_total, mt, st;
+  int64_t C, end;
+  __device__ __forceinline__ SparseWalk(const int32_t* cum_, int mt_total_, int st_total_, int64_t pair, int64_t num_pairs)
+      : cum(cum_), mt_total(mt_total_), st_total(st_total_), mt(0), st(st_total_), C(cum_ != nullptr ? cum_[mt_total_] : 0),
+        end(0) {
+    const int64_t T = (int64_t)st_total * C;
+    if (T == 0) return;
+    const int64_t begin = (pair * T + num_pairs - 1) / num_pairs;
+    end = ((pair + 1) * T + num_pairs - 1) / num_pairs;
+    st = (int)(begin / C);
+    const int64_t r = begin - (int64_t)st * C;
+    int lo = 0, hi = mt_total;                            // first mt with cum[mt] >= r (mt_total: none in this super tile)
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (cum[mid] < r) lo = mid + 1; else hi = mid;
+    }
+    mt = lo;
+    if (mt == mt_total) { mt = 0; ++st; }
+  }
+  __device__ __forceinline__ bool next(int& mt_out, int& st_out, int& nkb) {
+    while (st < st_total) {
+      const int c0 = cum[mt], c1 = cum[mt + 1];
+      if ((int64_t)st * C + c0 >= end) return false;
+      mt_out = mt;
+      st_out = st;
+      if (++mt == mt_total) { mt = 0; ++st; }
+      if (c1 > c0) { nkb = c1 - c0; return true; }
+    }
+    return false;
+  }
+};
+
+// The units of one CTA pair for all three warp roles: the dense raster (SuperTileIter, every K block) or, with a K-block
+// table, the block-sparse walk.  nkb = K blocks of the unit; the producer reads their indices from the list (kb_list).
+struct UnitWalk {
+  SuperTileIter dense;
+  SparseWalk sparse;
+  bool is_sparse;
+  int kb_total;
+  __device__ __forceinline__ UnitWalk(const EpiArgs& ea, bool sym, int64_t pair, int64_t num_pairs, int mt_total,
+                                      int st_total, int kb_total_, int group_m)
+      : dense(sym, pair, num_pairs, (int64_t)mt_total * st_total, mt_total, st_total, group_m),
+        sparse(ea.kb_table, mt_total, st_total, pair, num_pairs),
+        is_sparse(ea.kb_table != nullptr), kb_total(kb_total_) {}
+  __device__ __forceinline__ bool next(const EpiArgs& ea, int& mt, int& st, int& nkb) {
+    if (is_sparse) return sparse.next(mt, st, nkb);
+    nkb = kb_total;
+    return dense.next(ea, mt, st);
+  }
+};
+
 template <int EPI>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 gemm_f4s_2sm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b0,
@@ -1119,7 +1182,6 @@ gemm_f4s_2sm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
   const int64_t pair = blockIdx.x >> 1, num_pairs = gridDim.x >> 1;
-  const int64_t total_tiles = (int64_t)mt_total * st_total;   // super tiles
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES_S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
@@ -1155,26 +1217,32 @@ gemm_f4s_2sm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       int stage = 0;
       uint32_t phase = 0;
       const uint32_t sb = warp_uniform(smem_base);
-      SuperTileIter tiles(EPI == EPI_STORE && ea.symmetric, pair, num_pairs, total_tiles, mt_total, st_total, group_m);
-      int mt, st;
-      while (tiles.next(ea, mt, st)) {
+      UnitWalk units(ea, EPI == EPI_STORE && ea.symmetric, pair, num_pairs, mt_total, st_total, kb_total, group_m);
+      const int32_t* kb_lists = ea.kb_table != nullptr ? ea.kb_table + mt_total + 1 : nullptr;
+      int mt, st, nkb;
+      while (units.next(ea, mt, st, nkb)) {
 #pragma unroll 1
         for (int sub = 0; sub < 2; ++sub) {
           const int half = sub ? SUB1 / 2 : SUB0 / 2;                       // data rows this CTA stages
           const int row0 = st * SUPER_ROWS + (sub ? SUB0 : 0) + (int)rank * half;
           const CUtensorMap* mb = sub ? &tmap_b1 : &tmap_b0;
           const uint32_t tx = 2u * (uint32_t)(A_OP + half * BK);
-          for (int kb = 0; kb < kb_total; ++kb) {
-            mbar_wait(empty_bar(stage), phase ^ 1u);
-            const uint32_t leader_full = full_bar(stage) & PEER_MASK;
-            const uint32_t a_dst = sb + stage * STAGE_BYTES_S;
-            if (elect_one()) {
-              if (leader) mbar_expect_tx(full_bar(stage), tx);
-              tma_load_2d_2sm(a_dst, &tmap_a, leader_full, kb * BK, mt * BM4 + (int)rank * HALFM, ea.policy_a);
-              tma_load_2d_2sm(a_dst + A_OP, mb, leader_full, kb * BK, row0, ea.policy_b);
+          for (int i0 = 0; i0 < nkb; i0 += 32) {                          // the list, 32 entries per coalesced load
+            const int kv = (kb_lists != nullptr && i0 + lane < nkb) ? kb_lists[(int64_t)mt * kb_total + i0 + lane] : 0;
+            const int nb = min(32, nkb - i0);
+            for (int j = 0; j < nb; ++j) {
+              const int kb = kb_lists != nullptr ? __shfl_sync(0xffffffffu, kv, j) : i0 + j;
+              mbar_wait(empty_bar(stage), phase ^ 1u);
+              const uint32_t leader_full = full_bar(stage) & PEER_MASK;
+              const uint32_t a_dst = sb + stage * STAGE_BYTES_S;
+              if (elect_one()) {
+                if (leader) mbar_expect_tx(full_bar(stage), tx);
+                tma_load_2d_2sm(a_dst, &tmap_a, leader_full, kb * BK, mt * BM4 + (int)rank * HALFM, ea.policy_a);
+                tma_load_2d_2sm(a_dst + A_OP, mb, leader_full, kb * BK, row0, ea.policy_b);
+              }
+              __syncwarp();
+              if (++stage == STAGES_S) { stage = 0; phase ^= 1u; }
             }
-            __syncwarp();
-            if (++stage == STAGES_S) { stage = 0; phase ^= 1u; }
           }
         }
       }
@@ -1186,16 +1254,16 @@ gemm_f4s_2sm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       uint32_t phase = 0, acc_phase = 0;
       const uint32_t tb = warp_uniform(tmem_base), sb = warp_uniform(smem_base);
       const uint32_t sfa = tb + (uint32_t)SF_COL_S, sfb = tb + (uint32_t)SF_COL_S + 8u;
-      SuperTileIter tiles(EPI == EPI_STORE && ea.symmetric, pair, num_pairs, total_tiles, mt_total, st_total, group_m);
-      int mt, st;
-      while (tiles.next(ea, mt, st)) {
+      UnitWalk units(ea, EPI == EPI_STORE && ea.symmetric, pair, num_pairs, mt_total, st_total, kb_total, group_m);
+      int mt, st, nkb;
+      while (units.next(ea, mt, st, nkb)) {
 #pragma unroll 1
         for (int sub = 0; sub < 2; ++sub) {
           mbar_wait(tempty_bar(sub), acc_phase ^ 1u);
           tcgen05_fence_after();
           const uint32_t d_tmem = tb + (uint32_t)(sub ? SUB0 : 0);
           const uint32_t idesc = sub ? idesc_f4(SUB1) : idesc_f4(SUB0);
-          for (int kb = 0; kb < kb_total; ++kb) {
+          for (int kb = 0; kb < nkb; ++kb) {                              // kb counts the unit's blocks (0 = first)
             mbar_wait(full_bar(stage), phase);
             tcgen05_fence_after();
             const uint32_t a_addr = sb + stage * STAGE_BYTES_S;
@@ -1220,10 +1288,11 @@ gemm_f4s_2sm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   } else {
     const int quad = warp & 3;
     uint32_t acc_phase = 0;
-    SuperTileIter tiles(EPI == EPI_STORE && ea.symmetric, pair, num_pairs, total_tiles, mt_total, st_total, group_m);
-    int mt, st;
-    while (tiles.next(ea, mt, st)) {
-      const int64_t row = (int64_t)mt * BM4 + (int64_t)rank * HALFM + quad * 32 + lane;
+    UnitWalk units(ea, EPI == EPI_STORE && ea.symmetric, pair, num_pairs, mt_total, st_total, kb_total, group_m);
+    int mt, st, nkb;
+    while (units.next(ea, mt, st, nkb)) {
+      const int64_t plane_row = (int64_t)mt * BM4 + (int64_t)rank * HALFM + quad * 32 + lane;
+      const int64_t row = (EPI == EPI_GAIN && ea.cand_id != nullptr) ? (int64_t)ea.cand_id[plane_row] : plane_row;
       const uint32_t lane_base = tmem_base + ((uint32_t)(quad * 32) << 16);
       mbar_wait(tfull_bar(0), acc_phase);
       tcgen05_fence_after();
@@ -1543,15 +1612,18 @@ extern "C" int bmf_gemm_f4_nt(const uint8_t* a_plane, int64_t a_rows_pad, const 
   return tc::f4::launch_gemm_f4<tc::EPI_STORE>(a_plane, a_rows_pad, b_plane, b_rows_pad, ld_bytes, ea, as_stream(stream));
 }
 
-extern "C" int bmf_cover_score_f4(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* rows_plane,
-                                  int64_t rows_pad, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
-                                  int64_t* gain, bmf_stream_t stream) {
+extern "C" int bmf_cover_score_f4_blocks(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* rows_plane,
+                                         int64_t rows_pad, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
+                                         const int32_t* kb_table, const int32_t* cand_id, int64_t* gain, bmf_stream_t stream) {
   BMF_REQUIRE(cand_plane && rows_plane && gain, "bmf_cover_score_f4: null pointer");
   BMF_REQUIRE(cand_pad > 0 && cand_pad % tc::f4::BM4 == 0, "bmf_cover_score_f4: cand_pad must be a positive multiple of 256");
   BMF_REQUIRE(rows_pad > 0 && (rows_pad % tc::f4::BN4 == 0 || rows_pad % tc::f4::SUPER_ROWS == 0),
               "bmf_cover_score_f4: rows_pad must be a positive multiple of 240 or of 496");
   BMF_REQUIRE(ld_bytes > 0 && ld_bytes % tc::BK == 0, "bmf_cover_score_f4: ld_bytes must be a positive multiple of 128");
   BMF_REQUIRE(cand_pop != nullptr || bias_scale == 0, "bmf_cover_score_f4: a bias needs cand_pop");
+  const bool super = rows_pad % tc::f4::SUPER_ROWS == 0 && !tc::f4::super_tiles_disabled();
+  BMF_REQUIRE(super || (kb_table == nullptr && cand_id == nullptr),
+              "bmf_cover_score_f4_blocks: a K-block table / candidate map needs rows_pad padded to 496 (super-tile kernel)");
   int rc = check_cuda(cudaMemsetAsync(gain, 0, sizeof(int64_t) * cand_pad, as_stream(stream)), "bmf_cover_score_f4");
   if (rc) return rc;
   tc::EpiArgs ea = {};
@@ -1560,15 +1632,25 @@ extern "C" int bmf_cover_score_f4(const uint8_t* cand_plane, int64_t cand_pad, c
   ea.bias_scale = bias_scale;
   ea.gain_sign = 1;
   ea.gain = reinterpret_cast<unsigned long long*>(gain);
-  if (rows_pad % tc::f4::SUPER_ROWS == 0 && !tc::f4::super_tiles_disabled())
+  ea.kb_table = kb_table;
+  ea.cand_id = cand_id;
+  if (super)
     return tc::f4::launch_gemm_f4s<tc::EPI_GAIN>(cand_plane, cand_pad, rows_plane, rows_pad, ld_bytes, ea, as_stream(stream));
   BMF_REQUIRE(rows_pad % tc::f4::BN4 == 0, "bmf_cover_score_f4: rows_pad must be a multiple of 240 for the plain-tile kernel");
   return tc::f4::launch_gemm_f4<tc::EPI_GAIN>(cand_plane, cand_pad, rows_plane, rows_pad, ld_bytes, ea, as_stream(stream));
 }
 
-extern "C" int bmf_cover_rescore_f4(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* compact_plane,
-                                    int64_t rows_cap, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
-                                    const int32_t* dyn_rows, int32_t gain_sign, int64_t* gain, bmf_stream_t stream) {
+extern "C" int bmf_cover_score_f4(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* rows_plane,
+                                  int64_t rows_pad, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
+                                  int64_t* gain, bmf_stream_t stream) {
+  return bmf_cover_score_f4_blocks(cand_plane, cand_pad, rows_plane, rows_pad, ld_bytes, cand_pop, bias_scale, nullptr,
+                                   nullptr, gain, stream);
+}
+
+extern "C" int bmf_cover_rescore_f4_blocks(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* compact_plane,
+                                           int64_t rows_cap, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
+                                           const int32_t* kb_table, const int32_t* cand_id, const int32_t* dyn_rows,
+                                           int32_t gain_sign, int64_t* gain, bmf_stream_t stream) {
   BMF_REQUIRE(cand_plane && compact_plane && gain && dyn_rows, "bmf_cover_rescore_f4: null pointer");
   BMF_REQUIRE(gain_sign == 1 || gain_sign == -1, "bmf_cover_rescore_f4: gain_sign must be +1 or -1");
   BMF_REQUIRE(cand_pad > 0 && cand_pad % tc::f4::BM4 == 0, "bmf_cover_rescore_f4: cand_pad must be a positive multiple of 256");
@@ -1582,7 +1664,16 @@ extern "C" int bmf_cover_rescore_f4(const uint8_t* cand_plane, int64_t cand_pad,
   ea.gain_sign = gain_sign;
   ea.dyn_rows = dyn_rows;
   ea.gain = reinterpret_cast<unsigned long long*>(gain);
+  ea.kb_table = kb_table;
+  ea.cand_id = cand_id;
   return tc::f4::launch_gemm_f4s<tc::EPI_GAIN>(cand_plane, cand_pad, compact_plane, rows_cap, ld_bytes, ea, as_stream(stream));
+}
+
+extern "C" int bmf_cover_rescore_f4(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* compact_plane,
+                                    int64_t rows_cap, int64_t ld_bytes, const int32_t* cand_pop, int32_t bias_scale,
+                                    const int32_t* dyn_rows, int32_t gain_sign, int64_t* gain, bmf_stream_t stream) {
+  return bmf_cover_rescore_f4_blocks(cand_plane, cand_pad, compact_plane, rows_cap, ld_bytes, cand_pop, bias_scale, nullptr,
+                                     nullptr, dyn_rows, gain_sign, gain, stream);
 }
 
 static int cover_score_f4_general_impl(const uint8_t* cand_plane, int64_t cand_pad, const uint8_t* pq_plane, int64_t m,

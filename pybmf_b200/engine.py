@@ -24,6 +24,49 @@ from . import _native, device
 
 ROW_ALIGN = 256        # shard boundaries are multiples of the MMA N tile (and of 64-bit u words)
 F4_ROW_PAD = 496       # BMF_F4_SUPER_ROWS: data rows of the FP4 planes are padded to whole super tiles (256 + 240)
+# The block-sparse walk keeps every nonzero 256 x 256 candidate block (32 KB) in L2 while the data rows stream.  Candidate
+# panels up to 55 MB stayed resident (24 tiles of the dense raster); 80 MB fell off the L2 (DESIGN section 4.1), and a
+# denser basis is scored in natural order on the dense raster.
+SPARSE_PANEL_BYTES = 55 << 20
+# ... and only on enough data rows: at c2 (6040 rows, 13 super tiles) a dense pass takes ~50 us, fewer units than CTA pairs
+# are dealt either way, and the reordered pass measured slower (64 against 52 us) on top of the reorder's own launches.
+SPARSE_MIN_ROWS = 64 * F4_ROW_PAD
+
+
+def block_sparse_order(basis_bits, cand_pop, n, words, cand_pad, ld4, cand_plane):
+    """Reorder for the block-sparse FP4 scorer, computed on the device from the basis alone (so every rank gets the same):
+      candidate order pi: by (multi-column first, then single-column, then empty; lowest set column; index);
+      column order sigma: by (position in pi of the first candidate whose row holds the column; column).
+    Writes cand_plane (packed E2M1 0/1, plane row p = basis row pi[p], columns in sigma order) and returns
+    (cand_id, col_pos, kb_table): cand_id[p] = pi[p] (padding rows map to themselves), col_pos = sigma^-1, and kb_table =
+    [mt_total + 1] prefix sums of the per-candidate-tile counts of nonzero 256 x 256 K blocks followed by the
+    [mt_total][kb_total] ascending block lists (see bmf_cover_score_f4_blocks)."""
+    dev = basis_bits.device
+    i32 = torch.int32
+    ar = torch.arange(n, device=dev, dtype=torch.int64)
+    minc = torch.empty((n,), dtype=i32, device=dev)
+    _native.call("bmf_bits_first_set", basis_bits, n, n, words, None, minc, None)
+    pop = cand_pop[:n].to(torch.int64)
+    group = torch.where(pop >= 2, 0, torch.where(pop == 1, 1, 2))
+    pi = torch.argsort((group * (n + 1) + minc.to(torch.int64)) * n + ar)          # unique keys: a deterministic order
+    rank = torch.empty((n,), dtype=i32, device=dev)
+    rank[pi] = ar.to(i32)
+    first = torch.full((n,), torch.iinfo(i32).max, dtype=i32, device=dev)
+    _native.call("bmf_bits_first_set", basis_bits, n, n, words, rank, None, first)
+    sigma = torch.argsort(first.to(torch.int64) * n + ar)
+    col_pos = torch.empty((n,), dtype=i32, device=dev)
+    col_pos[sigma] = ar.to(i32)
+    cand_id = torch.arange(cand_pad, device=dev, dtype=i32)
+    cand_id[:n] = pi.to(i32)
+    _native.call("bmf_expand_bits_f4_mapped", basis_bits, None, n, n, words, 2, 0, 0, cand_id[:n], col_pos, cand_plane,
+                 cand_pad, ld4)
+    mt_total, kb_total = cand_pad // 256, ld4 // 128
+    nz = cand_plane.view(torch.int64).view(mt_total, 256, kb_total, 16).ne(0).any(dim=3).any(dim=1)   # [mt][kb]
+    cum = torch.zeros((mt_total + 1,), dtype=torch.int64, device=dev)
+    cum[1:] = torch.cumsum(nz.sum(dim=1), 0)
+    kb = torch.arange(kb_total, device=dev, dtype=torch.int64)
+    lists = torch.argsort((~nz).to(torch.int64) * kb_total + kb, dim=1)             # nonzero blocks first, ascending
+    return cand_id, col_pos, torch.cat([cum, lists.reshape(-1)]).to(i32)
 
 
 def integer_weights(w_fp, w_fn, max_int=127, max_shift=30):
@@ -220,6 +263,9 @@ class CoverEngine:
         self.cand_pad = device.round_up(self.n, 256)           # multiple of 256 -> the 2-SM (cta_group::2) kernel
         self.cand_plane = None
         self.rows_plane = None
+        # block-sparse FP4 scoring (set by build_basis): candidate plane row -> candidate, column -> plane position, and the
+        # per-candidate-tile lists of nonzero K blocks; None = natural order, dense walk
+        self.cand_id = self.col_pos = self.kb_table = None
         # gain buffer [gain_p | tail (8) | gain_n]: the tail carries (#used, sum P, sum N) of the last apply, so ONE
         # all-reduce per greedy step moves the gains and the counters (integer mode reduces only gain_p + tail)
         cp = self.cand_pad
@@ -422,12 +468,28 @@ class CoverEngine:
             self.launches += 1
         if self.scorer == "tcgen05" and self.operand == "f4":   # candidate rows as packed E2M1 0/1
             self.cand_plane = device.empty((self.cand_pad, self.ld4), torch.uint8)
-            _native.call("bmf_expand_bits_f4", self.basis_bits, None, n, n, self.words, 2, 0, 0, self.cand_plane,
-                         self.cand_pad, self.ld4)
-            self.launches += 1
+            if self.encoding == "zero" and self.m_loc >= SPARSE_MIN_ROWS:
+                self._block_sparse_order()
+            else:
+                _native.call("bmf_expand_bits_f4", self.basis_bits, None, n, n, self.words, 2, 0, 0, self.cand_plane,
+                             self.cand_pad, self.ld4)
+                self.launches += 1
         if self.scorer == "tcgen05":
             self._rebuild_rows_plane()
         self.trace.mark("basis_planes")
+
+    def _block_sparse_order(self):
+        """Candidate plane of the block-sparse FP4 scorer (see block_sparse_order); keeps the natural order when the nonzero
+        candidate blocks would not stay resident in L2."""
+        cand_id, col_pos, table = block_sparse_order(self.basis_bits, self.cand_pop, self.n, self.words, self.cand_pad,
+                                                     self.ld4, self.cand_plane)
+        self.launches += 3
+        if int(table[self.cand_pad // 256].item()) * 32768 <= SPARSE_PANEL_BYTES:
+            self.cand_id, self.col_pos, self.kb_table = cand_id, col_pos, table
+            return
+        _native.call("bmf_expand_bits_f4", self.basis_bits, None, self.n, self.n, self.words, 2, 0, 0, self.cand_plane,
+                     self.cand_pad, self.ld4)
+        self.launches += 1
 
     def _rebuild_rows_plane(self):
         """rows_plane[i][k] = 0 if covered, +wb if x, -wa otherwise (the signed operand of D = wb*P - wa*N)."""
@@ -454,8 +516,9 @@ class CoverEngine:
             rows_pad = device.round_up(max(self.m_loc, 1), F4_ROW_PAD)
             if self.rows_plane is None:
                 self.rows_plane = device.empty((rows_pad, self.ld4), torch.uint8)
-            _native.call("bmf_expand_bits_f4", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
-                         lib.bmf_e2m1_code(one), 0, lib.bmf_e2m1_code(covered), self.rows_plane, rows_pad, self.ld4)
+            _native.call("bmf_expand_bits_f4_mapped", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
+                         lib.bmf_e2m1_code(one), 0, lib.bmf_e2m1_code(covered), None, self.col_pos, self.rows_plane,
+                         rows_pad, self.ld4)
             self.launches += 1
             return
         self.rows_plane = device.expand_bits_i8(self.x_bits, self.m_loc, self.n, one, zero, 256,
@@ -519,9 +582,10 @@ class CoverEngine:
                          self.basis_bits, self.alive, self.record, self.tp_old, self.fp_old, self.w_fp, self.w_fn,
                          self.rows_plane, self.ld, u_bits, self.record[2:5])
         elif self.m_loc > 0 and self.scorer == "tcgen05" and self.operand == "f4":
-            _native.call("bmf_cover_apply_f4", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
+            _native.call("bmf_cover_apply_f4_mapped", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
                          self.basis_bits, self.alive, self.record, self.tp_old, self.fp_old, self.wa, self.wb,
-                         self.rows_plane, self.ld4, _native.load().bmf_e2m1_code(self.wa), u_bits, self.record[2:5])
+                         self.rows_plane, self.ld4, _native.load().bmf_e2m1_code(self.wa), self.col_pos, u_bits,
+                         self.record[2:5])
         elif self.m_loc > 0:
             _native.call("bmf_cover_apply", self.x_bits, self.c_bits, self.m_loc, self.n, self.words, self.basis_bits,
                          self.alive, self.record, self.tp_old, self.fp_old, self.wa, self.wb, self.w_fp, self.w_fn,
@@ -589,8 +653,9 @@ class CoverEngine:
                          self.ld, self.cand_pop, self.tp_old, self.fp_old, self.w_fp, self.w_fn, self.gain_p,
                          self.gain_n)
         elif self.scorer == "tcgen05" and self.operand == "f4":
-            _native.call("bmf_cover_score_f4", self.cand_plane, self.cand_pad, self.rows_plane,
-                         self.rows_plane.shape[0], self.ld4, self.cand_pop, self.wa, self.gain_p)
+            _native.call("bmf_cover_score_f4_blocks", self.cand_plane, self.cand_pad, self.rows_plane,
+                         self.rows_plane.shape[0], self.ld4, self.cand_pop, self.wa, self.kb_table, self.cand_id,
+                         self.gain_p)
         elif self.scorer == "tcgen05":
             _native.call("bmf_cover_score_i8", self.cand_plane, self.cand_pad, self.rows_plane,
                          self.rows_plane.shape[0], self.ld, self.plane_sign,
@@ -661,11 +726,11 @@ class CoverEngine:
             else:
                 kind, (one, zero, cov) = 2, self._plane_values()
                 tile = 256
-            _native.call("bmf_cover_apply_compact", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
+            _native.call("bmf_cover_apply_compact_mapped", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
                          self.basis_bits, self.alive, self.record, self.tp_old, self.fp_old, self.wa, self.wb,
                          kind if compact else 0, one, zero, cov, self.comp_old, self.comp_new,
                          self.comp_old.shape[1], self.comp_old.shape[0], tile, self.nused, u_bits, None, 0, 0, None,
-                         self.tail)
+                         self.col_pos if compact else None, self.tail)
             self.plane_stale = True                            # the big plane is no longer patched
             self.launches += 2 if compact else 1
             return
@@ -678,9 +743,9 @@ class CoverEngine:
                          self.basis_bits, self.alive, self.record, self.tp_old, self.fp_old, self.w_fp, self.w_fn,
                          self.rows_plane, self.ld, u_bits, self.tail)
         elif self.scorer == "tcgen05" and self.operand == "f4":
-            _native.call("bmf_cover_apply_f4", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
+            _native.call("bmf_cover_apply_f4_mapped", self.x_bits, self.c_bits, self.m_loc, self.n, self.words,
                          self.basis_bits, self.alive, self.record, self.tp_old, self.fp_old, self.wa, self.wb,
-                         self.rows_plane, self.ld4, lib.bmf_e2m1_code(self.wa), u_bits, self.tail)
+                         self.rows_plane, self.ld4, lib.bmf_e2m1_code(self.wa), self.col_pos, u_bits, self.tail)
         else:
             _native.call("bmf_cover_apply", self.x_bits, self.c_bits, self.m_loc, self.n, self.words, self.basis_bits,
                          self.alive, self.record, self.tp_old, self.fp_old, self.wa, self.wb, self.w_fp, self.w_fn,
@@ -704,8 +769,8 @@ class CoverEngine:
             return
         for plane, sign in ((self.comp_old, -1), (self.comp_new, 1)):
             if self.operand == "f4":
-                _native.call("bmf_cover_rescore_f4", self.cand_plane, self.cand_pad, plane, cap, self.ld4, self.cand_pop,
-                             self.wa, self.nused, sign, self.gain_p)
+                _native.call("bmf_cover_rescore_f4_blocks", self.cand_plane, self.cand_pad, plane, cap, self.ld4,
+                             self.cand_pop, self.wa, self.kb_table, self.cand_id, self.nused, sign, self.gain_p)
             else:
                 _native.call("bmf_cover_rescore_i8", self.cand_plane, self.cand_pad, plane, cap, self.ld, self.plane_sign,
                              self.cand_pop if self.encoding == "zero" else None, self.wa, self.nused, sign, self.gain_p)
