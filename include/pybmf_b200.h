@@ -435,6 +435,36 @@ int bmf_refine_sweep(const uint64_t* x_bits, int64_t m, int64_t n, int64_t words
                      const uint64_t* vt_bits, int64_t k, int64_t col0, int64_t ncols, int32_t wa, int32_t wb,
                      double w_fp, double w_fn, int64_t* out, bmf_stream_t stream);
 
+/* ---- GreConD's concept search (bmf_concept.cu, pybmf_b200/concept.py) ------------------------------------------------
+ * Bit rows x / res (the residual) are [rows][words] with n <= 64 words columns; a row mask (nullable: every row) selects
+ * the extent C.  Columns are scored a column word (64 columns) at a time, for the column words cw0 .. cw0 + ncw - 1; the
+ * live candidates are the columns j with lo <= j < n and j not in d_bits (nullable), where lo = state[0] + 1 when state
+ * (nullable; int64 [pos, best, done, accepted]) is given, else col_lo.  With state[2] != 0 the kernels do nothing.
+ * bmf_concept_intents: intents[(j - 64 cw0)][.] = AND of the rows of C with bit j (all ones when there are none) for
+ *   every live j; counts (nullable, int64 [64 ncw]) = the number of those rows.  Other rows of intents are unspecified.
+ * bmf_concept_covers : covers[(j - 64 cw0)] = sum over the rows r of C with bit j of popc(res[r] & I_j), where I_j is the
+ *   AND over q < parts of intents[q * part_stride + (j - 64 cw0) * words + .]; 0 for the other columns.
+ * bmf_concept_decide : one block: the first live j (state given) with covers[j] > state[1]; if there is one, pos = j,
+ *   best = covers[j], accepted += 1, d_bits = intents[j], c_bits &= X[:, j] (c_bits: rows bits over the rows of xc);
+ *   else done = 1.  covers / intents hold column j at index j.
+ * bmf_concept_extent : the rows of x with bit col, compacted: xc / rc [cap][words] get their x / res rows and idx [cap]
+ *   their logical rows row0 + r (-1 after the last); fill (int64) = the number of such rows; rows beyond cap are dropped.
+ * bmf_concept_residual: res[idx[c] - row0] &= ~d_bits for every compact row c < rows in c_bits with row0 <= idx[c] < row1
+ *   (res holds rows [row0, row1)). */
+int bmf_concept_intents(const uint64_t* x, int64_t rows, int64_t words, int64_t n, const uint64_t* row_mask, int64_t cw0,
+                        int64_t ncw, int64_t col_lo, const int64_t* state, const uint64_t* d_bits, uint64_t* intents,
+                        int64_t* counts, bmf_stream_t stream);
+int bmf_concept_covers(const uint64_t* x, const uint64_t* res, int64_t rows, int64_t words, int64_t n,
+                       const uint64_t* row_mask, int64_t cw0, int64_t ncw, int64_t col_lo, const int64_t* state,
+                       const uint64_t* d_bits, const uint64_t* intents, int64_t parts, int64_t part_stride, int64_t* covers,
+                       bmf_stream_t stream);
+int bmf_concept_decide(const uint64_t* xc, int64_t rows, int64_t words, int64_t n, const int64_t* covers,
+                       const uint64_t* intents, int64_t* state, uint64_t* c_bits, uint64_t* d_bits, bmf_stream_t stream);
+int bmf_concept_extent(const uint64_t* x, const uint64_t* res, int64_t rows, int64_t words, int64_t row0, int64_t col,
+                       int64_t cap, uint64_t* xc, uint64_t* rc, int64_t* idx, int64_t* fill, bmf_stream_t stream);
+int bmf_concept_residual(uint64_t* res, int64_t row0, int64_t row1, int64_t words, const int64_t* idx, int64_t rows,
+                         const uint64_t* c_bits, const uint64_t* d_bits, bmf_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -83,6 +83,11 @@ SIGNATURES = {
     "bmf_probe_mma_rate": [_i32, _i32, _p, _p],
     "bmf_refine_column": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
     "bmf_refine_sweep": [_p, _i64, _i64, _i64, _p, _i64, _p, _i64, _i64, _i64, _i32, _i32, _f64, _f64, _p, _p],
+    "bmf_concept_intents": [_p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p],
+    "bmf_concept_covers": [_p, _p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _i64, _p, _p],
+    "bmf_concept_decide": [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p],
+    "bmf_concept_extent": [_p, _p, _i64, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p],
+    "bmf_concept_residual": [_p, _i64, _i64, _i64, _p, _i64, _p, _p, _p],
 }
 
 

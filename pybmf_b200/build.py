@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbmf_b200.so")
-SOURCES = ["bmf_core.cu", "bmf_bits.cu", "bmf_tc.cu"]
+SOURCES = ["bmf_core.cu", "bmf_bits.cu", "bmf_tc.cu", "bmf_concept.cu"]
 HEADERS = [os.path.join(CSRC, "bmf_common.cuh"), os.path.join(HERE, "..", "include", "pybmf_b200.h")]
 NVCC_FLAGS = os.environ.get("BMF_EXTRA_NVCC", "").split() + ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

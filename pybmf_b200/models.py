@@ -20,7 +20,7 @@ import scipy.sparse as sp
 import torch
 from scipy.sparse import csr_matrix, hstack, lil_matrix
 
-from . import _native, device, generate
+from . import _native, concept, device, generate
 from . import utils as U_
 from .engine import CoverEngine, _Trace, all_reduce_sum, dist_ctx, integer_weights, local_plan
 
@@ -881,6 +881,87 @@ def _transposed(X):
     if hasattr(X, "zeros"):
         return generate.DeviceEntries(generate.transpose(X.ones), generate.transpose(X.zeros))
     return generate.transpose(X) if hasattr(X, "bits") else X.T
+
+
+def _grecond_params(k, tol):
+    if tol != 0:
+        raise NotImplementedError("GreConD: only tol=0 is supported (the meaning of tol > 0 is not pinned)")
+    if k is not None and (isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1):
+        raise ValueError("GreConD: k must be None or a positive integer, got %r" % (k,))
+
+
+class GreConD(BaseModel):
+    """GreConD (Belohlavek and Vychodil's greedy search for formal concepts), as the reference runs it: each factor is
+    grown by ONE first-improvement pass over the columns (pybmf_b200.concept; DESIGN.md section 1 row f5).
+
+    `k=None` fits until the residual is empty; `k` stops after k factors.  Fewer factors come out when no column covers a
+    residual one.  Only `tol=0` is supported.  U, V are lil float64 with one column per factor; logs["updates"] has one row
+    per factor: head ("k") and train ("cover": the residual ones the factor covers, "shape": [|extent|, |intent|]), which
+    are this project's choice, then the default metrics of every split.  X_train is a host matrix, a
+    generate.DeviceBits or a generate.DeviceEntries (trained on its ones); under an initialised process group the rows are
+    sharded over the ranks and every rank gets the same factors."""
+
+    def __init__(self, k=None, tol=0):
+        _grecond_params(k, tol)
+        self.check_params(k=k, tol=tol)
+
+    def fit(self, X_train, X_val=None, X_test=None, **kwargs):
+        _native.require_gpu()
+        for name in ("U", "V", "X_pd"):                        # a fit always starts from empty factors
+            self.__dict__.pop(name, None)
+        super().fit(X_train, X_val, X_test, **kwargs)
+        self._dev_log_batch = []
+        try:
+            self._fit()
+        finally:
+            self._flush_logs()
+            self.__dict__.pop("_dev_log_batch", None)
+            self.__dict__.pop("_dev_counts", None)
+        self.U, self.V = _csr_to_lil_fast(self.U), _csr_to_lil_fast(self.V)
+        self.__dict__.pop("X_pd", None)
+        self.finish(show_logs=self.show_logs, save_model=self.save_model, show_result=self.show_result)
+
+    def check_params(self, **kwargs):
+        super().check_params(**kwargs)
+        _grecond_params(getattr(self, "k", None), getattr(self, "tol", 0))
+
+    def _init_factors(self):
+        self.U, self.V = csr_matrix((self.m, 0)), csr_matrix((self.n, 0))
+
+    def _fit(self):
+        _plan, r0, r1, x_bits = _local_rows(self.X_train)
+        search = concept.Concepts(x_bits, self.m, self.n, r0, r1)
+        size = self.m * self.n
+        extents, intents, tp = [], [], 0
+        while self.k is None or len(extents) < self.k:
+            got = search.factor()
+            if got is None:
+                self._early_stop(msg="No column covers a residual one.", verbose=True)
+                break
+            extent, intent, cover = got
+            extents.append(extent)
+            intents.append(intent)
+            tp += cover
+            self.U, self.V = _columns(extents, self.m), _columns(intents, self.n)
+            self._dev_counts = (tp, 0, search.ones - tp, size)       # every factor is a concept of X: no false positive
+            t = len(extents) - 1
+            self.evaluate(df_name="updates", head_info={"k": t},
+                          train_info={"cover": cover, "shape": [len(extent), len(intent)]}, verbose=self.verbose)
+            err = U_.rates(tp, 0, search.ones - tp, size)["ERR"]
+            if not self.early_stop(error=err) or not self.early_stop(n_factor=len(extents)):
+                break
+
+    def _split_counts(self, name):
+        if name == "train" and "_dev_counts" in self.__dict__ and self.task == "reconstruction":
+            return self._dev_counts
+        return super()._split_counts(name)
+
+
+def _columns(sets, rows):
+    """Index arrays (one per factor) -> a rows x len(sets) csr float64 with ones at those indices."""
+    r = np.concatenate(sets) if sets else np.zeros(0, np.int64)
+    c = np.repeat(np.arange(len(sets)), [len(s) for s in sets])
+    return csr_matrix((np.ones(len(r)), (r, c)), shape=(rows, len(sets)))
 
 
 class AssoOpt(Asso):
